@@ -15,6 +15,10 @@ One process per GPU; each rank runs its own independent stream (no data-path col
 `--impl reference` times the reference's algorithm on the host CPU cores (the oracle port of the OpenCL
 kernels, OpenMP on all cores; the reference itself needs an OpenCL device, which this box lacks) on a
 bounded sample of the same workload.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step computed (its output frames and the flow
+field its search produced) as DIR/<name>.npy, so that two builds run with the same arguments can be compared output for
+output: the inputs are seeded, the same from run to run.
 """
 import argparse
 import json
@@ -169,6 +173,31 @@ def dist_env():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     return rank, world, local
+
+
+DUMP_SAMPLES = 1 << 20         # values kept of a larger array: a fixed, seeded sample
+DUMP_BYTES = 64 * 1000 * 1000  # all arrays of one dump together
+
+
+def dump_outputs(out_dir, calc, blends, hdr):
+    """The arrays a caller of the timed step receives after it: the len(blends) output frames of warpFramesBatch, in order,
+    as output<k>.npy, and the flow field the step's calculateOpticalFlowAsync produced, as flow.npy.  float32 (exact for
+    the 8/16-bit samples and 16-bit offsets).  An array longer than the per-array share of DUMP_BYTES (at most
+    DUMP_SAMPLES values) is stored as the values at sorted indices drawn with a fixed seed: the same positions in every
+    run."""
+    n_el = calc.outputFrameBytes // (2 if hdr else 1)
+    arrays = {}
+    for k in range(len(blends)):
+        a = np.empty(n_el, np.uint16 if hdr else np.uint8)
+        calc.downloadFrame(a)
+        arrays[f"output{k}"] = a
+    arrays["flow"] = calc.readFlow(latest=True).reshape(-1)
+    cap = min(DUMP_SAMPLES, (DUMP_BYTES - 1024 * len(arrays)) // 4 // len(arrays))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 def algorithmic_bytes(wl):
@@ -606,7 +635,11 @@ def main():
     ap.add_argument("--no-batch", action="store_true", help="one warpFrames call per output frame, as the reference's loop does (A/B of warpFramesBatch)")
     ap.add_argument("--radius", type=int, default=SEARCH_RADIUS)
     ap.add_argument("--streams-per-gpu", type=int, default=1, help="independent video streams (handles) per GPU; >1 prints the multi-stream line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the output frames and the flow of the last timed "
+                    "step to DIR/<name>.npy (float32, 64 MB at most; rank 0; single-stream CUDA path only)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "cfg4" or args.streams_per_gpu > 1):
+        ap.error("--dump-outputs applies to the single-stream CUDA path (--impl ours, one stream per GPU, not cfg4)")
     claim_stdout()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     wl = WORKLOADS[args.workload]
@@ -764,6 +797,8 @@ def main():
     launches = sum_over_ranks(hr.kernel_launch_count() - launches0)
     total_frames = sum_over_ranks(frames)
     value = total_frames / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, calc, sched[idx - 1], hdr)
 
     # ---- the same loop at the auto-tuner's lower bound R=5 (SURVEY.md section 8(d): "also report R = 5") ----
     r5 = None

@@ -18,17 +18,23 @@ import pytest
 from oracle import OracleCalc, kernels
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-FILES = sorted(glob.glob(os.path.join(GOLDEN, "*.npz")))
+FILES = sorted(f for f in glob.glob(os.path.join(GOLDEN, "*.npz")) if not f.endswith(".outputs.npz"))
+CASE_IDS = [os.path.basename(f)[:-4] for f in FILES]
 
 
 from conftest import oob_windows  # noqa: E402
 
 
-@pytest.fixture(scope="module", params=FILES, ids=[os.path.basename(f)[:-4] for f in FILES])
+def load_case(path):
+    """One recorded case: <case>.npz (spec, input frames, search taps, flows) and <case>.outputs.npz (output frames)."""
+    g = dict(np.load(path))
+    g.update(np.load(path[:-4] + ".outputs.npz"))
+    return g, json.loads(str(g["spec"]))
+
+
+@pytest.fixture(scope="module", params=FILES, ids=CASE_IDS)
 def golden(request):
-    g = np.load(request.param)
-    spec = json.loads(str(g["spec"]))
-    return g, spec
+    return load_case(request.param)
 
 
 def test_manifest_names_the_reference_device():
@@ -110,7 +116,7 @@ def test_warp_and_copy_outputs(golden):
     from make_golden import WARPS  # the exact (blendingScalar, mode) pairs the reference was driven with
     for t, mode in WARPS:
         key = f"warp_m{mode}_t{t:.4f}"
-        if key not in g.files:  # the larger cases keep a subset of the outputs (MANIFEST.json)
+        if key not in g:  # the larger cases keep a subset of the outputs (MANIFEST.json)
             continue
         o.warpFrames(t, mode)
         out = np.zeros(o.outputFrameBytes // dt().itemsize, dt)
