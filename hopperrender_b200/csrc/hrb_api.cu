@@ -175,7 +175,9 @@ static int issueFlowKernels(hrb_ofc* h, int R, int ws0, int iterations, bool iss
             a.rawDelta = (iter == 0 && step == 0) ? h->rawDeltaDev : nullptr;
             a.tapSums = nullptr;
             a.tapLayer = nullptr;
-            a.dbg = h->dbgDev ? h->dbgDev + (size_t)(iter * 2 + step) * h->dbgStride : nullptr;
+            const bool dbgPass = h->dbgDev && iter * 2 + step < 32;
+            a.dbg = dbgPass ? h->dbgDev + (size_t)(iter * 2 + step) * h->dbgStride : nullptr;
+            a.dbgWords = dbgPass ? h->dbgStride : 0;
             a.winLanes = h->searchVariant != 4;
             if (h->tapMode) {
                 PassTapDev t;
@@ -1186,8 +1188,9 @@ int hrb_ofc_set_search_variant(hrb_ofc* h, int variant) {
     return HRB_OK;
 }
 
-// Debug aid: per-CTA timelines of the tile search kernels (8 words per CTA: start, boxes landed, runs done, end
-// [globaltimer ns], SM id, block x, block y, rounds), `words_per_pass` words for each of up to 32 passes.
+// Debug aid: per-CTA timelines of the tile search kernels (16 words per CTA: start, boxes landed, runs done, end
+// [globaltimer ns], SM id, block x, block y, rounds, warps per CTA, 7 spare), `words_per_pass` words for each of up to 32
+// passes.  CTA i of a pass records only if its record fits the slice (16 * (i + 1) <= words_per_pass).
 int hrb_ofc_debug_timeline(hrb_ofc* h, size_t words_per_pass) {
     HRB_REQUIRE(h, "null handle");
     HRB_CUDA(cudaSetDevice(h->device));

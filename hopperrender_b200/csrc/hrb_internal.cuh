@@ -76,7 +76,8 @@ struct SearchArgs {
     uint32_t* rawDelta;    // non-null in pass 0: receives sums[R/2-1][window 0]
     uint32_t* tapSums;     // optional [R][nWy][nWx]
     uint8_t* tapLayer;     // optional [nWy][nWx]
-    unsigned long long* dbg;  // optional per-CTA timeline of this pass (hrb_ofc_debug_timeline): 8 words per CTA
+    unsigned long long* dbg;  // optional per-CTA timeline of this pass (hrb_ofc_debug_timeline): 16 words per CTA ...
+    size_t dbgWords;          // ... in a slice of this many words; CTAs whose record does not fit it record nothing
     bool winLanes;         // windows of 2 and 4: one lane per window (off: search variant 4, the butterfly form, for A/B runs)
 };
 

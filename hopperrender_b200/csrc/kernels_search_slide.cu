@@ -181,6 +181,9 @@ struct BoxGeom {
         return whole ? (sc >= 0 && sc < nCh) : (pc >= 0 && pc < nCh);
     }
     __device__ __forceinline__ bool outsideChunks() const { return pc0 < 0 || pc0 + nK > nCh; }
+    // the box reaches the last, partial chunk of a row (plane width not a multiple of 16): stageIssue leaves it to
+    // stageFixup even where the tile reads only in-plane bytes of it
+    __device__ __forceinline__ bool partialTail() const { return !whole && pc0 + nK > nCh; }
 };
 
 __device__ __noinline__ void stageIssue(const BoxGeom g, int tid, int nThreads) {
@@ -270,7 +273,9 @@ __global__ void __maxnreg__(128)
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
         return t;
     };
-    unsigned long long* const dbg = a.dbg ? a.dbg + 16 * (size_t)(blockIdx.y * gridDim.x + blockIdx.x) : nullptr;
+    // 16 words per CTA; a CTA whose record does not fit the pass's slice records nothing (CTA-uniform)
+    const size_t cta = (size_t)blockIdx.y * gridDim.x + blockIdx.x;
+    unsigned long long* const dbg = a.dbg && 16 * (cta + 1) <= a.dbgWords ? a.dbg + 16 * cta : nullptr;
     if (tid == 0) {
         mbarInit(&barY, NT);  // every thread arrives once its own cp.async copies of the luma box have landed
         mbarInit(&barC, 1);   // the elected thread arrives with the byte count of the chroma TMA box
@@ -283,6 +288,7 @@ __global__ void __maxnreg__(128)
             dbg[4] = smid;
             dbg[5] = blockIdx.x;
             dbg[6] = blockIdx.y;
+            dbg[8] = blockDim.y;  // warps of the CTA (NWV)
         }
     }
     for (int i = tid; i < 128; i += NT) s_red[i >> 4][i & 15] = 0;
@@ -409,7 +415,9 @@ __global__ void __maxnreg__(128)
         const BoxGeom gy(bufY, BW, vw.y1, vw.pitch, vw.dimU, vw.dimV, rb, ca, subR0, subR1, subC0, subC1);
         const BoxGeom gc(bufC, BW, vw.c1, vw.pitch, vw.dimU, vw.dimV >> 1, rbc, caC, subR0C, subR1C, subC0C, subC1C);
         const bool needFix = gc.outsideChunks() || gy.outsideChunks();                  // chunks left / right of the plane: reversed after landing
-        const bool tmaStage = staged && !manual && !border && round == 0;               // CTA-uniform, like the two below
+        // CTA-uniform, like the two below.  The TMA branch runs no fix-up: a luma box that reaches the partial last chunk
+        // of a row is staged like a border tile
+        const bool tmaStage = staged && !manual && !border && round == 0 && !gy.partialTail();
         const bool pipeStage = staged && round == 0 && !tmaStage && !needFix;
         const bool asyncStage = tmaStage || pipeStage;
         if (tmaStage) {

@@ -231,9 +231,11 @@ HRB_API int hrb_ofc_set_flow_overlap(hrb_ofc* h, int on);
 /* Orders the compute stream (hrb_ofc_stream) behind the flow calculation still running on the flow stream, without
  * blocking the host: work a caller enqueues on the compute stream afterwards sees the finished flow. */
 HRB_API int hrb_ofc_join_flow(hrb_ofc* h);
-/* Debug aid: record a per-CTA timeline of every tile search kernel of the following flow calculations (8 uint64 per
- * CTA: start, boxes landed, runs done, end [globaltimer ns], SM id, block x, block y, rounds; `words_per_pass` words for
- * each of up to 32 passes; 0 switches it off).  Used by tools/cta_timeline.py. */
+/* Debug aid: record a per-CTA timeline of every tile search kernel of the following flow calculations (16 uint64 per
+ * CTA: start, boxes landed, runs done, end [globaltimer ns], SM id, block x, block y, rounds (+100 on a border tile; 5 =
+ * the per-pixel remainder), warps per CTA, then 7 zero words; `words_per_pass` words for each of up to 32 passes; 0
+ * switches it off).  CTA i of a pass records only if 16 * (i + 1) <= words_per_pass, so passes never overlap.  The
+ * buffer is zeroed here, not per calculation.  Used by tools/cta_timeline.py. */
 HRB_API int hrb_ofc_debug_timeline(hrb_ofc* h, size_t words_per_pass);
 HRB_API int hrb_ofc_debug_timeline_read(hrb_ofc* h, void* dst, size_t bytes);
 /* number of kernels this library has launched in this process */

@@ -178,23 +178,31 @@ SEARCH_CASES = [
     (False, 320, 200, 270, 0, 9, "ramp"),
     (True, 384, 224, 270, 0, 16, "scene"),
     (False, 16, 16, 270, 0, 5, "random"),
-    (False, 722, 430, 430, 0, 16, "scene"),     # partial 32x32 tiles on both edges, windows 512..2
+    (False, 722, 430, 430, 0, 16, "scene"),     # both sizes = 2 (mod 4): no tile kernel; partial tiles on both edges of the small-window and generic kernels, windows 512..2
     (True, 640, 384, 384, 672, 7, "scene"),
-    (False, 450, 258, 258, 0, 12, "random"),    # large offsets: mirrored halos in the sliding-window kernels
+    (False, 450, 258, 258, 0, 12, "random"),    # large offsets; both sizes = 2 (mod 4), so the tile kernel is skipped (the 452x260 row reaches it)
     (False, 200, 120, 270, 0, 2, "scene"),      # radii below the filter's minimum of 5 take the generic kernel
     (True, 200, 120, 270, 0, 3, "random"),
     (False, 290, 170, 270, 0, 13, "scene"),
     (True, 290, 170, 270, 300, 15, "random"),
     (False, 272, 160, 270, 0, 4, "ramp"),
+    # both sizes multiples of 4: the tile kernel serves windows >= 16 (>= 4 under variants 2 and 3), one row per radius
+    (True, 128, 96, 270, 0, 6, "random"),
+    (False, 256, 128, 270, 0, 8, "scene"),
+    (True, 320, 180, 270, 0, 10, "random"),
+    (False, 452, 260, 270, 0, 12, "random"),    # large offsets: mirrored halos of the tile kernel's boxes
+    (True, 292, 172, 270, 0, 13, "scene"),
+    (False, 384, 216, 270, 416, 14, "random"),
+    (True, 288, 168, 270, 0, 15, "scene"),
 ]
 
 
-@pytest.mark.parametrize("variant", [0, 1, 2, 3, 4], ids=["auto", "generic", "notma", "perpixel", "butterfly"])
-@pytest.mark.parametrize("hdr,W,H,maxres,inS,R,kind", SEARCH_CASES)
-def test_search_ladder_taps(synth, hdr, W, H, maxres, inS, R, kind, variant):
-    """Every pass of the ladder: window sums, arg-min layers and offsets are bit-exact — with the automatic kernel
-    selection (sliding-window kernels for windows >= 32) and with the generic kernel forced for every pass."""
-    g, o = make_pair(hdr, H, W, inS, 0, maxres=maxres, R=R)
+def check_ladder_taps(synth, hdr, W, H, maxres, inS, R, kind, variant, ds=8, ns=6):
+    """Every pass of the ladder against the oracle with taps: window sums, arg-min layers and offsets bit-exact, then the
+    final offsets, the blurred flow and the frame delta.  Then the same frames without taps, where the ladder runs from a
+    CUDA graph: the two blurred-flow buffers alternate, so calculations 1 and 2 capture a graph each and calculation 3
+    replays the first; each must give the same offsets, flow and frame delta as the tap run and the oracle."""
+    g, o = make_pair(hdr, H, W, inS, 0, ds=ds, ns=ns, maxres=maxres, R=R)
     g.setSearchVariant(variant)
     g.setTapMode(True)
     o.enableTaps(True)
@@ -215,9 +223,62 @@ def test_search_ladder_taps(synth, hdr, W, H, maxres, inS, R, kind, variant):
         l_ref = o.readPassLayers(p)[::ws, ::ws]
         assert np.array_equal(g.readPassLayers(p), l_ref), f"pass {p}: layers differ"
         assert np.array_equal(g.readPassOffsets(p), o.readPassOffsets(p)), f"pass {p}: offsets differ"
-    assert np.array_equal(g.readOffsetArray(), o.readOffsetArray())
-    assert np.array_equal(g.readFlow(latest=True), o.readFlow(latest=True)), "blurred flow differs"
-    assert g.m_totalFrameDelta == o.state().totalFrameDelta
+    off, flow, delta = o.readOffsetArray(), o.readFlow(latest=True), o.state().totalFrameDelta
+    assert np.array_equal(g.readOffsetArray(), off)
+    assert np.array_equal(g.readFlow(latest=True), flow), "blurred flow differs"
+    assert g.m_totalFrameDelta == delta
+    g.setTapMode(False)
+    for k in range(3):
+        g.calculateOpticalFlow()
+        assert np.array_equal(g.readOffsetArray(), off), f"production calculation {k}: offsets differ"
+        assert np.array_equal(g.readFlow(latest=True), flow), f"production calculation {k}: blurred flow differs"
+        assert g.m_totalFrameDelta == delta, f"production calculation {k}: frame delta"
+
+
+@pytest.mark.parametrize("variant", [0, 1, 2, 3, 4], ids=["auto", "generic", "notma", "perpixel", "butterfly"])
+@pytest.mark.parametrize("hdr,W,H,maxres,inS,R,kind", SEARCH_CASES)
+def test_search_ladder_taps(synth, hdr, W, H, maxres, inS, R, kind, variant):
+    """Every pass of the ladder: window sums, arg-min layers and offsets are bit-exact — with the automatic kernel
+    selection (sliding-window kernels for windows >= 32) and with the generic kernel forced for every pass — and the
+    production path (no taps, CUDA graph) gives the same final offsets, flow and frame delta."""
+    check_ladder_taps(synth, hdr, W, H, maxres, inS, R, kind, variant)
+
+
+@pytest.mark.parametrize("ds,ns", [(0, 0), (31, 31), (24, 31), (31, 0)])
+@pytest.mark.parametrize("hdr,W,H,maxres,inS,R,kind", [
+    (False, 512, 256, 270, 0, 16, "scene"),    # tile kernel for windows >= 16
+    (True, 258, 146, 270, 0, 11, "random"),    # sizes = 2 (mod 4): small-window kernel for windows <= 32, generic above
+])
+def test_search_ladder_scalar_extremes(synth, hdr, W, H, maxres, inS, R, kind, ds, ns):
+    """deltaScalar / neighborBiasScalar at the ends of 0..31, where the uint32 window sums wrap: bit-exact pass by pass."""
+    check_ladder_taps(synth, hdr, W, H, maxres, inS, R, kind, 0, ds=ds, ns=ns)
+
+
+def test_flow_graph_cache_beyond_64_keys(synth):
+    """More than 64 distinct (radius, scalars, input slots, output buffer) flow-graph keys through one small handle (the
+    cache starts over past 64), the flow checked against the oracle after every calculation; then early keys again."""
+    W, H = 96, 64
+    g, o = make_pair(False, H, W, R=5)
+    fs = frames(synth, W, H, False, 6)
+    for fr in fs[:3]:
+        g.updateFrame(fr)
+        o.updateFrame(fr)
+    keys = [(R, ds, ns) for ds, ns in [(8, 6), (0, 0), (31, 31), (4, 10), (12, 1)] for R in range(2, 17)]
+    assert len(keys) > 64
+    for k, (R, ds, ns) in enumerate(keys + keys[:10]):
+        if k % 9 == 8:   # rotate the input slots now and then
+            fr = fs[3 + (k // 9) % 3]
+            g.updateFrame(fr)
+            o.updateFrame(fr)
+        g.m_opticalFlowSearchRadius = R
+        g.m_deltaScalar = ds
+        g.m_neighborBiasScalar = ns
+        o.setParams(R, ds, ns)
+        g.calculateOpticalFlow()
+        o.calculateOpticalFlow()
+        assert np.array_equal(g.readOffsetArray(), o.readOffsetArray()), f"calculation {k} {(R, ds, ns)}: offsets differ"
+        assert np.array_equal(g.readFlow(latest=True), o.readFlow(latest=True)), f"calculation {k} {(R, ds, ns)}: flow differs"
+        assert g.m_totalFrameDelta == o.state().totalFrameDelta, f"calculation {k} {(R, ds, ns)}: frame delta"
 
 
 @pytest.mark.parametrize("hdr,W,H,maxres,R", [(False, 1920, 1080, 270, 16), (False, 1920, 1080, 540, 16), (True, 960, 540, 2160, 5)])

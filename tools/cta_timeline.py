@@ -17,7 +17,10 @@ for f in fr[:3]:
     g.updateFrame(f)
 g.calculateOpticalFlow()
 g.updateFrame(fr[3]); g.calculateOpticalFlow()
-WPP = 16 * 1024
+# 16 words per CTA.  A tile CTA covers 128 flow pixels along u and 32 * NWV >= 64 along v (u = x for Y steps, u = y for X
+# steps), so no pass launches more CTAs than the bound below; a CTA whose record does not fit the slice records nothing.
+lh, lw = g.m_opticalFlowFrameHeight, g.m_opticalFlowFrameWidth
+WPP = 16 * max(-(-lw // 128) * -(-lh // 64), -(-lh // 128) * -(-lw // 64))
 g.debugTimeline(WPP)
 g.updateFrame(fr[4]); g.calculateOpticalFlow()
 tl = g.readDebugTimeline(WPP)
@@ -36,7 +39,7 @@ for p in range(32):
           f"rounds max {rounds.max()} mean {rounds.mean():.2f} border {border.sum()}")
     worst = np.argsort(-en)[:4]
     for i in worst:
-        print("          dbg:", [round((int(t[i, k]) - int(t0)) / 1e3, 1) if t[i, k] else 0 for k in (0, 8, 9, 10, 11, 1, 2, 3)], int(t[i,5]), int(t[i,6]))
+        print("          dbg:", [round((int(t[i, k]) - int(t0)) / 1e3, 1) if t[i, k] else 0 for k in (0, 1, 2, 3)], int(t[i,5]), int(t[i,6]), f"nwv{int(t[i,8])}")
     print("          slowest:", [(int(t[i, 5]), int(t[i, 6]), f"sm{int(t[i,4])}", f"st{st[i]:.1f}", f"bx{bx[i]-st[i]:.1f}", f"run{rn[i]-bx[i]:.1f}", f"end{en[i]:.1f}", int(t[i, 7])) for i in worst])
     # CTAs per SM and per-SM busy time
     sm = t[:, 4].astype(int)
