@@ -6,9 +6,9 @@ loads the CUDA library and fails loudly when it is missing — there is no CPU f
 """
 from . import _lib
 from .ofc import (BlendedFrame, GreyFlow, HSVFlow, OpticalFlowCalc, OpticalFlowCalcHDR, OpticalFlowCalcSDR, SideBySide1,
-                  SideBySide2, WarpedFrame12, WarpedFrame21, kernel_launch_count, microbench_sad_peak)
+                  SideBySide2, SplitSearch, WarpedFrame12, WarpedFrame21, kernel_launch_count, microbench_sad_peak, split_plan)
 
 _lib.load()
 
 __all__ = ["OpticalFlowCalc", "OpticalFlowCalcSDR", "OpticalFlowCalcHDR", "WarpedFrame12", "WarpedFrame21", "BlendedFrame",
-           "HSVFlow", "GreyFlow", "SideBySide1", "SideBySide2", "kernel_launch_count", "microbench_sad_peak"]
+           "HSVFlow", "GreyFlow", "SideBySide1", "SideBySide2", "SplitSearch", "split_plan", "kernel_launch_count", "microbench_sad_peak"]

@@ -75,6 +75,12 @@ PROTOTYPES = {
     "hrb_host_alloc": (C.c_int, [C.POINTER(_P), C.c_size_t]),
     "hrb_host_free": (C.c_int, [_P]),
     "hrb_ofc_set_output_stripe": (C.c_int, [_P, C.c_int, C.c_int]),
+    "hrb_split_plan": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_int)]),
+    "hrb_split_create": (C.c_int, [C.POINTER(_P), C.POINTER(_P), C.c_int]),
+    "hrb_split_destroy": (None, [_P]),
+    "hrb_split_stripe": (C.c_int, [_P, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "hrb_split_calculate_optical_flow": (C.c_int, [_P]),
+    "hrb_split_calculate_optical_flow_async": (C.c_int, [_P]),
     "hrb_ofc_set_tap_mode": (C.c_int, [_P, C.c_int]),
     "hrb_ofc_num_passes": (C.c_int, [_P, C.POINTER(C.c_int)]),
     "hrb_ofc_pass_info": (C.c_int, [_P, C.c_int] + [C.POINTER(C.c_int)] * 5),

@@ -1,5 +1,6 @@
 // hrb_api.cu — handle management, the per-frame host schedule and the C ABI (include/hrb.h).
 // The schedule restates HopperRender/opticalFlowCalcSDR.cpp / opticalFlowCalcHDR.cpp on one CUDA stream.
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -135,10 +136,9 @@ static int resolveFlow(hrb_ofc* h) {
     return HRB_OK;
 }
 
-// The search ladder and the blur of one flow calculation.  issue = false only replays the host-side bookkeeping
-// (the kernels are then launched from a captured graph).
-static int issueFlowKernels(hrb_ofc* h, int R, int ws0, int iterations, bool issue) {
-    const int lw = h->flowWidth, lh = h->flowHeight;
+// One iteration (two passes) of the ladder on one handle; the passes compute the windows of flow rows [rowBegin, rowEnd).
+static int issueIteration(hrb_ofc* h, int R, int ws, int iter, int prevNWx, int prevNWy, int rowBegin, int rowEnd, bool issue) {
+    const int par = iter & 1;
     SearchArgs a;
     memset(&a, 0, sizeof(a));
     const SearchPlanes& f1 = h->searchPlane[1];  // frame1 = m_inputFrameArray[1], opticalFlowCalcSDR.cpp:79
@@ -149,96 +149,244 @@ static int issueFlowKernels(hrb_ofc* h, int R, int ws0, int iterations, bool iss
     a.pitchT = h->planePitchT;
     a.W = h->frameWidth;
     a.H = h->frameHeight;
-    a.lw = lw;
-    a.lh = lh;
+    a.lw = h->flowWidth;
+    a.lh = h->flowHeight;
     a.rs = h->resScalar;
     a.deltaScalar = h->deltaScalar;
     a.neighborBiasScalar = h->neighborBiasScalar;
     a.winSums = h->winSums;
     a.winTicket = h->winTicket;
+    a.ws = ws;
+    a.wsLog2 = ilog2(ws);
+    a.iteration = iter;
+    a.nWx = (a.lw + ws - 1) / ws;
+    a.nWy = (a.lh + ws - 1) / ws;
+    a.rowBegin = rowBegin;
+    a.rowEnd = rowEnd;
+    a.prevNWx = prevNWx;
+    a.prevX = iter ? h->levelOffsets[par ^ 1][0] : nullptr;
+    a.prevY = iter ? h->levelOffsets[par ^ 1][1] : nullptr;
+    a.curX = h->levelOffsets[par][0];
+    a.curY = h->levelOffsets[par][1];
+    for (int step = 0; step < 2; ++step) {
+        a.rawDelta = (iter == 0 && step == 0) ? h->rawDeltaDev : nullptr;
+        a.tapSums = nullptr;
+        a.tapLayer = nullptr;
+        const bool dbgPass = h->dbgDev && iter * 2 + step < 32;
+        a.dbg = dbgPass ? h->dbgDev + (size_t)(iter * 2 + step) * h->dbgStride : nullptr;
+        a.dbgWords = dbgPass ? h->dbgStride : 0;
+        a.winLanes = h->searchVariant != 4;
+        if (h->tapMode) {
+            PassTapDev t;
+            t.g.windowSize = ws;
+            t.g.wsLog2 = a.wsLog2;
+            t.g.iteration = iter;
+            t.g.step = step;
+            t.g.nWx = a.nWx;
+            t.g.nWy = a.nWy;
+            t.g.prevNWx = prevNWx;
+            t.g.prevNWy = prevNWy;
+            const size_t nW = (size_t)a.nWx * a.nWy;
+            HRB_CUDA(cudaMalloc(&t.sums, nW * R * sizeof(uint32_t)));
+            HRB_CUDA(cudaMalloc(&t.layer, nW));
+            HRB_CUDA(cudaMalloc(&t.offX, nW * sizeof(int16_t)));
+            HRB_CUDA(cudaMalloc(&t.offY, nW * sizeof(int16_t)));
+            // zeroed, so that the windows a sharded pass does not compute read back as zero
+            HRB_CUDA(cudaMemsetAsync(t.sums, 0, nW * R * sizeof(uint32_t), h->stream));
+            HRB_CUDA(cudaMemsetAsync(t.layer, 0, nW, h->stream));
+            a.tapSums = t.sums;
+            a.tapLayer = t.layer;
+            h->taps.push_back(t);
+        }
+        if (issue) {
+            const int rc = launchSearchPass(h, a, R, step);
+            if (rc) return rc;
+        }
+        if (h->tapMode) {
+            PassTapDev& t = h->taps.back();
+            const size_t nW = (size_t)a.nWx * a.nWy;
+            HRB_CUDA(cudaMemcpyAsync(t.offX, a.curX, nW * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
+            t.wsX = ws;
+            t.nWxX = a.nWx;
+            t.nWyX = a.nWy;
+            if (step == 1) {
+                HRB_CUDA(cudaMemcpyAsync(t.offY, a.curY, nW * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
+                t.wsY = ws;
+                t.nWxY = a.nWx;
+                t.nWyY = a.nWy;
+            } else if (iter > 0) {
+                HRB_CUDA(cudaMemcpyAsync(t.offY, a.prevY, (size_t)prevNWx * prevNWy * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
+                t.wsY = ws * 2;
+                t.nWxY = prevNWx;
+                t.nWyY = prevNWy;
+            } else {
+                t.wsY = 0;  // all zero
+            }
+        }
+    }
+    h->lastIterParity = par;
+    h->lastNWx = a.nWx;
+    h->lastNWy = a.nWy;
+    h->lastWs = ws;
+    return HRB_OK;
+}
 
+}  // namespace hrb
+
+// A group of handles that compute one flow together (include/hrb.h, split search).  It owns no device memory: the level
+// arrays exchanged are the handles' own.
+struct hrb_split {
+    std::vector<hrb_ofc*> shard;
+    std::vector<int> bounds;          // shard k owns the flow rows [bounds[k], bounds[k + 1])
+    std::vector<cudaEvent_t> done;    // per shard, created on its device: its part of an iteration / its pushes are enqueued
+};
+
+namespace hrb {
+
+constexpr int kMaxShards = 64;
+
+// The handles one ladder runs on: a lone handle (one shard that owns every flow row) or the shards of a group.
+struct Shards {
+    hrb_ofc* const* h;
+    const int* bounds;   // n + 1 flow-row bounds
+    int n;
+    cudaEvent_t* done;   // n > 1 only
+    explicit Shards(hrb_ofc* lone) : h(&one), bounds(rows), n(1), done(nullptr), one(lone), rows{0, lone->flowHeight} {}
+    explicit Shards(hrb_split* s) : h(s->shard.data()), bounds(s->bounds.data()), n((int)s->shard.size()), done(s->done.data()), one(nullptr), rows{0, 0} {}
+    Shards(const Shards&) = delete;
+    Shards& operator=(const Shards&) = delete;
+
+   private:
+    hrb_ofc* one;
+    int rows[2];
+};
+
+// `bytes` from device memory of shard `from` to device memory of shard `to`, on `st`
+static int copyShard(const hrb_ofc* to, void* dst, const hrb_ofc* from, const void* src, size_t bytes, cudaStream_t st) {
+    if (to->device == from->device)
+        HRB_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st));
+    else
+        HRB_CUDA(cudaMemcpyPeerAsync(dst, to->device, src, from->device, bytes, st));
+    return HRB_OK;
+}
+
+// Between two sharded iterations: the neighbour bias of a window of the next level reads parent windows w/2 +- 1
+// (SURVEY.md A.1), so every shard pulls the parent-level window row just above and just below its stripe, both axes,
+// from the shards that own them.  Each shard waits for its neighbours' part of the iteration first.  The neighbour
+// overwrites these rows two iterations later, after it has waited for this shard's next iteration, which follows the
+// copies on this shard's stream.
+static int exchangeHalo(const Shards& s, int par, int ws, int nWx, int nWy) {
+    for (int k = 0; k < s.n; ++k) {
+        HRB_CUDA(cudaSetDevice(s.h[k]->device));
+        HRB_CUDA(cudaEventRecord(s.done[k], s.h[k]->stream));
+    }
+    for (int k = 0; k < s.n; ++k) {
+        hrb_ofc* h = s.h[k];
+        HRB_CUDA(cudaSetDevice(h->device));
+        const int nb[2] = {k - 1, k + 1};
+        const int row[2] = {s.bounds[k] / ws - 1, s.bounds[k + 1] / ws};  // bounds are multiples of ws (or lh, which has no shard below)
+        for (int i = 0; i < 2; ++i) {
+            if (nb[i] < 0 || nb[i] >= s.n || row[i] < 0 || row[i] >= nWy) continue;
+            const hrb_ofc* from = s.h[nb[i]];
+            HRB_CUDA(cudaStreamWaitEvent(h->stream, s.done[nb[i]], 0));
+            for (int ax = 0; ax < 2; ++ax) {
+                const size_t off = (size_t)row[i] * nWx;
+                const int rc = copyShard(h, h->levelOffsets[par][ax] + off, from, from->levelOffsets[par][ax] + off, (size_t)nWx * sizeof(int16_t), h->stream);
+                if (rc) return rc;
+            }
+        }
+    }
+    return HRB_OK;
+}
+
+// After the last iteration: every shard pushes the window rows it owns of the final level (and shard 0 the raw frame
+// delta, when pass 0 was sharded) to every other shard, then each waits for all pushes into it.
+// The pushes start only once EVERY shard has finished its last iteration (an all-to-all barrier, not the neighbour
+// ordering of exchangeHalo): the receiver's array of the final level's parity is also the array of levels L-2, L-4, ...,
+// which it read and wrote in earlier iterations at a coarser geometry whose offsets overlap the pushed rows, and a
+// shard n - 1 hops away is ordered behind the receiver's iteration L - (n - 1) only.  The tap copies of the last
+// iteration are enqueued before the barrier too, so they never see a push.
+static int gatherLevel(const Shards& s, int par, int ws, int nWx, int nWy, bool rawDelta) {
+    for (int k = 0; k < s.n; ++k) {
+        HRB_CUDA(cudaSetDevice(s.h[k]->device));
+        HRB_CUDA(cudaEventRecord(s.done[k], s.h[k]->stream));
+    }
+    for (int j = 0; j < s.n; ++j) {
+        hrb_ofc* from = s.h[j];
+        HRB_CUDA(cudaSetDevice(from->device));
+        for (int k = 0; k < s.n; ++k)
+            if (k != j) HRB_CUDA(cudaStreamWaitEvent(from->stream, s.done[k], 0));  // (the wait takes the record above)
+    }
+    for (int j = 0; j < s.n; ++j) {
+        hrb_ofc* from = s.h[j];
+        HRB_CUDA(cudaSetDevice(from->device));
+        const int r0 = s.bounds[j] / ws, r1 = std::min((s.bounds[j + 1] + ws - 1) / ws, nWy);
+        for (int k = 0; k < s.n; ++k) {
+            if (k == j) continue;
+            hrb_ofc* to = s.h[k];
+            for (int ax = 0; ax < 2; ++ax) {
+                const size_t off = (size_t)r0 * nWx;
+                const int rc = copyShard(to, to->levelOffsets[par][ax] + off, from, from->levelOffsets[par][ax] + off, (size_t)(r1 - r0) * nWx * sizeof(int16_t),
+                                         from->stream);
+                if (rc) return rc;
+            }
+            if (rawDelta && j == 0) {
+                const int rc = copyShard(to, to->rawDeltaDev, from, from->rawDeltaDev, sizeof(uint32_t), from->stream);
+                if (rc) return rc;
+            }
+        }
+        HRB_CUDA(cudaEventRecord(s.done[j], from->stream));
+    }
+    for (int k = 0; k < s.n; ++k) {
+        HRB_CUDA(cudaSetDevice(s.h[k]->device));
+        for (int j = 0; j < s.n; ++j)
+            if (j != k) HRB_CUDA(cudaStreamWaitEvent(s.h[k]->stream, s.done[j], 0));
+    }
+    return HRB_OK;
+}
+
+// The search ladder and the blur of one flow calculation, on a lone handle or on the shards of a group.  Passes with
+// windows of at most kSplitAlign rows are sharded on a group: shard k computes only the windows of its rows, with
+// exchangeHalo between iterations and gatherLevel after the last one.  Passes with taller windows straddle stripes and
+// run replicated, on the whole frame, on every shard.  issue = false only replays the host-side bookkeeping (the
+// kernels are then launched from a captured graph; lone handles only).
+static int issueFlowKernels(const Shards& s, int R, int ws0, int iterations, bool issue) {
+    const int lw = s.h[0]->flowWidth, lh = s.h[0]->flowHeight;
     int prevNWx = 0, prevNWy = 0;
+    bool prevSharded = false;
     for (int iter = 0; iter < iterations; ++iter) {
         const int ws = ws0 >> iter;
         const int par = iter & 1;
-        a.ws = ws;
-        a.wsLog2 = ilog2(ws);
-        a.iteration = iter;
-        a.nWx = (lw + ws - 1) / ws;
-        a.nWy = (lh + ws - 1) / ws;
-        a.prevNWx = prevNWx;
-        a.prevX = iter ? h->levelOffsets[par ^ 1][0] : nullptr;
-        a.prevY = iter ? h->levelOffsets[par ^ 1][1] : nullptr;
-        a.curX = h->levelOffsets[par][0];
-        a.curY = h->levelOffsets[par][1];
-        for (int step = 0; step < 2; ++step) {
-            a.rawDelta = (iter == 0 && step == 0) ? h->rawDeltaDev : nullptr;
-            a.tapSums = nullptr;
-            a.tapLayer = nullptr;
-            const bool dbgPass = h->dbgDev && iter * 2 + step < 32;
-            a.dbg = dbgPass ? h->dbgDev + (size_t)(iter * 2 + step) * h->dbgStride : nullptr;
-            a.dbgWords = dbgPass ? h->dbgStride : 0;
-            a.winLanes = h->searchVariant != 4;
-            if (h->tapMode) {
-                PassTapDev t;
-                t.g.windowSize = ws;
-                t.g.wsLog2 = a.wsLog2;
-                t.g.iteration = iter;
-                t.g.step = step;
-                t.g.nWx = a.nWx;
-                t.g.nWy = a.nWy;
-                t.g.prevNWx = prevNWx;
-                t.g.prevNWy = prevNWy;
-                const size_t nW = (size_t)a.nWx * a.nWy;
-                HRB_CUDA(cudaMalloc(&t.sums, nW * R * sizeof(uint32_t)));
-                HRB_CUDA(cudaMalloc(&t.layer, nW));
-                HRB_CUDA(cudaMalloc(&t.offX, nW * sizeof(int16_t)));
-                HRB_CUDA(cudaMalloc(&t.offY, nW * sizeof(int16_t)));
-                HRB_CUDA(cudaMemsetAsync(t.sums, 0, nW * R * sizeof(uint32_t), h->stream));
-                a.tapSums = t.sums;
-                a.tapLayer = t.layer;
-                h->taps.push_back(t);
-            }
-            if (issue) {
-                const int rc = launchSearchPass(h, a, R, step);
-                if (rc) return rc;
-            }
-            if (h->tapMode) {
-                PassTapDev& t = h->taps.back();
-                const size_t nW = (size_t)a.nWx * a.nWy;
-                HRB_CUDA(cudaMemcpyAsync(t.offX, a.curX, nW * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
-                t.wsX = ws;
-                t.nWxX = a.nWx;
-                t.nWyX = a.nWy;
-                if (step == 1) {
-                    HRB_CUDA(cudaMemcpyAsync(t.offY, a.curY, nW * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
-                    t.wsY = ws;
-                    t.nWxY = a.nWx;
-                    t.nWyY = a.nWy;
-                } else if (iter > 0) {
-                    HRB_CUDA(cudaMemcpyAsync(t.offY, a.prevY, (size_t)prevNWx * prevNWy * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
-                    t.wsY = ws * 2;
-                    t.nWxY = prevNWx;
-                    t.nWyY = prevNWy;
-                } else {
-                    t.wsY = 0;  // all zero
-                }
-            }
+        const bool sharded = s.n > 1 && ws <= kSplitAlign;
+        if (sharded && prevSharded) {  // the first sharded iteration reads a parent level every shard computed in full
+            const int rc = exchangeHalo(s, par ^ 1, ws * 2, prevNWx, prevNWy);
+            if (rc) return rc;
         }
-        prevNWx = a.nWx;
-        prevNWy = a.nWy;
-        h->lastIterParity = par;
-        h->lastNWx = a.nWx;
-        h->lastNWy = a.nWy;
-        h->lastWs = ws;
+        for (int k = 0; k < s.n; ++k) {
+            hrb_ofc* h = s.h[k];
+            if (s.n > 1) HRB_CUDA(cudaSetDevice(h->device));
+            const int rc = issueIteration(h, R, ws, iter, prevNWx, prevNWy, sharded ? s.bounds[k] : 0, sharded ? s.bounds[k + 1] : lh, issue);
+            if (rc) return rc;
+        }
+        prevNWx = (lw + ws - 1) / ws;
+        prevNWy = (lh + ws - 1) / ws;
+        prevSharded = sharded;
     }
-    h->haveFlowLevels = true;
+    if (prevSharded) {
+        const int rc = gatherLevel(s, (iterations - 1) & 1, ws0 >> (iterations - 1), prevNWx, prevNWy, ws0 <= kSplitAlign);
+        if (rc) return rc;
+    }
 
     // blur into m_blurredOffsetArray[0], then swap (opticalFlowCalcSDR.cpp:113-123)
-    if (issue) {
-        const int rc = launchBlurFlow(h, h->levelOffsets[h->lastIterParity][0], h->levelOffsets[h->lastIterParity][1], h->lastNWx, ilog2(h->lastWs),
-                                      h->blurredOffsetArray[0], h->flowMaxDev[0]);
-        if (rc) return rc;
+    for (int k = 0; k < s.n; ++k) {
+        hrb_ofc* h = s.h[k];
+        h->haveFlowLevels = true;
+        if (issue) {
+            if (s.n > 1) HRB_CUDA(cudaSetDevice(h->device));
+            const int rc = launchBlurFlow(h, h->levelOffsets[h->lastIterParity][0], h->levelOffsets[h->lastIterParity][1], h->lastNWx, ilog2(h->lastWs),
+                                          h->blurredOffsetArray[0], h->flowMaxDev[0]);
+            if (rc) return rc;
+        }
     }
     return HRB_OK;
 }
@@ -252,7 +400,7 @@ static void dropFlowGraphs(hrb_ofc* h) {
 // Launches the flow kernels through a CUDA graph captured on first use for this combination of buffers and parameters
 // (24 dependent launches at 4K become one); falls back to plain launches whenever capture is not possible.
 static int launchFlowKernels(hrb_ofc* h, int R, int ws0, int iterations) {
-    if (!h->flowGraphsOn || h->tapMode || h->prof.on || h->dbgDev) return issueFlowKernels(h, R, ws0, iterations, true);
+    if (!h->flowGraphsOn || h->tapMode || h->prof.on || h->dbgDev) return issueFlowKernels(Shards(h), R, ws0, iterations, true);
     hrb_ofc::FlowGraph key;
     key.plane1 = h->searchPlane[1].base;
     key.plane2 = h->searchPlane[2].base;
@@ -272,9 +420,9 @@ static int launchFlowKernels(hrb_ofc* h, int R, int ws0, int iterations) {
         if (cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
             cudaGetLastError();
             h->flowGraphsOn = false;  // e.g. the caller's stream is the legacy default stream
-            return issueFlowKernels(h, R, ws0, iterations, true);
+            return issueFlowKernels(Shards(h), R, ws0, iterations, true);
         }
-        const int rc = issueFlowKernels(h, R, ws0, iterations, true);
+        const int rc = issueFlowKernels(Shards(h), R, ws0, iterations, true);
         cudaGraph_t graph = nullptr;
         const cudaError_t ce = cudaStreamEndCapture(h->stream, &graph);
         key.launches = (unsigned)(t_launchCount - before);
@@ -289,10 +437,10 @@ static int launchFlowKernels(hrb_ofc* h, int R, int ws0, int iterations) {
             cudaGetLastError();
             h->flowGraphsOn = false;
             if (rc) return rc;
-            return issueFlowKernels(h, R, ws0, iterations, true);
+            return issueFlowKernels(Shards(h), R, ws0, iterations, true);
         }
     } else {
-        const int rc = issueFlowKernels(h, R, ws0, iterations, false);
+        const int rc = issueFlowKernels(Shards(h), R, ws0, iterations, false);
         if (rc) return rc;
     }
     HRB_CUDA(cudaGraphLaunch(hit->exec, h->stream));
@@ -300,44 +448,59 @@ static int launchFlowKernels(hrb_ofc* h, int R, int ws0, int iterations) {
     return HRB_OK;
 }
 
-static int enqueueFlow(hrb_ofc* h) {
-    HRB_CUDA(cudaSetDevice(h->device));
-    hrb_ofc::FlowRecord& rec = h->flowRec[h->curRec];
-    if (rec.pending) {  // a second calculate on the same upload: its end event is about to be re-recorded
-        const int rc = resolveFlow(h);
-        if (rc) return rc;
+// One flow calculation on every shard's current stream (a lone handle is the group of one): the ladder, the blur, the
+// raw-delta copy, the flow record and the buffer swap of each handle.
+static int enqueueFlow(const Shards& s) {
+    hrb_ofc* const h0 = s.h[0];
+    const int R = h0->searchRadius;  // m_lowGrid8x8xL[2] = m_opticalFlowSearchRadius, opticalFlowCalcSDR.cpp:46 (equal on every shard)
+    for (int k = 0; k < s.n; ++k) {
+        hrb_ofc* h = s.h[k];
+        HRB_CUDA(cudaSetDevice(h->device));
+        if (h->flowRec[h->curRec].pending) {  // a second calculate on the same upload: its end event is about to be re-recorded
+            const int rc = resolveFlow(h);
+            if (rc) return rc;
+        }
+        if (h->searchRadius < 2 || h->searchRadius > 16) {
+            setLastError("[hopperrender_b200] search radius %d outside 2..16", h->searchRadius);
+            return HRB_ERR_INVALID_ARG;
+        }
+        if (h->deltaScalar < 0 || h->deltaScalar > 31 || h->neighborBiasScalar < 0 || h->neighborBiasScalar > 31) {
+            setLastError("[hopperrender_b200] delta/neighbor scalar outside 0..31");
+            return HRB_ERR_INVALID_ARG;
+        }
     }
-    const int R = h->searchRadius;  // m_lowGrid8x8xL[2] = m_opticalFlowSearchRadius, opticalFlowCalcSDR.cpp:46
-    if (R < 2 || R > 16) {
-        setLastError("[hopperrender_b200] search radius %d outside 2..16", R);
-        return HRB_ERR_INVALID_ARG;
-    }
-    if (h->deltaScalar < 0 || h->deltaScalar > 31 || h->neighborBiasScalar < 0 || h->neighborBiasScalar > 31) {
-        setLastError("[hopperrender_b200] delta/neighbor scalar outside 0..31");
-        return HRB_ERR_INVALID_ARG;
-    }
-    const int lw = h->flowWidth, lh = h->flowHeight;
     int ws0, iterations;
-    ladder(lw, lh, &ws0, &iterations);
-    if (!rec.startValid) {  // calculate without a preceding updateFrame: time from here
-        HRB_CUDA(cudaEventRecord(rec.start, h->stream));
-        rec.startValid = true;
+    ladder(h0->flowWidth, h0->flowHeight, &ws0, &iterations);
+    for (int k = 0; k < s.n; ++k) {
+        hrb_ofc* h = s.h[k];
+        hrb_ofc::FlowRecord& rec = h->flowRec[h->curRec];
+        if (s.n > 1) HRB_CUDA(cudaSetDevice(h->device));
+        if (!rec.startValid) {  // calculate without a preceding updateFrame: time from here
+            HRB_CUDA(cudaEventRecord(rec.start, h->stream));
+            rec.startValid = true;
+        }
+        if (h->tapMode) freeTaps(h);
     }
-    if (h->tapMode) freeTaps(h);
 
     {
-        const int rc = launchFlowKernels(h, R, ws0, iterations);
+        // a group runs plain launches: its ladder has cross-shard waits and copies between iterations
+        const int rc = s.n == 1 ? launchFlowKernels(h0, R, ws0, iterations) : issueFlowKernels(s, R, ws0, iterations, true);
         if (rc) return rc;
     }
-    HRB_CUDA(cudaMemcpyAsync(rec.rawDeltaHost, h->rawDeltaDev, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
-    HRB_CUDA(cudaEventRecord(rec.end, h->stream));
-    int16_t* t0 = h->blurredOffsetArray[0];
-    h->blurredOffsetArray[0] = h->blurredOffsetArray[1];
-    h->blurredOffsetArray[1] = t0;
-    uint32_t* m0 = h->flowMaxDev[0];
-    h->flowMaxDev[0] = h->flowMaxDev[1];
-    h->flowMaxDev[1] = m0;
-    rec.pending = true;
+    for (int k = 0; k < s.n; ++k) {
+        hrb_ofc* h = s.h[k];
+        hrb_ofc::FlowRecord& rec = h->flowRec[h->curRec];
+        if (s.n > 1) HRB_CUDA(cudaSetDevice(h->device));
+        HRB_CUDA(cudaMemcpyAsync(rec.rawDeltaHost, h->rawDeltaDev, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+        HRB_CUDA(cudaEventRecord(rec.end, h->stream));
+        int16_t* t0 = h->blurredOffsetArray[0];
+        h->blurredOffsetArray[0] = h->blurredOffsetArray[1];
+        h->blurredOffsetArray[1] = t0;
+        uint32_t* m0 = h->flowMaxDev[0];
+        h->flowMaxDev[0] = h->flowMaxDev[1];
+        h->flowMaxDev[1] = m0;
+        rec.pending = true;
+    }
     return HRB_OK;
 }
 
@@ -748,33 +911,52 @@ static int joinFlow(hrb_ofc* h) {
 // opticalFlowCalcSDR.cpp:113-123,150) and the search touches nothing the warp writes, so the calculation of source
 // frame N and the warps issued after it are independent: the asynchronous entry point runs the search ladder on its
 // own stream, forked behind everything already enqueued (the ingest of frame N, the last readers of the flow buffer
-// it overwrites) and joined before the next calculation — i.e. before any warp that needs its result.
+// it overwrites) and joined before the next calculation — i.e. before any warp that needs its result.  On a group
+// every shard makes this choice for itself, exactly as its own calculate_optical_flow_async would.
+static int calculateFlow(const Shards& s, bool async) {
+    for (int k = 0; k < s.n; ++k) {
+        const int rc = joinFlow(s.h[k]);
+        if (rc) return rc;
+    }
+    if (!async) {
+        int rc = enqueueFlow(s);
+        for (int k = 0; k < s.n && !rc; ++k) rc = resolveFlow(s.h[k]);
+        return rc;
+    }
+    cudaStream_t compute[kMaxShards];
+    bool forked[kMaxShards];
+    for (int k = 0; k < s.n; ++k) {
+        hrb_ofc* h = s.h[k];
+        forked[k] = h->flowOverlap && !h->tapMode && !h->prof.on;
+        compute[k] = h->stream;
+        if (!forked[k]) continue;
+        HRB_CUDA(cudaSetDevice(h->device));
+        HRB_CUDA(cudaEventRecord(h->flowForkEvent, h->stream));
+        HRB_CUDA(cudaStreamWaitEvent(h->flowStream, h->flowForkEvent, 0));
+        h->stream = h->flowStream;
+    }
+    const int rc = enqueueFlow(s);
+    for (int k = 0; k < s.n; ++k) s.h[k]->stream = compute[k];
+    if (rc) return rc;
+    for (int k = 0; k < s.n; ++k) {
+        hrb_ofc* h = s.h[k];
+        if (!forked[k]) continue;
+        if (s.n > 1) HRB_CUDA(cudaSetDevice(h->device));
+        HRB_CUDA(cudaEventRecord(h->flowJoinEvent, h->flowStream));
+        h->flowJoinPending = true;
+        h->updatesSinceFlow = 0;
+    }
+    return HRB_OK;
+}
+
 int hrb_ofc_calculate_optical_flow_async(hrb_ofc* h) {
     HRB_REQUIRE(h, "null handle");
-    int rc = joinFlow(h);
-    if (rc) return rc;
-    if (!h->flowOverlap || h->tapMode || h->prof.on) return enqueueFlow(h);
-    HRB_CUDA(cudaSetDevice(h->device));
-    HRB_CUDA(cudaEventRecord(h->flowForkEvent, h->stream));
-    HRB_CUDA(cudaStreamWaitEvent(h->flowStream, h->flowForkEvent, 0));
-    cudaStream_t compute = h->stream;
-    h->stream = h->flowStream;
-    rc = enqueueFlow(h);
-    h->stream = compute;
-    if (rc) return rc;
-    HRB_CUDA(cudaEventRecord(h->flowJoinEvent, h->flowStream));
-    h->flowJoinPending = true;
-    h->updatesSinceFlow = 0;
-    return HRB_OK;
+    return calculateFlow(Shards(h), true);
 }
 
 int hrb_ofc_calculate_optical_flow(hrb_ofc* h) {
     HRB_REQUIRE(h, "null handle");
-    int rc = joinFlow(h);
-    if (rc) return rc;
-    rc = enqueueFlow(h);
-    if (rc) return rc;
-    return resolveFlow(h);
+    return calculateFlow(Shards(h), false);
 }
 
 int hrb_ofc_warp_frames(hrb_ofc* h, float blending_scalar, int frame_output_mode) {
@@ -1211,6 +1393,133 @@ int hrb_ofc_debug_timeline_read(hrb_ofc* h, void* dst, size_t bytes) {
     HRB_CUDA(cudaDeviceSynchronize());
     HRB_CUDA(cudaMemcpy(dst, h->dbgDev, bytes, cudaMemcpyDeviceToHost));
     return HRB_OK;
+}
+
+// ---- split search ----------------------------------------------------------------------------------
+// b_k = 128 * round(k * lh / (n * 128)), b_0 = 0, b_n = lh; false when a stripe would be empty
+static bool planStripes(int lh, int n, int* b) {
+    if (n < 1 || n > kMaxShards || lh < 1) return false;
+    for (int k = 0; k < n; ++k) b[k] = kSplitAlign * (int)((2LL * k * lh + (long long)n * kSplitAlign) / (2LL * n * kSplitAlign));
+    b[n] = lh;
+    for (int k = 0; k < n; ++k)
+        if (b[k + 1] <= b[k]) return false;
+    return true;
+}
+
+// every shard must compute the flow shard 0 would: same geometry, format and search parameters
+static int checkShards(hrb_ofc* const* sh, int n, const char* fn) {
+    const hrb_ofc* a = sh[0];
+    for (int k = 1; k < n; ++k) {
+        const hrb_ofc* b = sh[k];
+        const char* f = a->frameWidth != b->frameWidth               ? "frame_width"
+                        : a->frameHeight != b->frameHeight           ? "frame_height"
+                        : a->hdr != b->hdr                           ? "is_hdr"
+                        : a->resScalar != b->resScalar               ? "res_scalar"
+                        : a->searchRadius != b->searchRadius         ? "search_radius"
+                        : a->deltaScalar != b->deltaScalar           ? "delta_scalar"
+                        : a->neighborBiasScalar != b->neighborBiasScalar ? "neighbor_bias_scalar"
+                        : a->searchVariant != b->searchVariant       ? "search_variant"
+                                                                     : nullptr;
+        if (f) {
+            setLastError("[hopperrender_b200] %s: shard %d differs from shard 0 in %s", fn, k, f);
+            return HRB_ERR_INVALID_ARG;
+        }
+    }
+    return HRB_OK;
+}
+
+int hrb_split_plan(int flow_height, int n, int* bounds) {
+    HRB_REQUIRE(bounds, "null argument");
+    std::vector<int> b((size_t)std::max(n, 0) + 1);
+    if (!planStripes(flow_height, n, b.data())) {
+        setLastError("[hopperrender_b200] hrb_split_plan: %d shards do not fit %d flow rows (1..%d shards, every stripe at least one row, bounds at multiples of %d)",
+                     n, flow_height, kMaxShards, kSplitAlign);
+        return HRB_ERR_INVALID_ARG;
+    }
+    memcpy(bounds, b.data(), b.size() * sizeof(int));
+    return HRB_OK;
+}
+
+int hrb_split_create(hrb_split** out, hrb_ofc* const* shards, int n) {
+    HRB_REQUIRE(out && shards, "null argument");
+    *out = nullptr;
+    HRB_REQUIRE(n >= 1 && n <= kMaxShards, "shard count outside 1..64");
+    for (int k = 0; k < n; ++k) {
+        HRB_REQUIRE(shards[k], "null handle");
+        for (int j = 0; j < k; ++j) HRB_REQUIRE(shards[j] != shards[k], "a handle appears twice");
+    }
+    int rc = checkShards(shards, n, "hrb_split_create");
+    if (rc) return rc;
+    std::vector<int> b((size_t)n + 1);
+    if (!planStripes(shards[0]->flowHeight, n, b.data())) {
+        setLastError("[hopperrender_b200] hrb_split_create: %d shards do not fit %d flow rows", n, shards[0]->flowHeight);
+        return HRB_ERR_INVALID_ARG;
+    }
+    // direct peer copies where the devices allow them (a context attribute; otherwise the copies are staged by the driver)
+    for (int i = 0; i < n; ++i)
+        for (int j = 0; j < n; ++j) {
+            const int di = shards[i]->device, dj = shards[j]->device;
+            int can = 0;
+            if (di == dj || cudaDeviceCanAccessPeer(&can, di, dj) != cudaSuccess || !can) continue;
+            HRB_CUDA(cudaSetDevice(di));
+            const cudaError_t e = cudaDeviceEnablePeerAccess(dj, 0);
+            if (e == cudaErrorPeerAccessAlreadyEnabled)
+                cudaGetLastError();
+            else
+                HRB_CUDA(e);
+        }
+    hrb_split* s = new (std::nothrow) hrb_split();
+    HRB_REQUIRE(s, "out of host memory");
+    s->shard.assign(shards, shards + n);
+    s->bounds = b;
+    s->done.assign((size_t)n, nullptr);
+    for (int k = 0; k < n; ++k) {
+        cudaError_t e = cudaSetDevice(shards[k]->device);
+        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->done[k], cudaEventDisableTiming);
+        if (e != cudaSuccess) {
+            setLastError("[hopperrender_b200] CUDA error %d (%s) in hrb_split_create", (int)e, cudaGetErrorString(e));
+            hrb_split_destroy(s);
+            return HRB_ERR_CUDA;
+        }
+    }
+    *out = s;
+    return HRB_OK;
+}
+
+void hrb_split_destroy(hrb_split* s) {
+    if (!s) return;
+    for (auto e : s->done)
+        if (e) cudaEventDestroy(e);
+    delete s;
+}
+
+int hrb_split_stripe(hrb_split* s, int shard, int* flow_row_begin, int* flow_row_end) {
+    HRB_REQUIRE(s && flow_row_begin && flow_row_end, "null argument");
+    HRB_REQUIRE(shard >= 0 && shard < (int)s->shard.size(), "shard out of range");
+    *flow_row_begin = s->bounds[shard];
+    *flow_row_end = s->bounds[shard + 1];
+    return HRB_OK;
+}
+
+static int splitCalculate(hrb_split* s, bool async, const char* fn) {
+    const int rc = checkShards(s->shard.data(), (int)s->shard.size(), fn);
+    if (rc) return rc;
+    for (hrb_ofc* h : s->shard)
+        if (h->prof.on || h->dbgDev) {
+            setLastError("[hopperrender_b200] %s: the profile and the debug timeline are not available on a grouped calculate (switch them off on every shard)", fn);
+            return HRB_ERR_STATE;
+        }
+    return calculateFlow(Shards(s), async);
+}
+
+int hrb_split_calculate_optical_flow(hrb_split* s) {
+    HRB_REQUIRE(s, "null handle");
+    return splitCalculate(s, false, "hrb_split_calculate_optical_flow");
+}
+
+int hrb_split_calculate_optical_flow_async(hrb_split* s) {
+    HRB_REQUIRE(s, "null handle");
+    return splitCalculate(s, true, "hrb_split_calculate_optical_flow_async");
 }
 
 uint64_t hrb_kernel_launch_count(void) { return g_launchCount.load(std::memory_order_relaxed); }

@@ -67,6 +67,10 @@ struct SearchArgs {
     int ws, wsLog2, iteration;
     int deltaScalar, neighborBiasScalar;
     int nWx, nWy, prevNWx;
+    // The pass computes (and writes sums, layers, offsets and taps of) only the windows whose flow rows lie in
+    // [rowBegin, rowEnd): [0, lh) for a lone handle, a shard's row stripe in the sharded passes of a split search
+    // (hrb_split).  Both bounds are multiples of kSplitAlign or lh, so no window straddles them.
+    int rowBegin, rowEnd;
     const int16_t* prevX;  // level i-1 offsets (nullptr at iteration 0: all zero)
     const int16_t* prevY;
     int16_t* curX;         // level i offsets: written by step 0, read by step 1
@@ -80,6 +84,20 @@ struct SearchArgs {
     size_t dbgWords;          // ... in a slice of this many words; CTAs whose record does not fit it record nothing
     bool winLanes;         // windows of 2 and 4: one lane per window (off: search variant 4, the butterfly form, for A/B runs)
 };
+
+// Row stripes of a split search start at multiples of this many flow rows: the u-extent of the tile kernel's CTA tile
+// (kernels_search_slide.cu).  X steps run on the transposed planes (u = y), so an X-step tile never straddles a stripe,
+// and a window of up to kSplitAlign rows lies inside one stripe.
+constexpr int kSplitAlign = 128;
+
+// The (u, v) range a pass covers, in the orientation of View (search_common.cuh): u in [u0, lu), v in [v0, lv).  The
+// flow rows [rowBegin, rowEnd) lie along v in Y steps (step 1) and along u in X steps (step 0, transposed planes).
+struct PassRange {
+    int u0, lu, v0, lv;
+};
+__host__ __device__ inline PassRange passRange(const SearchArgs& a, int step) {
+    return step == 1 ? PassRange{0, a.lw, a.rowBegin, a.rowEnd} : PassRange{a.rowBegin, a.rowEnd, 0, a.lw};
+}
 
 // The search representation of one input slot: 8-bit planes in both orientations, one allocation.
 struct SearchPlanes {

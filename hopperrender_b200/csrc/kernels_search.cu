@@ -33,8 +33,9 @@ template <int R, int STEP, bool WIDE> __global__ void __launch_bounds__(256) sad
         s_sums[tid >> 4][tid & 15] = 0;
         __syncthreads();
     }
-    const int cu = blockIdx.x * TILE + lane;
-    const int rowBase = blockIdx.y * TILE + warp * 4;
+    const int U0 = vw.u0 + blockIdx.x * TILE, V0 = vw.v0 + blockIdx.y * TILE;  // (u0, v0): multiples of kSplitAlign
+    const int cu = U0 + lane;
+    const int rowBase = V0 + warp * 4;
     const int gh = ws < 4 ? ws : 4;  // rows of one accumulation group (inside one window row)
     constexpr int LO = candOffset<R>(0), HI = candOffset<R>(R - 1);
 
@@ -114,7 +115,7 @@ template <int R, int STEP, bool WIDE> __global__ void __launch_bounds__(256) sad
             bfly<4>(acc, 4, b2);
             int z0 = (b0 ? 8 : 0) + (b1 ? 4 : 0) + (b2 ? 2 : 0);
             int lwin = 0;
-            if (ws <= TILE) lwin = ((cv0 - blockIdx.y * TILE) >> a.wsLog2) * (TILE >> a.wsLog2) + (lane >> a.wsLog2);
+            if (ws <= TILE) lwin = ((cv0 - V0) >> a.wsLog2) * (TILE >> a.wsLog2) + (lane >> a.wsLog2);
             if (ws == 8) {
                 atomicAdd(&s_sums[lwin][z0], acc[0]);
                 atomicAdd(&s_sums[lwin][z0 + 1], acc[1]);
@@ -136,16 +137,17 @@ template <int R, int STEP, bool WIDE> __global__ void __launch_bounds__(256) sad
         if (ws <= TILE) {
             const int perEdge = TILE >> a.wsLog2;
             if (tid < perEdge * perEdge) {
-                const int wu = blockIdx.x * perEdge + (tid % perEdge);
-                const int wv = blockIdx.y * perEdge + (tid / perEdge);
+                const int wu = (U0 >> a.wsLog2) + (tid % perEdge);
+                const int wv = (V0 >> a.wsLog2) + (tid / perEdge);
                 const int wx = View<STEP>::wx(wu, wv), wy = View<STEP>::wy(wu, wv);
-                if (wx < a.nWx && wy < a.nWy) finalizeWindow<R, STEP>(a, wx, wy, s_sums[tid]);
+                if ((wu << a.wsLog2) < vw.lu && (wv << a.wsLog2) < vw.lv) finalizeWindow<R, STEP>(a, wx, wy, s_sums[tid]);
             }
         } else {
             // the tile lies inside one window larger than the tile: add to the window's global sums; the CTA that
-            // arrives last (ticket) finds them complete, does the arg-min and leaves sums and ticket zeroed for the next pass
+            // arrives last (ticket) finds them complete, does the arg-min and leaves sums and ticket zeroed for the next pass.
+            // In a sharded pass every tile of an owned window lies inside the stripe, so the ticket count is unchanged.
             __shared__ bool s_last;
-            const int wu = (blockIdx.x * TILE) >> a.wsLog2, wv = (blockIdx.y * TILE) >> a.wsLog2;
+            const int wu = U0 >> a.wsLog2, wv = V0 >> a.wsLog2;
             const int wx = View<STEP>::wx(wu, wv), wy = View<STEP>::wy(wu, wv);
             const size_t w = (size_t)(wy * a.nWx + wx);
             if (tid < R) {
@@ -176,8 +178,8 @@ template <int R, int STEP, bool WIDE> __global__ void __launch_bounds__(256) sad
 
 template <int R> int launchPassR(hrb_ofc* h, const SearchArgs& a, int step, unsigned* launches) {
     const dim3 block(32, 8, 1);
-    const int lu = step == 1 ? a.lw : a.lh, lv = step == 1 ? a.lh : a.lw;  // X steps run on the transposed planes (View)
-    const dim3 grid((lu + TILE - 1) / TILE, (lv + TILE - 1) / TILE, 1);
+    const PassRange r = passRange(a, step);  // X steps run on the transposed planes (View)
+    const dim3 grid((r.lu - r.u0 + TILE - 1) / TILE, (r.lv - r.v0 + TILE - 1) / TILE, 1);
     bool done = false;
     if (a.rs == 0 && a.ws >= 4 && h->searchVariant != 1) {  // tile kernels on the planar planes (kernels_search_slide.cu), finalize fused
         const int rc = launchSearchPassSlide(h, a, R, step);

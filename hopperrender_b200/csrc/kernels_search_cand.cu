@@ -298,6 +298,10 @@ template <int R, int STEP, bool TAPS, int WS> __global__ void __launch_bounds__(
     const int lane = threadIdx.x, warp = threadIdx.y;
     const int tid = warp * 32 + lane;
     const int U0 = blockIdx.x * CT_U, V0 = blockIdx.y * CT_V;
+    // A sharded pass (split search) launches its grid from flow row 0 and the CTAs above the stripe return here: the tile
+    // origin stays plain blockIdx arithmetic, which this kernel (64 registers) cannot afford to keep an offset for.
+    // (u0, v0) is a multiple of 128, so the remaining tiles are exactly those of a grid started at the stripe.
+    if ((STEP == 1 ? V0 : U0) < a.rowBegin) return;  // CTA-uniform, before any barrier
 
     // windows of 2 and 4 on a full tile: frame-2 samples of the lane's first window, in flight while the tile is staged
     constexpr int WSW = WS <= 4 ? WS : 2;
@@ -414,6 +418,8 @@ template <int R, int STEP, bool TAPS, int WS> __global__ void __launch_bounds__(
         if (tid < nwu * nwv) {
             const int wu = (U0 >> wsLog2) + (tid % nwu), wv = (V0 >> wsLog2) + (tid / nwu);
             const int wx = View<STEP>::wx(wu, wv), wy = View<STEP>::wy(wu, wv);
+            // (tiles start at multiples of 32 / 128 from a stripe origin, a multiple of 128: a tile never crosses an
+            // interior stripe end, so the field bound is the stripe bound)
             if (wx < a.nWx && wy < a.nWy) finalizeWindow<R, STEP>(a, wx, wy, s_sums[tid]);
         }
     }
@@ -426,8 +432,8 @@ template <int R, int STEP, bool TAPS, int WS> int launchCandOne(hrb_ofc* h, cons
         HRB_CUDA(cudaFuncSetAttribute(sadCandKernel<R, STEP, TAPS, WS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)candSmem<WS>()));
         cfg.store(true, std::memory_order_release);
     }
-    const int lu = STEP == 1 ? a.lw : a.lh, lv = STEP == 1 ? a.lh : a.lw;
-    const dim3 grid((lu + CT_U - 1) / CT_U, (lv + CT_V - 1) / CT_V, 1);
+    const PassRange r = passRange(a, STEP);  // up to the end of the pass's rows: a stripe on a shard of a split search
+    const dim3 grid((r.lu + CT_U - 1) / CT_U, (r.lv + CT_V - 1) / CT_V, 1);
     sadCandKernel<R, STEP, TAPS, WS><<<grid, dim3(32, 8, 1), candSmem<WS>(), h->stream>>>(a);
     HRB_LAUNCH_CHECK();
     return HRB_OK;

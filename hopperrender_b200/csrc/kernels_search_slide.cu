@@ -29,6 +29,11 @@
 //   * windows up to 32 pixels are reduced and finalized inside the warp (butterfly over the window's lanes), 64-pixel
 //     windows inside the CTA, larger ones through R atomics per CTA into the per-window scratch: the last CTA of a
 //     window (arrival ticket) finalizes it.  No fills, no extra launch.
+//   * row stripes (split search, hrb_split): a sharded pass computes only the windows of flow rows [rowBegin, rowEnd).
+//     The grid starts at the stripe's first row (v in Y steps, u in X steps) and tiles that run past the stripe end are
+//     masked like tiles at the end of the field.  Borders stay frame-relative: a stripe edge inside the frame is not a
+//     mirror edge, the `border` test and the staging are unchanged there, and boxes read the rows beyond the stripe from
+//     the frame like any other rows.
 #include <cuda.h>
 
 #include <climits>
@@ -263,7 +268,7 @@ __global__ void __maxnreg__(128)
     const int lane = threadIdx.x, warp = threadIdx.y;
     const int NT = 32 * tp.nwv;
     const int tid = warp * 32 + lane;
-    const int U0 = blockIdx.x * 128, V0 = blockIdx.y * TV;
+    const int U0 = vw.u0 + blockIdx.x * 128, V0 = vw.v0 + blockIdx.y * TV;  // (u0, v0): multiples of kSplitAlign
     const int wsLog2 = WSC < 128 ? WSL : a.wsLog2;
     const int tileRows = min(TV, vw.lv - V0);            // flow rows of the tile that exist (> 0 by the grid)
     const int tileCols = min(128, vw.lu - U0);           // ... columns (a multiple of 4)
@@ -668,7 +673,9 @@ __global__ void __maxnreg__(128)
             }
         } else {
             // add the CTA's sums to the window's scratch; the LAST CTA to arrive (ticket) finds them complete, finalizes the
-            // window and leaves scratch and ticket zeroed for the next pass — no finalize kernel, no memset between passes
+            // window and leaves scratch and ticket zeroed for the next pass — no finalize kernel, no memset between passes.
+            // A sharded pass (split search) has windows of at most 128 rows here, and every CTA covering an owned window
+            // lies inside the stripe (tiles are 128 rows, stripes start at multiples of 128): the count is unchanged.
             const int wu = U0 >> wsLog2, wv = V0 >> wsLog2;
             const int wx = View<STEP>::wx(wu, wv), wy = View<STEP>::wy(wu, wv);
             const size_t widx = (size_t)(wy * a.nWx + wx);
@@ -826,7 +833,8 @@ template <int R, int WSC> int chooseWarps(const hrb_ofc* h, int lu, int lv) {
 
 template <int R, int STEP, int WSC> int launchTile(hrb_ofc* h, const SearchArgs& a) {
     using C = Cls<WSC>;
-    const int lu = STEP == 1 ? a.lw : a.lh, lv = STEP == 1 ? a.lh : a.lw;
+    const PassRange r = passRange(a, STEP);  // the pass's rows: a stripe on a shard of a split search
+    const int lu = r.lu - r.u0, lv = r.lv - r.v0;
     const int dimU = STEP == 1 ? a.W : a.H, dimV = STEP == 1 ? a.H : a.W;
     const uint8_t* y1 = STEP == 1 ? a.y1 : a.yT1;
     const uint8_t* c1 = STEP == 1 ? a.c1 : a.cT1;

@@ -33,18 +33,27 @@ __device__ __forceinline__ uint32_t sad4(uint32_t a, uint32_t b, uint32_t c) {
 // (u = y, v = x).  Both steps therefore run the same code and every warp access is a contiguous row segment.  In
 // either orientation the chroma bytes that belong to luma sample (v, u) are c[(v >> 1) * pitch + (u & ~1)] and + 1
 // (hrb_internal.cuh, SearchArgs).  Window bookkeeping (offset arrays, biases) stays in (x, y).
+//
+// The pass covers u in [u0, lu) and v in [v0, lv) (passRange): the whole flow field, or on a shard of a split search the
+// flow rows [rowBegin, rowEnd) — along v in Y steps, along u in X steps.  Grids start at (u0, v0) (the small-window
+// kernel's at 0: its CTAs before the stripe return at once); lu / lv bound the pixels and windows a CTA computes, so a
+// tile that runs past the stripe end is masked like one at the field's end.
+// Everything else stays frame-relative: dimU / dimV are the frame, a stripe edge inside the frame is NOT a mirror edge,
+// and staging reads the rows beyond a stripe edge from the frame like any other rows.
 template <int STEP> struct View {
     const uint8_t* __restrict__ y1;
     const uint8_t* __restrict__ c1;
     const uint8_t* __restrict__ y2;
     const uint8_t* __restrict__ c2;
-    int pitch, dimU, dimV, lu, lv;
+    int pitch, dimU, dimV, u0, lu, v0, lv;
     __device__ __forceinline__ explicit View(const SearchArgs& a) {
         if (STEP == 1) {
-            y1 = a.y1; c1 = a.c1; y2 = a.y2; c2 = a.c2; pitch = a.pitch; dimU = a.W; dimV = a.H; lu = a.lw; lv = a.lh;
+            y1 = a.y1; c1 = a.c1; y2 = a.y2; c2 = a.c2; pitch = a.pitch; dimU = a.W; dimV = a.H;
         } else {
-            y1 = a.yT1; c1 = a.cT1; y2 = a.yT2; c2 = a.cT2; pitch = a.pitchT; dimU = a.H; dimV = a.W; lu = a.lh; lv = a.lw;
+            y1 = a.yT1; c1 = a.cT1; y2 = a.yT2; c2 = a.cT2; pitch = a.pitchT; dimU = a.H; dimV = a.W;
         }
+        const PassRange r = passRange(a, STEP);
+        u0 = r.u0; lu = r.lu; v0 = r.v0; lv = r.lv;
     }
     static __device__ __forceinline__ int wx(int wu, int wv) { return STEP == 1 ? wu : wv; }
     static __device__ __forceinline__ int wy(int wu, int wv) { return STEP == 1 ? wv : wu; }

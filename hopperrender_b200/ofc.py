@@ -358,6 +358,60 @@ class OpticalFlowCalcHDR(OpticalFlowCalc):
     _is_hdr = True
 
 
+def split_plan(flowHeight, n):
+    """Flow-row bounds [b_0 .. b_n] of n shards of a split search (hrb_split_plan); needs no device."""
+    b = (C.c_int * (max(int(n), 0) + 1))()
+    rc = L.load().hrb_split_plan(int(flowHeight), int(n), b)
+    if rc != L.HRB_OK:
+        raise RuntimeError(f"hrb error {rc}: {L.last_error()}")
+    return list(b)
+
+
+class SplitSearch:
+    """A group of calculators (one per shard, usually one per GPU) that compute ONE flow together (hrb_split_*): shard k
+    searches the windows of its flow-row stripe, and afterwards every calculator holds exactly the flow a lone
+    calculateOpticalFlow would have computed, so warpFrames / setOutputStripe / downloadFrame work on each unchanged.
+    Every calculator must already hold both source frames (updateFrame / updateFrameDevice on each).  The group owns
+    nothing: close it before its calculators."""
+
+    def __init__(self, calcs):
+        self._lib = L.load()
+        self._calcs = list(calcs)  # keeps the handles alive as long as the group
+        self._s = C.c_void_p()
+        arr = (C.c_void_p * len(self._calcs))(*[c._h.value for c in self._calcs])
+        self._check(self._lib.hrb_split_create(C.byref(self._s), arr, len(self._calcs)))
+
+    def _check(self, rc):
+        if rc != L.HRB_OK:
+            raise RuntimeError(f"hrb error {rc}: {L.last_error()}")
+
+    def calculateOpticalFlow(self):
+        self._check(self._lib.hrb_split_calculate_optical_flow(self._s))
+
+    def calculateOpticalFlowAsync(self):
+        self._check(self._lib.hrb_split_calculate_optical_flow_async(self._s))
+
+    def stripe(self, k):
+        """(first flow row, end flow row) shard k owns."""
+        b, e = C.c_int(), C.c_int()
+        self._check(self._lib.hrb_split_stripe(self._s, int(k), C.byref(b), C.byref(e)))
+        return b.value, e.value
+
+    def __len__(self):
+        return len(self._calcs)
+
+    def close(self):
+        if getattr(self, "_s", None) is not None and self._s.value:
+            self._lib.hrb_split_destroy(self._s)
+            self._s = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def kernel_launch_count():
     return int(L.load().hrb_kernel_launch_count())
 

@@ -182,9 +182,47 @@ HRB_API int hrb_ofc_get_side_data(hrb_ofc* h, hrb_side_data* items, int capacity
 /* ---- spatial split of one stream over several GPUs ----------------------------------------------------------- */
 /* Restrict warp_frames / copy_frame / download_frame to the luma rows [row_begin, row_end) (even bounds) and the
  * chroma rows that belong to them.  Every GPU of the split holds the full source frames and the full flow (the
- * search is replicated, it is not the PCIe-bound part); each produces and downloads only its stripe, into the same
- * offsets of a full-frame host buffer.  Default: the whole frame. */
+ * search is replicated, it is not the PCIe-bound part, unless the handles form a split group, below); each produces and
+ * downloads only its stripe, into the same offsets of a full-frame host buffer.  Default: the whole frame. */
 HRB_API int hrb_ofc_set_output_stripe(hrb_ofc* h, int row_begin, int row_end);
+
+/* ---- split search: one flow computed by a group of handles ----------------------------------------------------- */
+/* A group of n handles ("shards", usually one per GPU; several may share a device) that together compute ONE flow.
+ * Shard k owns the flow rows [b_k, b_k+1), b_k = 128 * round(k * flow_height / (n * 128)), b_0 = 0, b_n = flow_height.
+ * The passes of the search ladder whose windows are at most 128 rows tall are sharded: each shard searches only the
+ * windows of its stripe, and between two such iterations it copies one parent-level window row above and one below its
+ * stripe from its neighbours (peer to peer between devices).  Passes with taller windows straddle stripes and run on
+ * every shard over the whole frame, as on a lone handle.  After the last iteration every shard receives the other
+ * shards' windows and blurs the whole field, so that afterwards EVERY handle of the group holds exactly the flow,
+ * flow peak, offset array and total_frame_delta a lone calculate_optical_flow on it would have produced, bit for bit:
+ * warp_frames, set_output_stripe and download_frame work on it unchanged.
+ *
+ * Preconditions: every handle already holds both full source frames (the caller runs update_frame /
+ * update_frame_device on each of them: the search reads frame 1 at unbounded offsets); the handles agree on frame size,
+ * is_hdr, res_scalar, search radius, delta / neighbour scalars and search variant (checked at create and at every
+ * calculate: HRB_ERR_INVALID_ARG naming the field).  Profile and debug timeline must be off on every shard
+ * (HRB_ERR_STATE otherwise).  Tap mode works: a shard records every pass; in a sharded pass only the window rows of its
+ * stripe are meaningful, and the sums and layer taps are zero elsewhere.
+ *
+ * The group owns nothing: a handle in a group remains a normal handle (its own calculate_optical_flow still runs the
+ * whole ladder), and the group must be destroyed before its handles.  Up to 64 shards. */
+typedef struct hrb_split hrb_split;
+/* The flow-row bounds bounds[0..n] of n shards for a flow of flow_height rows; needs no device.  HRB_ERR_INVALID_ARG for
+ * n < 1, n > 64 or an n that would leave a stripe empty. */
+HRB_API int hrb_split_plan(int flow_height, int n, int* bounds);
+/* Shard k of the group is shards[k] (distinct handles); the handles' streams must be usable from this thread. */
+HRB_API int hrb_split_create(hrb_split** out, hrb_ofc* const* shards, int n);
+HRB_API void hrb_split_destroy(hrb_split* s);
+/* the flow rows shard `shard` owns */
+HRB_API int hrb_split_stripe(hrb_split* s, int shard, int* flow_row_begin, int* flow_row_end);
+/* calculate_optical_flow on every shard at once: blocks until the flow is complete on all of them, and leaves each
+ * handle in the state its own calculate_optical_flow would (flow record, statistics, buffer swap). */
+HRB_API int hrb_split_calculate_optical_flow(hrb_split* s);
+/* calculate_optical_flow_async on every shard at once: each shard runs its part on its flow stream (flow overlap on) or
+ * its compute stream, forked and joined exactly as its own calculate_optical_flow_async would, so warp_frames issued
+ * afterwards reads the previous flow.  The shards order each other with events and copy with cudaMemcpyPeerAsync
+ * (cudaMemcpyAsync when two shards share a device); plain launches, no CUDA graph. */
+HRB_API int hrb_split_calculate_optical_flow_async(hrb_split* s);
 
 /* ---- test taps --------------------------------------------------------------------------------- */
 /* With tap mode on, calculate_optical_flow also records, per (iteration, step) pass: the window sums,
