@@ -175,7 +175,6 @@ static int issueIteration(hrb_ofc* h, int R, int ws, int iter, int prevNWx, int 
         const bool dbgPass = h->dbgDev && iter * 2 + step < 32;
         a.dbg = dbgPass ? h->dbgDev + (size_t)(iter * 2 + step) * h->dbgStride : nullptr;
         a.dbgWords = dbgPass ? h->dbgStride : 0;
-        a.winLanes = h->searchVariant != 4;
         if (h->tapMode) {
             PassTapDev t;
             t.g.windowSize = ws;

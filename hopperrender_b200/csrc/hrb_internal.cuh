@@ -6,6 +6,7 @@
 
 #include <atomic>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "hrb.h"
@@ -37,6 +38,28 @@ constexpr int HRB_MAX_DEVICES = 64;  // per-device launch configuration caches (
         ::hrb::t_launchCount++;                                                                          \
         HRB_CUDA(cudaGetLastError());                                                                    \
     } while (0)
+
+// f(std::integral_constant<int, v>()) for a run-time v in [LO, HI]: picks the template instance of a launcher.  Any other
+// v: HRB_ERR_STATE, with a message naming what and v.
+template <int LO, int HI, class F> int withConstant(const char* what, int v, const F& f) {
+    if (v == LO) return f(std::integral_constant<int, LO>());
+    if constexpr (LO < HI) {
+        return withConstant<LO + 1, HI>(what, v, f);
+    } else {
+        setLastError("[hopperrender_b200] %s %d: no such kernel instance", what, v);
+        return HRB_ERR_STATE;
+    }
+}
+
+// Raises Kernel's dynamic shared memory limit on the device to bytes, unless it already allows that much.
+template <auto Kernel> int allowDynamicSmem(int device, int bytes) {
+    static std::atomic<int> allowed[HRB_MAX_DEVICES];  // per device; handles may be created on several host threads
+    std::atomic<int>& cur = allowed[device & (HRB_MAX_DEVICES - 1)];
+    if (cur.load(std::memory_order_acquire) >= bytes) return HRB_OK;
+    HRB_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    cur.store(bytes, std::memory_order_release);
+    return HRB_OK;
+}
 
 // ------------------------------------------------------------------------------------------------
 // geometry of one search pass (one (iteration, step) of HopperRender/opticalFlowCalcSDR.cpp:72-107)
@@ -82,8 +105,18 @@ struct SearchArgs {
     uint8_t* tapLayer;     // optional [nWy][nWx]
     unsigned long long* dbg;  // optional per-CTA timeline of this pass (hrb_ofc_debug_timeline): 16 words per CTA ...
     size_t dbgWords;          // ... in a slice of this many words; CTAs whose record does not fit it record nothing
-    bool winLanes;         // windows of 2 and 4: one lane per window (off: search variant 4, the butterfly form, for A/B runs)
+    bool winLanes;         // small-window kernel: SearchPlan::winLanes, set by its launcher
 };
+
+// How one search pass runs.  planSearchPass (kernels_search.cu) is the one place that decides it, from the search variant
+// (hrb_ofc_set_search_variant) and the pass; the launchers launch what it says.
+struct SearchPlan {
+    enum Kernel { Generic, Cand, Tile } kernel;  // sadPassKernel, sadCandKernel, sadTileKernel
+    bool useTma;     // tile kernel: the chroma box by TMA (off: variant 2, cp.async only)
+    bool forceSlow;  // tile kernel: the per-pixel path for every window (variant 3)
+    bool winLanes;   // small-window kernel: one lane per window of 2 and 4 (off: variant 4, the butterfly form)
+};
+SearchPlan planSearchPass(int variant, const SearchArgs& a, int R, int step);
 
 // Row stripes of a split search start at multiples of this many flow rows: the u-extent of the tile kernel's CTA tile
 // (kernels_search_slide.cu).  X steps run on the transposed planes (u = y), so an X-step tile never straddles a stripe,
@@ -200,7 +233,7 @@ struct hrb_ofc {
     bool haveFlowLevels;
 
     // taps / profiling
-    int searchVariant;  // 0: automatic kernel selection, 1: generic sadPassKernel for every pass, 2: sliding kernel without TMA, 3: ... without the aligned fast path
+    int searchVariant;  // hrb_ofc_set_search_variant: the search kernels it selects are planned by planSearchPass
     int smCount;
     bool tapMode;
     // instantiated CUDA graphs of the flow calculation (search ladder + blur), one per combination of buffers and
@@ -235,23 +268,16 @@ int launchCopyFrame(hrb_ofc* h, int slot);
 int launchWarpFrames(hrb_ofc* h, int n, const float* t, uint8_t* const* out, int mode);
 // kernels_search.cu
 int launchSearchPass(hrb_ofc* h, const SearchArgs& a, int R, int step);
-// kernels_search_slide.cu: HRB_OK, an error code, or -1 when this (R, geometry) is not covered
-int launchSearchPassSlidePart0(hrb_ofc* h, const SearchArgs& a, int R, int step);  // R 5..8   (kernels_search_slide.cu, three builds)
-int launchSearchPassSlidePart1(hrb_ofc* h, const SearchArgs& a, int R, int step);  // R 9..12
-int launchSearchPassSlidePart2(hrb_ofc* h, const SearchArgs& a, int R, int step);  // R 13..16
-inline int launchSearchPassSlide(hrb_ofc* h, const SearchArgs& a, int R, int step) {
-    if (R < 5 || R > 16) return -1;
-    return R <= 8 ? launchSearchPassSlidePart0(h, a, R, step) : R <= 12 ? launchSearchPassSlidePart1(h, a, R, step) : launchSearchPassSlidePart2(h, a, R, step);
-}
+// The tile and small-window kernels exist for radii 5..16.  Each family is compiled as kSearchParts objects of four
+// consecutive radii (-DHRB_SEARCH_PART, Makefile), so that they build in parallel; radius R lives in part searchPart(R).
+constexpr int kSearchParts = 3;
+constexpr int searchPart(int R) { return (R - 5) / 4; }
+constexpr int firstRadiusOf(int part) { return 5 + 4 * part; }
+// A pass the plan sends to the tile kernel (kernels_search_slide.cu) / small-window kernel (kernels_search_cand.cu),
+// whose radius lies in PART.
+template <int PART> int launchTilePart(hrb_ofc* h, const SearchArgs& a, const SearchPlan& p, int R, int step);
+template <int PART> int launchCandPart(hrb_ofc* h, const SearchArgs& a, const SearchPlan& p, int R, int step);
 void freeTmaCache(hrb_ofc* h);  // tensor maps of the handle's search planes (kernels_search_slide.cu)
-// kernels_search_cand.cu: a whole pass for 2 <= ws <= 16 at full flow resolution; same return convention
-int launchSearchPassCandPart0(hrb_ofc* h, const SearchArgs& a, int R, int step);  // R 5..8   (kernels_search_cand.cu, three builds)
-int launchSearchPassCandPart1(hrb_ofc* h, const SearchArgs& a, int R, int step);  // R 9..12
-int launchSearchPassCandPart2(hrb_ofc* h, const SearchArgs& a, int R, int step);  // R 13..16
-inline int launchSearchPassCand(hrb_ofc* h, const SearchArgs& a, int R, int step) {
-    if (R < 5 || R > 16) return -1;
-    return R <= 8 ? launchSearchPassCandPart0(h, a, R, step) : R <= 12 ? launchSearchPassCandPart1(h, a, R, step) : launchSearchPassCandPart2(h, a, R, step);
-}
 int launchBlurFlow(hrb_ofc* h, const int16_t* lvlX, const int16_t* lvlY, int nWx, int wsLog2, int16_t* out, uint32_t* flowMax);
 int launchExpandOffsets(hrb_ofc* h, const int16_t* lvlX, int nWxX, int wsLog2X, const int16_t* lvlY, int nWxY, int wsLog2Y,
                         int16_t* out);

@@ -176,38 +176,24 @@ template <int R, int STEP, bool WIDE> __global__ void __launch_bounds__(256) sad
     }
 }
 
-template <int R> int launchPassR(hrb_ofc* h, const SearchArgs& a, int step, unsigned* launches) {
+// the generic kernel; windows larger than its tile are finalized by the last CTA of each window
+template <int R> int launchGeneric(hrb_ofc* h, const SearchArgs& a, int step) {
     const dim3 block(32, 8, 1);
     const PassRange r = passRange(a, step);  // X steps run on the transposed planes (View)
     const dim3 grid((r.lu - r.u0 + TILE - 1) / TILE, (r.lv - r.v0 + TILE - 1) / TILE, 1);
-    bool done = false;
-    if (a.rs == 0 && a.ws >= 4 && h->searchVariant != 1) {  // tile kernels on the planar planes (kernels_search_slide.cu), finalize fused
-        const int rc = launchSearchPassSlide(h, a, R, step);
-        if (rc > 0) return rc;
-        done = rc == HRB_OK;
+    const bool wide = grid.x * grid.y <= 2u * (unsigned)h->smCount;
+    if (step == 0) {
+        if (wide)
+            sadPassKernel<R, 0, true><<<grid, block, 0, h->stream>>>(a);
+        else
+            sadPassKernel<R, 0, false><<<grid, block, 0, h->stream>>>(a);
+    } else {
+        if (wide)
+            sadPassKernel<R, 1, true><<<grid, block, 0, h->stream>>>(a);
+        else
+            sadPassKernel<R, 1, false><<<grid, block, 0, h->stream>>>(a);
     }
-    if (!done && a.rs == 0 && a.ws <= 32 && h->searchVariant != 1) {  // staged small-window kernel (kernels_search_cand.cu): 2x2 windows
-        const int rc = launchSearchPassCand(h, a, R, step);
-        if (rc > 0) return rc;
-        done = rc == HRB_OK;
-    }
-    if (!done) {
-        // generic kernel; windows larger than its tile are finalized by the last CTA of each window
-        const bool wide = grid.x * grid.y <= 2u * (unsigned)h->smCount;
-        if (step == 0) {
-            if (wide)
-                sadPassKernel<R, 0, true><<<grid, block, 0, h->stream>>>(a);
-            else
-                sadPassKernel<R, 0, false><<<grid, block, 0, h->stream>>>(a);
-        } else {
-            if (wide)
-                sadPassKernel<R, 1, true><<<grid, block, 0, h->stream>>>(a);
-            else
-                sadPassKernel<R, 1, false><<<grid, block, 0, h->stream>>>(a);
-        }
-        HRB_LAUNCH_CHECK();
-    }
-    *launches = 1;
+    HRB_LAUNCH_CHECK();
     return HRB_OK;
 }
 
@@ -348,20 +334,39 @@ __global__ void __launch_bounds__(256) sadPeakKernel(uint32_t* out, uint32_t see
 
 }  // namespace
 
+SearchPlan planSearchPass(int variant, const SearchArgs& a, int R, int step) {
+    // The tile and small-window kernels run radii of 5 and more on full-resolution flows, on the planar planes; variant 1
+    // runs the generic kernel everywhere.  The tile kernel needs whole 4-pixel columns along u, over the whole field
+    // (also on a shard of a split search).  It covers windows of 4 and 8 too (variants 2 and 3 run it there, which is how
+    // the parity tests reach those classes), but the small-window kernel is faster on them and is the default.
+    const bool planar = R >= 5 && a.rs == 0 && variant != 1;
+    const int minWs = variant == 2 || variant == 3 ? 4 : 16;
+    const int lu = step == 1 ? a.lw : a.lh;
+    SearchPlan p;
+    p.kernel = planar && a.ws >= minWs && lu % 4 == 0 ? SearchPlan::Tile : planar && a.ws <= 32 ? SearchPlan::Cand : SearchPlan::Generic;
+    p.useTma = variant != 2;
+    p.forceSlow = variant == 3;
+    p.winLanes = variant != 4;
+    return p;
+}
+
 int launchSearchPass(hrb_ofc* h, const SearchArgs& a, int R, int step) {
-    unsigned launches = 0;
-    int rc = HRB_OK;
-    profBegin(h, CLS_SEARCH);
-    switch (R) {
-#define HRB_CASE(N) case N: rc = launchPassR<N>(h, a, step, &launches); break;
-        HRB_CASE(5) HRB_CASE(6) HRB_CASE(7) HRB_CASE(8) HRB_CASE(9) HRB_CASE(10) HRB_CASE(11) HRB_CASE(12) HRB_CASE(13) HRB_CASE(14)
-        HRB_CASE(15) HRB_CASE(16) HRB_CASE(2) HRB_CASE(3) HRB_CASE(4)
-#undef HRB_CASE
-        default:
-            setLastError("[hopperrender_b200] search radius %d outside 2..16", R);
-            return HRB_ERR_INVALID_ARG;
+    if (R < 2 || R > 16) {
+        setLastError("[hopperrender_b200] search radius %d outside 2..16", R);
+        return HRB_ERR_INVALID_ARG;
     }
-    profEnd(h, CLS_SEARCH, launches);
+    const SearchPlan p = planSearchPass(h->searchVariant, a, R, step);
+    profBegin(h, CLS_SEARCH);
+    int rc;
+    if (p.kernel == SearchPlan::Tile)
+        rc = withConstant<0, kSearchParts - 1>("tile kernel, search part", searchPart(R),
+                                               [&](auto part) { return launchTilePart<decltype(part)::value>(h, a, p, R, step); });
+    else if (p.kernel == SearchPlan::Cand)
+        rc = withConstant<0, kSearchParts - 1>("small-window kernel, search part", searchPart(R),
+                                               [&](auto part) { return launchCandPart<decltype(part)::value>(h, a, p, R, step); });
+    else
+        rc = withConstant<2, 16>("generic kernel, search radius", R, [&](auto r) { return launchGeneric<decltype(r)::value>(h, a, step); });
+    profEnd(h, CLS_SEARCH, rc == HRB_OK ? 1 : 0);
     return rc;
 }
 

@@ -426,12 +426,8 @@ template <int R, int STEP, bool TAPS, int WS> __global__ void __launch_bounds__(
 }
 
 template <int R, int STEP, bool TAPS, int WS> int launchCandOne(hrb_ofc* h, const SearchArgs& a) {
-    static std::atomic<bool> configured[HRB_MAX_DEVICES];  // the attribute is per device; handles may be created on several host threads
-    std::atomic<bool>& cfg = configured[h->device & (HRB_MAX_DEVICES - 1)];
-    if (!cfg.load(std::memory_order_acquire)) {
-        HRB_CUDA(cudaFuncSetAttribute(sadCandKernel<R, STEP, TAPS, WS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)candSmem<WS>()));
-        cfg.store(true, std::memory_order_release);
-    }
+    const int rc = allowDynamicSmem<sadCandKernel<R, STEP, TAPS, WS>>(h->device, (int)candSmem<WS>());
+    if (rc) return rc;
     const PassRange r = passRange(a, STEP);  // up to the end of the pass's rows: a stripe on a shard of a split search
     const dim3 grid((r.lu + CT_U - 1) / CT_U, (r.lv + CT_V - 1) / CT_V, 1);
     sadCandKernel<R, STEP, TAPS, WS><<<grid, dim3(32, 8, 1), candSmem<WS>(), h->stream>>>(a);
@@ -446,39 +442,25 @@ template <int R, int STEP, bool TAPS> int launchCandWs(hrb_ofc* h, const SearchA
         case 8: return launchCandOne<R, STEP, TAPS, 8>(h, a);
         case 16: return launchCandOne<R, STEP, TAPS, 16>(h, a);
         case 32: return launchCandOne<R, STEP, TAPS, 32>(h, a);
-        default: return -1;
     }
-}
-
-template <int R> int launchCandR(hrb_ofc* h, const SearchArgs& a, int step) {
-    const bool taps = a.tapSums || a.tapLayer || a.rawDelta;
-    if (step == 1) return taps ? launchCandWs<R, 1, true>(h, a) : launchCandWs<R, 1, false>(h, a);
-    return taps ? launchCandWs<R, 0, true>(h, a) : launchCandWs<R, 0, false>(h, a);
+    setLastError("[hopperrender_b200] small-window kernel, window size %d: no such kernel instance", a.ws);
+    return HRB_ERR_STATE;
 }
 
 }  // namespace
 
-// One whole pass (SAD + arg-min + offset update) for 2 <= ws <= 32 at full flow resolution.
-// The 12 search radii x 2 steps x 2 (taps) x 5 window sizes are 240 kernels: this file is compiled three times
-// (-DHRB_CAND_PART=0/1/2, see the Makefile), each part instantiating four radii, so the parts build in parallel.
-#ifndef HRB_CAND_PART
-#error "compile with -DHRB_CAND_PART=0, 1 or 2"
-#endif
-#define HRB_CAND_CONCAT2(a, b) a##b
-#define HRB_CAND_CONCAT(a, b) HRB_CAND_CONCAT2(a, b)
-int HRB_CAND_CONCAT(launchSearchPassCandPart, HRB_CAND_PART)(hrb_ofc* h, const SearchArgs& a, int R, int step) {
-    switch (R) {
-#define HRB_CASE(N) case N: return launchCandR<N>(h, a, step);
-#if HRB_CAND_PART == 0
-        HRB_CASE(5) HRB_CASE(6) HRB_CASE(7) HRB_CASE(8)
-#elif HRB_CAND_PART == 1
-        HRB_CASE(9) HRB_CASE(10) HRB_CASE(11) HRB_CASE(12)
-#else
-        HRB_CASE(13) HRB_CASE(14) HRB_CASE(15) HRB_CASE(16)
-#endif
-#undef HRB_CASE
-        default: return -1;
-    }
+// One whole pass (SAD + arg-min + offset update) for 2 <= ws <= 32 at full flow resolution, for the radii of part PART
+// (hrb_internal.cuh): the 12 search radii x 2 steps x 2 (taps) x 5 window sizes are 240 kernels.
+template <int PART> int launchCandPart(hrb_ofc* h, const SearchArgs& pass, const SearchPlan& p, int R, int step) {
+    SearchArgs a = pass;
+    a.winLanes = p.winLanes;
+    const bool taps = a.tapSums || a.tapLayer || a.rawDelta;
+    return withConstant<firstRadiusOf(PART), firstRadiusOf(PART) + 3>("small-window kernel, search radius", R, [&](auto r) {
+        constexpr int RC = decltype(r)::value;
+        if (step == 1) return taps ? launchCandWs<RC, 1, true>(h, a) : launchCandWs<RC, 1, false>(h, a);
+        return taps ? launchCandWs<RC, 0, true>(h, a) : launchCandWs<RC, 0, false>(h, a);
+    });
 }
+template int launchCandPart<HRB_SEARCH_PART>(hrb_ofc* h, const SearchArgs& pass, const SearchPlan& p, int R, int step);
 
 }  // namespace hrb

@@ -749,7 +749,7 @@ struct TmaCache {
     std::vector<Entry*> entries;
 };
 
-#if HRB_SLIDE_PART == 0
+#if HRB_SEARCH_PART == 0
 void freeTmaCache(hrb_ofc* h) {
     if (!h->tmaCache) return;
     for (auto* e : h->tmaCache->entries) delete e;
@@ -831,24 +831,19 @@ template <int R, int WSC> int chooseWarps(const hrb_ofc* h, int lu, int lv) {
     return best;
 }
 
-template <int R, int STEP, int WSC> int launchTile(hrb_ofc* h, const SearchArgs& a) {
+template <int R, int STEP, int WSC> int launchTile(hrb_ofc* h, const SearchArgs& a, const SearchPlan& p) {
     using C = Cls<WSC>;
     const PassRange r = passRange(a, STEP);  // the pass's rows: a stripe on a shard of a split search
     const int lu = r.lu - r.u0, lv = r.lv - r.v0;
     const int dimU = STEP == 1 ? a.W : a.H, dimV = STEP == 1 ? a.H : a.W;
-    const uint8_t* y1 = STEP == 1 ? a.y1 : a.yT1;
     const uint8_t* c1 = STEP == 1 ? a.c1 : a.cT1;
     const int pitch = STEP == 1 ? a.pitch : a.pitchT;
     TileParams tp = tileParams<R, WSC>(chooseWarps<R, WSC>(h, lu, lv));
-    tp.useTma = h->searchVariant != 2;
-    tp.forceSlow = h->searchVariant == 3;
+    tp.useTma = p.useTma;
+    tp.forceSlow = p.forceSlow;
     const int smem = tileSmem<WSC>(tp);
-    static std::atomic<int> configured[HRB_MAX_DEVICES];  // largest dynamic shared memory size set per device
-    std::atomic<int>& cfg = configured[h->device & (HRB_MAX_DEVICES - 1)];
-    if (cfg.load(std::memory_order_acquire) < smem) {
-        HRB_CUDA(cudaFuncSetAttribute(sadTileKernel<R, STEP, WSC>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        cfg.store(smem, std::memory_order_release);
-    }
+    const int rc = allowDynamicSmem<sadTileKernel<R, STEP, WSC>>(h->device, smem);
+    if (rc) return rc;
     const CUtensorMap* mC = tp.useTma ? tensorMapFor(h, c1, dimU, dimV / 2, pitch, C::BW, tp.boxHC) : nullptr;
     CUtensorMap dummy;
     memset(&dummy, 0, sizeof(dummy));
@@ -856,53 +851,34 @@ template <int R, int STEP, int WSC> int launchTile(hrb_ofc* h, const SearchArgs&
         tp.useTma = 0;
         mC = &dummy;
     }
-    (void)y1;
     const dim3 grid((lu + 127) / 128, (lv + 32 * tp.nwv - 1) / (32 * tp.nwv), 1);
     sadTileKernel<R, STEP, WSC><<<grid, dim3(32, tp.nwv, 1), smem, h->stream>>>(a, *mC, tp);
     HRB_LAUNCH_CHECK();
     return HRB_OK;
 }
 
-template <int R, int STEP> int launchTileStep(hrb_ofc* h, const SearchArgs& a) {
+template <int R, int STEP> int launchTileStep(hrb_ofc* h, const SearchArgs& a, const SearchPlan& p) {
     switch (a.ws) {
-        case 4: return launchTile<R, STEP, 4>(h, a);
-        case 8: return launchTile<R, STEP, 8>(h, a);
-        case 16: return launchTile<R, STEP, 16>(h, a);
-        case 32: return launchTile<R, STEP, 32>(h, a);
-        case 64: return launchTile<R, STEP, 64>(h, a);
-        default: return a.ws >= 128 ? launchTile<R, STEP, 128>(h, a) : -1;
+        case 4: return launchTile<R, STEP, 4>(h, a, p);
+        case 8: return launchTile<R, STEP, 8>(h, a, p);
+        case 16: return launchTile<R, STEP, 16>(h, a, p);
+        case 32: return launchTile<R, STEP, 32>(h, a, p);
+        case 64: return launchTile<R, STEP, 64>(h, a, p);
     }
+    if (a.ws >= 128) return launchTile<R, STEP, 128>(h, a, p);
+    setLastError("[hopperrender_b200] tile kernel, window size %d: no such kernel instance", a.ws);
+    return HRB_ERR_STATE;
 }
-
-template <int R> int launchTileR(hrb_ofc* h, const SearchArgs& a, int step) { return step == 1 ? launchTileStep<R, 1>(h, a) : launchTileStep<R, 0>(h, a); }
 
 }  // namespace
 
-// One whole pass for ws >= 4 at full flow resolution.  -1: this (R, geometry) is not covered here.
-// Compiled three times (-DHRB_SLIDE_PART=0/1/2), four search radii per part, so the parts build in parallel.
-#ifndef HRB_SLIDE_PART
-#error "compile with -DHRB_SLIDE_PART=0, 1 or 2"
-#endif
-#define HRB_SLIDE_CONCAT2(a, b) a##b
-#define HRB_SLIDE_CONCAT(a, b) HRB_SLIDE_CONCAT2(a, b)
-int HRB_SLIDE_CONCAT(launchSearchPassSlidePart, HRB_SLIDE_PART)(hrb_ofc* h, const SearchArgs& a, int R, int step) {
-    const int lu = step == 1 ? a.lw : a.lh;
-    // windows of 4 and 8 pixels: the tile kernel covers them (variants 2 and 3 run it there, which is how the parity tests reach
-    // those classes), but the staged small-window kernel (kernels_search_cand.cu) is faster on them and is the default
-    const int minWs = h->searchVariant >= 2 ? 4 : 16;
-    if (a.rs != 0 || a.ws < minWs || (lu & 3) != 0) return -1;
-    switch (R) {
-#define HRB_CASE(N) case N: return launchTileR<N>(h, a, step);
-#if HRB_SLIDE_PART == 0
-        HRB_CASE(5) HRB_CASE(6) HRB_CASE(7) HRB_CASE(8)
-#elif HRB_SLIDE_PART == 1
-        HRB_CASE(9) HRB_CASE(10) HRB_CASE(11) HRB_CASE(12)
-#else
-        HRB_CASE(13) HRB_CASE(14) HRB_CASE(15) HRB_CASE(16)
-#endif
-#undef HRB_CASE
-        default: return -1;  // not handled here
-    }
+// One whole pass for ws >= 4 at full flow resolution, for the radii of part PART (hrb_internal.cuh).
+template <int PART> int launchTilePart(hrb_ofc* h, const SearchArgs& a, const SearchPlan& p, int R, int step) {
+    return withConstant<firstRadiusOf(PART), firstRadiusOf(PART) + 3>("tile kernel, search radius", R, [&](auto r) {
+        constexpr int RC = decltype(r)::value;
+        return step == 1 ? launchTileStep<RC, 1>(h, a, p) : launchTileStep<RC, 0>(h, a, p);
+    });
 }
+template int launchTilePart<HRB_SEARCH_PART>(hrb_ofc* h, const SearchArgs& a, const SearchPlan& p, int R, int step);
 
 }  // namespace hrb

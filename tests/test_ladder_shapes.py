@@ -10,6 +10,7 @@ pins it to OracleCalc bit for bit; the GPU tests compare the CUDA path with it:
   * motion-mosaic content, whose blocks move independently by up to ~40 px, so that tile CTAs need 2..4 rounds and the
     per-pixel remainder (round 5, timeline word 7), and small-window CTAs fall back to unstaged fetches;
   * the production path of the same frames (no taps, no timeline, CUDA graph captured and replayed);
+  * the search variants that force kernels and staging paths: which passes run the tile kernel, read from the timeline;
   * the timeline's own bound: CTAs whose record does not fit the pass's slice leave no trace.
 """
 import numpy as np
@@ -134,9 +135,10 @@ def span_of(R):
 
 
 def expected_kernel(ws, lu, R, rs, variant=0):
-    """The kernel launchPassR (kernels_search.cu) picks for a pass: 'tile', 'cand' or 'generic'."""
+    """The kernel planSearchPass (kernels_search.cu) picks for a pass: 'tile', 'cand' or 'generic'.  lu: the whole
+    field's extent along u (flow width in Y steps, flow height in X steps)."""
     if R >= 5 and rs == 0 and variant != 1:
-        if ws >= (4 if variant >= 2 else 16) and lu % 4 == 0:
+        if ws >= (4 if variant in (2, 3) else 16) and lu % 4 == 0:
             return "tile"
         if ws <= 32:
             return "cand"
@@ -380,6 +382,26 @@ def test_timeline_records_only_what_fits_its_slice(synth):
     # the last tile pass overflows into the slice of the first small-window pass, which must stay zero
     last_tile = max(p for p, r in enumerate(recs) if r["kind"] == "tile")
     assert last_tile in over and recs[last_tile + 1]["kind"] == "cand", (over, last_tile)
+    g.close()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("W,H", [(320, 192), (322, 190)])   # flow sides multiples of 4 / 2 (mod 4)
+@pytest.mark.parametrize("variant", [2, 3, 4])
+def test_search_variant_kernels_pass_by_pass(synth, variant, W, H):
+    """Search variants 2 (tile kernel without TMA, from windows of 4), 3 (... per-pixel path forced) and 4 (like 0, with
+    the butterfly form at windows of 2 and 4): every pass equals the oracle, and the timeline shows the tile kernel on
+    exactly the passes expected_kernel gives it — none when the sides are 2 (mod 4)."""
+    R = 11
+    label = f"variant {variant} {W}x{H}"
+    fs = _frames(synth, W, H, False, 3, seed=variant)
+    g = _calc(False, H, W, 0, H, R)
+    for fr in fs:
+        g.updateFrame(fr)
+    lad = OracleLadder.of(fs, False, W, H, 0, H, R)
+    recs = compare_ladder(g, lad, label, timeline_words(lad.lw, lad.lh), variant)
+    kinds = {r["kind"] for r in recs}
+    assert kinds == ({"tile", "cand"} if W % 4 == 0 else {"cand", "generic"}), f"{label}: {kinds}"
     g.close()
 
 
