@@ -59,9 +59,13 @@ def _smooth_flow(lh, lw, rng, amp):
 @pytest.mark.parametrize("hdr", [False, True])
 @pytest.mark.parametrize("mode,variant", [(0, 0), (1, 0), (2, 0), (0, 1), (1, 1), (2, 1), (3, 0), (4, 0), (5, 0), (6, 0)])
 @pytest.mark.parametrize("W,H,maxres,inS,outS", [(64, 48, 270, 0, 0), (130, 70, 35, 136, 144), (256, 144, 36, 0, 320), (320, 176, 22, 0, 0),
-                                                 (200, 120, 270, 200, 204)])
+                                                 (200, 120, 270, 200, 204),
+                                                 # wide enough for interior items (test_warp_shapes.py): the lean form at
+                                                 # rs 1 with an odd flow width, at rs 0, and warpItem's INSIDE form (odd outS)
+                                                 (1030, 580, 290, 1094, 1062), (1024, 576, 576, 0, 1056), (1280, 720, 360, 1344, 1281)])
 def test_warp_modes(synth, hdr, mode, variant, W, H, maxres, inS, outS):
-    """All seven output modes; modes 0-2 through both the table-driven fast kernel (variant 0) and the generic one (1)."""
+    """All seven output modes over flows from zero to far beyond the rounding tables and blend scalars 0 .. 1.  The warp
+    does not read the search variant: the variant-1 rows check that setting it leaves modes 0-2 unchanged."""
     g, o = make_pair(hdr, H, W, inS, outS, black=4.0, white=250.0, maxres=maxres)
     g.setSearchVariant(variant)
     for fr in frames(synth, W, H, hdr, 3, inS or None):
@@ -462,20 +466,38 @@ def test_cpp_shim_replay_matches_python_replay_over_the_oracle(synth, hdr, tmp_p
     assert any(not i["warped"] and i["source"] >= 3 for i, _ in exp), "the scene cut should have forced a copyFrame"
 
 
+def lean_sample_masks(W, H):
+    """(luma [H][W], chroma pairs [H/2][W/2]): the samples a zero-flow warp of a full frame sends through the lean form."""
+    from test_warp_shapes import ITEM, LEAN, warp_item_maps
+    maps = warp_item_maps(W, H, W, H, 0, W, None, 0, None, [0.5], 2)
+    luma = np.repeat(maps[0][1] == LEAN, ITEM, axis=1)[:, :W]
+    pairs = np.repeat(maps[1][1] == LEAN, ITEM // 2, axis=1)[:, :W // 2]
+    return luma, pairs
+
+
 @pytest.mark.parametrize("black,white", [(0.0, 255.0), (16.0, 235.0), (3.5, 200.25), (0.0, 1.0), (100.0, 101.0), (250.0, 5.0)])
 def test_levels_exhaustive(black, white):
     """Level correction for every 16-bit (P010 container) and 8-bit input value, luma and chroma, against the oracle's
-    IEEE division — pins the hoisted-reciprocal division of the CUDA kernels (copy, warp) to correctly rounded results."""
-    for hdr in (True, False):
-        W, H = 512, 128 if hdr else 16
+    IEEE division — pins the hoisted-reciprocal division of the CUDA kernels (copy, warp) to correctly rounded results.
+    At 512 wide every warp item takes warpItem; at 2048 wide every value also passes the lean form's division (HDR) and
+    its level tables (SDR), in luma items and as both the U and the V sample of chroma pairs."""
+    for hdr, W, H in [(True, 512, 128), (False, 512, 16), (True, 2048, 176), (False, 2048, 16)]:
         g, o = make_pair(hdr, H, W, black=black, white=white)
         dt = np.uint16 if hdr else np.uint8
         nvals = 65536 if hdr else 256
         fr = np.zeros((H + H // 2) * W, dt)
         fr[:H * W] = np.arange(H * W) % nvals            # every value in the luma plane ...
         fr[H * W:] = (np.arange(H * W // 2) * 2 + np.arange(H * W // 2) % 2) % nvals  # ... and in both chroma channels
-        if hdr:
+        if hdr and W == 512:
             assert H * W >= nvals and H * W // 2 >= nvals // 2
+        if W == 2048:  # at 2048 wide the warp's lean form runs: lay every value out in its luma items and chroma pairs
+            lean_luma, lean_pairs = lean_sample_masks(W, H)
+            planes = fr.reshape(H + H // 2, W)
+            planes[:H][lean_luma] = np.arange(np.count_nonzero(lean_luma)) % nvals
+            pairs = planes[H:].reshape(H // 2, W // 2, 2)
+            pairs[lean_pairs] = (np.arange(np.count_nonzero(lean_pairs)) % nvals)[:, None]  # the same value as U and as V
+            assert np.unique(planes[:H][lean_luma]).size == nvals
+            assert np.unique(pairs[lean_pairs][:, 0]).size == np.unique(pairs[lean_pairs][:, 1]).size == nvals
         for _ in range(3):
             g.updateFrame(fr)
             o.updateFrame(fr)
