@@ -81,6 +81,10 @@ PROTOTYPES = {
     "hrb_split_stripe": (C.c_int, [_P, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "hrb_split_calculate_optical_flow": (C.c_int, [_P]),
     "hrb_split_calculate_optical_flow_async": (C.c_int, [_P]),
+    "hrb_flow_batch_create": (C.c_int, [C.POINTER(_P), C.POINTER(_P), C.c_int]),
+    "hrb_flow_batch_destroy": (None, [_P]),
+    "hrb_flow_batch_calculate_optical_flow": (C.c_int, [_P]),
+    "hrb_flow_batch_calculate_optical_flow_async": (C.c_int, [_P]),
     "hrb_ofc_set_tap_mode": (C.c_int, [_P, C.c_int]),
     "hrb_ofc_num_passes": (C.c_int, [_P, C.POINTER(C.c_int)]),
     "hrb_ofc_pass_info": (C.c_int, [_P, C.c_int] + [C.POINTER(C.c_int)] * 5),

@@ -136,10 +136,10 @@ static int resolveFlow(hrb_ofc* h) {
     return HRB_OK;
 }
 
-// One iteration (two passes) of the ladder on one handle; the passes compute the windows of flow rows [rowBegin, rowEnd).
-static int issueIteration(hrb_ofc* h, int R, int ws, int iter, int prevNWx, int prevNWy, int rowBegin, int rowEnd, bool issue) {
+// The arguments of pass (iter, step) of one handle, which computes the windows of flow rows [rowBegin, rowEnd), and the
+// pass's tap buffers when tap mode is on.
+static int beginPass(hrb_ofc* h, int R, int ws, int iter, int step, int prevNWx, int prevNWy, int rowBegin, int rowEnd, SearchArgs& a) {
     const int par = iter & 1;
-    SearchArgs a;
     memset(&a, 0, sizeof(a));
     const SearchPlanes& f1 = h->searchPlane[1];  // frame1 = m_inputFrameArray[1], opticalFlowCalcSDR.cpp:79
     const SearchPlanes& f2 = h->searchPlane[2];  // frame2 = m_inputFrameArray[2], opticalFlowCalcSDR.cpp:80
@@ -168,65 +168,74 @@ static int issueIteration(hrb_ofc* h, int R, int ws, int iter, int prevNWx, int 
     a.prevY = iter ? h->levelOffsets[par ^ 1][1] : nullptr;
     a.curX = h->levelOffsets[par][0];
     a.curY = h->levelOffsets[par][1];
-    for (int step = 0; step < 2; ++step) {
-        a.rawDelta = (iter == 0 && step == 0) ? h->rawDeltaDev : nullptr;
-        a.tapSums = nullptr;
-        a.tapLayer = nullptr;
-        const bool dbgPass = h->dbgDev && iter * 2 + step < 32;
-        a.dbg = dbgPass ? h->dbgDev + (size_t)(iter * 2 + step) * h->dbgStride : nullptr;
-        a.dbgWords = dbgPass ? h->dbgStride : 0;
-        if (h->tapMode) {
-            PassTapDev t;
-            t.g.windowSize = ws;
-            t.g.wsLog2 = a.wsLog2;
-            t.g.iteration = iter;
-            t.g.step = step;
-            t.g.nWx = a.nWx;
-            t.g.nWy = a.nWy;
-            t.g.prevNWx = prevNWx;
-            t.g.prevNWy = prevNWy;
-            const size_t nW = (size_t)a.nWx * a.nWy;
-            HRB_CUDA(cudaMalloc(&t.sums, nW * R * sizeof(uint32_t)));
-            HRB_CUDA(cudaMalloc(&t.layer, nW));
-            HRB_CUDA(cudaMalloc(&t.offX, nW * sizeof(int16_t)));
-            HRB_CUDA(cudaMalloc(&t.offY, nW * sizeof(int16_t)));
-            // zeroed, so that the windows a sharded pass does not compute read back as zero
-            HRB_CUDA(cudaMemsetAsync(t.sums, 0, nW * R * sizeof(uint32_t), h->stream));
-            HRB_CUDA(cudaMemsetAsync(t.layer, 0, nW, h->stream));
-            a.tapSums = t.sums;
-            a.tapLayer = t.layer;
-            h->taps.push_back(t);
-        }
-        if (issue) {
-            const int rc = launchSearchPass(h, a, R, step);
-            if (rc) return rc;
-        }
-        if (h->tapMode) {
-            PassTapDev& t = h->taps.back();
-            const size_t nW = (size_t)a.nWx * a.nWy;
-            HRB_CUDA(cudaMemcpyAsync(t.offX, a.curX, nW * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
-            t.wsX = ws;
-            t.nWxX = a.nWx;
-            t.nWyX = a.nWy;
-            if (step == 1) {
-                HRB_CUDA(cudaMemcpyAsync(t.offY, a.curY, nW * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
-                t.wsY = ws;
-                t.nWxY = a.nWx;
-                t.nWyY = a.nWy;
-            } else if (iter > 0) {
-                HRB_CUDA(cudaMemcpyAsync(t.offY, a.prevY, (size_t)prevNWx * prevNWy * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
-                t.wsY = ws * 2;
-                t.nWxY = prevNWx;
-                t.nWyY = prevNWy;
-            } else {
-                t.wsY = 0;  // all zero
-            }
+    a.rawDelta = (iter == 0 && step == 0) ? h->rawDeltaDev : nullptr;
+    const bool dbgPass = h->dbgDev && iter * 2 + step < 32;
+    a.dbg = dbgPass ? h->dbgDev + (size_t)(iter * 2 + step) * h->dbgStride : nullptr;
+    a.dbgWords = dbgPass ? h->dbgStride : 0;
+    if (h->tapMode) {
+        PassTapDev t;
+        t.g.windowSize = ws;
+        t.g.wsLog2 = a.wsLog2;
+        t.g.iteration = iter;
+        t.g.step = step;
+        t.g.nWx = a.nWx;
+        t.g.nWy = a.nWy;
+        t.g.prevNWx = prevNWx;
+        t.g.prevNWy = prevNWy;
+        const size_t nW = (size_t)a.nWx * a.nWy;
+        HRB_CUDA(cudaMalloc(&t.sums, nW * R * sizeof(uint32_t)));
+        HRB_CUDA(cudaMalloc(&t.layer, nW));
+        HRB_CUDA(cudaMalloc(&t.offX, nW * sizeof(int16_t)));
+        HRB_CUDA(cudaMalloc(&t.offY, nW * sizeof(int16_t)));
+        // zeroed, so that the windows a sharded pass does not compute read back as zero
+        HRB_CUDA(cudaMemsetAsync(t.sums, 0, nW * R * sizeof(uint32_t), h->stream));
+        HRB_CUDA(cudaMemsetAsync(t.layer, 0, nW, h->stream));
+        a.tapSums = t.sums;
+        a.tapLayer = t.layer;
+        h->taps.push_back(t);
+    }
+    return HRB_OK;
+}
+
+// After the pass: the tap snapshots of the offsets, and the geometry of the handle's newest level.
+static int endPass(hrb_ofc* h, const SearchArgs& a, int step, int prevNWx, int prevNWy) {
+    if (h->tapMode) {
+        PassTapDev& t = h->taps.back();
+        const size_t nW = (size_t)a.nWx * a.nWy;
+        HRB_CUDA(cudaMemcpyAsync(t.offX, a.curX, nW * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
+        t.wsX = a.ws;
+        t.nWxX = a.nWx;
+        t.nWyX = a.nWy;
+        if (step == 1) {
+            HRB_CUDA(cudaMemcpyAsync(t.offY, a.curY, nW * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
+            t.wsY = a.ws;
+            t.nWxY = a.nWx;
+            t.nWyY = a.nWy;
+        } else if (a.iteration > 0) {
+            HRB_CUDA(cudaMemcpyAsync(t.offY, a.prevY, (size_t)prevNWx * prevNWy * sizeof(int16_t), cudaMemcpyDeviceToDevice, h->stream));
+            t.wsY = a.ws * 2;
+            t.nWxY = prevNWx;
+            t.nWyY = prevNWy;
+        } else {
+            t.wsY = 0;  // all zero
         }
     }
-    h->lastIterParity = par;
+    h->lastIterParity = a.iteration & 1;
     h->lastNWx = a.nWx;
     h->lastNWy = a.nWy;
-    h->lastWs = ws;
+    h->lastWs = a.ws;
+    return HRB_OK;
+}
+
+// One iteration (two passes) of the ladder on one handle; the passes compute the windows of flow rows [rowBegin, rowEnd).
+static int issueIteration(hrb_ofc* h, int R, int ws, int iter, int prevNWx, int prevNWy, int rowBegin, int rowEnd, bool issue) {
+    for (int step = 0; step < 2; ++step) {
+        SearchArgs a;
+        int rc = beginPass(h, R, ws, iter, step, prevNWx, prevNWy, rowBegin, rowEnd, a);
+        if (!rc && issue) rc = launchSearchPass(h, a, R, step);
+        if (!rc) rc = endPass(h, a, step, prevNWx, prevNWy);
+        if (rc) return rc;
+    }
     return HRB_OK;
 }
 
@@ -240,18 +249,34 @@ struct hrb_split {
     std::vector<cudaEvent_t> done;    // per shard, created on its device: its part of an iteration / its pushes are enqueued
 };
 
+// The members of a flow batch (include/hrb.h): independent handles on one device whose passes are launched together.  It
+// owns no frame or flow memory, only the stream the ladder runs on, an event that marks the end of a batch on it, and
+// the launch arguments (kernel parameters, copied at each launch).
+struct hrb_flow_batch {
+    std::vector<hrb_ofc*> member;
+    int device = 0;
+    cudaStream_t stream = nullptr;
+    cudaEvent_t done = nullptr;
+    hrb::SearchBatch pass;
+    hrb::BlurBatch blur;
+};
+
 namespace hrb {
 
 constexpr int kMaxShards = 64;
 
-// The handles one ladder runs on: a lone handle (one shard that owns every flow row) or the shards of a group.
+// The handles one ladder runs on: a lone handle (one shard that owns every flow row), the shards of a group, or the
+// members of a flow batch (each computes its own flow over every row; their passes are launched together).
 struct Shards {
     hrb_ofc* const* h;
-    const int* bounds;   // n + 1 flow-row bounds
+    const int* bounds;   // n + 1 flow-row bounds (split group and lone handle)
     int n;
-    cudaEvent_t* done;   // n > 1 only
-    explicit Shards(hrb_ofc* lone) : h(&one), bounds(rows), n(1), done(nullptr), one(lone), rows{0, lone->flowHeight} {}
-    explicit Shards(hrb_split* s) : h(s->shard.data()), bounds(s->bounds.data()), n((int)s->shard.size()), done(s->done.data()), one(nullptr), rows{0, 0} {}
+    cudaEvent_t* done;   // split group only
+    hrb_flow_batch* batch;  // flow batch only: every h[k]->stream is its stream while the ladder is enqueued
+    explicit Shards(hrb_ofc* lone) : h(&one), bounds(rows), n(1), done(nullptr), batch(nullptr), one(lone), rows{0, lone->flowHeight} {}
+    explicit Shards(hrb_split* s)
+        : h(s->shard.data()), bounds(s->bounds.data()), n((int)s->shard.size()), done(s->done.data()), batch(nullptr), one(nullptr), rows{0, 0} {}
+    explicit Shards(hrb_flow_batch* b) : h(b->member.data()), bounds(nullptr), n((int)b->member.size()), done(nullptr), batch(b), one(nullptr), rows{0, 0} {}
     Shards(const Shards&) = delete;
     Shards& operator=(const Shards&) = delete;
 
@@ -344,7 +369,23 @@ static int gatherLevel(const Shards& s, int par, int ws, int nWx, int nWy, bool 
     return HRB_OK;
 }
 
-// The search ladder and the blur of one flow calculation, on a lone handle or on the shards of a group.  Passes with
+// One iteration of the ladder on every member of a flow batch: per step, the members' arguments, then one batched pass.
+static int issueBatchIteration(const Shards& s, int R, int ws, int iter, int prevNWx, int prevNWy) {
+    SearchBatch& b = s.batch->pass;
+    for (int step = 0; step < 2; ++step) {
+        for (int k = 0; k < s.n; ++k) {
+            const int rc = beginPass(s.h[k], R, ws, iter, step, prevNWx, prevNWy, 0, s.h[k]->flowHeight, b.m[k]);
+            if (rc) return rc;
+        }
+        int rc = launchSearchBatch(s.h, b, s.n, R, step);
+        for (int k = 0; k < s.n && !rc; ++k) rc = endPass(s.h[k], b.m[k], step, prevNWx, prevNWy);
+        if (rc) return rc;
+    }
+    return HRB_OK;
+}
+
+// The search ladder and the blur of one flow calculation, on a lone handle, on the shards of a group or on the members
+// of a flow batch.  Passes with
 // windows of at most kSplitAlign rows are sharded on a group: shard k computes only the windows of its rows, with
 // exchangeHalo between iterations and gatherLevel after the last one.  Passes with taller windows straddle stripes and
 // run replicated, on the whole frame, on every shard.  issue = false only replays the host-side bookkeeping (the
@@ -356,12 +397,16 @@ static int issueFlowKernels(const Shards& s, int R, int ws0, int iterations, boo
     for (int iter = 0; iter < iterations; ++iter) {
         const int ws = ws0 >> iter;
         const int par = iter & 1;
-        const bool sharded = s.n > 1 && ws <= kSplitAlign;
+        const bool sharded = !s.batch && s.n > 1 && ws <= kSplitAlign;
         if (sharded && prevSharded) {  // the first sharded iteration reads a parent level every shard computed in full
             const int rc = exchangeHalo(s, par ^ 1, ws * 2, prevNWx, prevNWy);
             if (rc) return rc;
         }
-        for (int k = 0; k < s.n; ++k) {
+        if (s.batch) {
+            const int rc = issueBatchIteration(s, R, ws, iter, prevNWx, prevNWy);
+            if (rc) return rc;
+        }
+        for (int k = 0; k < s.n && !s.batch; ++k) {
             hrb_ofc* h = s.h[k];
             if (s.n > 1) HRB_CUDA(cudaSetDevice(h->device));
             const int rc = issueIteration(h, R, ws, iter, prevNWx, prevNWy, sharded ? s.bounds[k] : 0, sharded ? s.bounds[k + 1] : lh, issue);
@@ -377,6 +422,15 @@ static int issueFlowKernels(const Shards& s, int R, int ws0, int iterations, boo
     }
 
     // blur into m_blurredOffsetArray[0], then swap (opticalFlowCalcSDR.cpp:113-123)
+    if (s.batch) {
+        BlurBatch& b = s.batch->blur;
+        for (int k = 0; k < s.n; ++k) {
+            hrb_ofc* h = s.h[k];
+            h->haveFlowLevels = true;
+            b.m[k] = BlurMember{h->levelOffsets[h->lastIterParity][0], h->levelOffsets[h->lastIterParity][1], h->blurredOffsetArray[0], h->flowMaxDev[0]};
+        }
+        return launchBlurFlowBatch(s.h, b, s.n, s.h[0]->lastNWx, ilog2(s.h[0]->lastWs));
+    }
     for (int k = 0; k < s.n; ++k) {
         hrb_ofc* h = s.h[k];
         h->haveFlowLevels = true;
@@ -482,8 +536,8 @@ static int enqueueFlow(const Shards& s) {
     }
 
     {
-        // a group runs plain launches: its ladder has cross-shard waits and copies between iterations
-        const int rc = s.n == 1 ? launchFlowKernels(h0, R, ws0, iterations) : issueFlowKernels(s, R, ws0, iterations, true);
+        // a group or a batch runs plain launches: a group's ladder has cross-shard waits and copies between iterations
+        const int rc = s.n == 1 && !s.batch ? launchFlowKernels(h0, R, ws0, iterations) : issueFlowKernels(s, R, ws0, iterations, true);
         if (rc) return rc;
     }
     for (int k = 0; k < s.n; ++k) {
@@ -1044,6 +1098,7 @@ int hrb_ofc_synchronize(hrb_ofc* h) {
     HRB_CUDA(cudaStreamSynchronize(h->flowStream));
     HRB_CUDA(cudaStreamSynchronize(h->stream));
     HRB_CUDA(cudaStreamSynchronize(h->downStream));
+    if (h->flowJoinPending) HRB_CUDA(cudaEventSynchronize(h->flowJoinEvent));  // a flow batch's stream
     h->flowJoinPending = false;
     return resolveFlow(h);
 }
@@ -1519,6 +1574,120 @@ int hrb_split_calculate_optical_flow(hrb_split* s) {
 int hrb_split_calculate_optical_flow_async(hrb_split* s) {
     HRB_REQUIRE(s, "null handle");
     return splitCalculate(s, true, "hrb_split_calculate_optical_flow_async");
+}
+
+// ---- flow batch ------------------------------------------------------------------------------------
+// the members' passes must be the same launches: same flow geometry, radius and kernel plan, on one device
+static int checkMembers(hrb_ofc* const* m, int n, const char* fn) {
+    const hrb_ofc* a = m[0];
+    for (int k = 1; k < n; ++k) {
+        const hrb_ofc* b = m[k];
+        const char* f = a->frameWidth != b->frameWidth           ? "frame_width"
+                        : a->frameHeight != b->frameHeight       ? "frame_height"
+                        : a->resScalar != b->resScalar           ? "res_scalar"
+                        : a->searchRadius != b->searchRadius     ? "search_radius"
+                        : a->searchVariant != b->searchVariant   ? "search_variant"
+                        : a->device != b->device                 ? "device"
+                                                                 : nullptr;
+        if (f) {
+            setLastError("[hopperrender_b200] %s: member %d differs from member 0 in %s", fn, k, f);
+            return HRB_ERR_INVALID_ARG;
+        }
+    }
+    return HRB_OK;
+}
+
+int hrb_flow_batch_create(hrb_flow_batch** out, hrb_ofc* const* members, int n) {
+    HRB_REQUIRE(out && members, "null argument");
+    *out = nullptr;
+    HRB_REQUIRE(n >= 1 && n <= HRB_FLOW_BATCH_MAX, "member count outside 1..64");
+    for (int k = 0; k < n; ++k) {
+        HRB_REQUIRE(members[k], "null handle");
+        for (int j = 0; j < k; ++j) HRB_REQUIRE(members[j] != members[k], "a handle appears twice");
+    }
+    const int rc = checkMembers(members, n, "hrb_flow_batch_create");
+    if (rc) return rc;
+    hrb_flow_batch* b = new (std::nothrow) hrb_flow_batch();
+    HRB_REQUIRE(b, "out of host memory");
+    b->member.assign(members, members + n);
+    b->device = members[0]->device;
+    int prioLow = 0, prioHigh = 0;
+    cudaError_t e = cudaSetDevice(b->device);
+    if (e == cudaSuccess) e = cudaDeviceGetStreamPriorityRange(&prioLow, &prioHigh);
+    if (e == cudaSuccess) e = cudaStreamCreateWithPriority(&b->stream, cudaStreamNonBlocking, prioHigh);  // as the members' flow streams
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->done, cudaEventDisableTiming);
+    if (e != cudaSuccess) {
+        setLastError("[hopperrender_b200] CUDA error %d (%s) in hrb_flow_batch_create", (int)e, cudaGetErrorString(e));
+        hrb_flow_batch_destroy(b);
+        return HRB_ERR_CUDA;
+    }
+    *out = b;
+    return HRB_OK;
+}
+
+void hrb_flow_batch_destroy(hrb_flow_batch* b) {
+    if (!b) return;
+    cudaSetDevice(b->device);
+    if (b->stream) {
+        cudaStreamSynchronize(b->stream);
+        cudaStreamDestroy(b->stream);
+    }
+    if (b->done) cudaEventDestroy(b->done);
+    delete b;
+}
+
+// The ladder of every member on the batch's stream, forked behind each member's compute stream.  A member that would
+// have forked on its own (asynchronous, flow overlap on, no taps) is joined through its flowJoinEvent like after its own
+// calculate_optical_flow_async; every other member's compute stream waits for the batch at once.
+static int batchCalculate(hrb_flow_batch* b, bool async, const char* fn) {
+    Shards s(b);
+    int rc = checkMembers(s.h, s.n, fn);
+    if (rc) return rc;
+    for (int k = 0; k < s.n; ++k)
+        if (s.h[k]->prof.on || s.h[k]->dbgDev) {
+            setLastError("[hopperrender_b200] %s: the profile and the debug timeline are not available on a batched calculate (switch them off on every member)", fn);
+            return HRB_ERR_STATE;
+        }
+    HRB_CUDA(cudaSetDevice(b->device));
+    cudaStream_t compute[HRB_FLOW_BATCH_MAX];
+    for (int k = 0; k < s.n; ++k) {
+        hrb_ofc* h = s.h[k];
+        rc = joinFlow(h);
+        if (rc) return rc;
+        // the ingest of the member's newest frame and the last readers of the flow buffer it overwrites
+        HRB_CUDA(cudaEventRecord(h->flowForkEvent, h->stream));
+        HRB_CUDA(cudaStreamWaitEvent(b->stream, h->flowForkEvent, 0));
+    }
+    for (int k = 0; k < s.n; ++k) {
+        compute[k] = s.h[k]->stream;
+        s.h[k]->stream = b->stream;
+    }
+    rc = enqueueFlow(s);
+    for (int k = 0; k < s.n; ++k) s.h[k]->stream = compute[k];
+    if (rc) return rc;
+    HRB_CUDA(cudaEventRecord(b->done, b->stream));
+    for (int k = 0; k < s.n; ++k) {
+        hrb_ofc* h = s.h[k];
+        if (async && h->flowOverlap && !h->tapMode) {
+            HRB_CUDA(cudaEventRecord(h->flowJoinEvent, b->stream));
+            h->flowJoinPending = true;
+            h->updatesSinceFlow = 0;
+        } else {
+            HRB_CUDA(cudaStreamWaitEvent(h->stream, b->done, 0));
+        }
+    }
+    for (int k = 0; k < s.n && !async && !rc; ++k) rc = resolveFlow(s.h[k]);
+    return rc;
+}
+
+int hrb_flow_batch_calculate_optical_flow(hrb_flow_batch* b) {
+    HRB_REQUIRE(b, "null handle");
+    return batchCalculate(b, false, "hrb_flow_batch_calculate_optical_flow");
+}
+
+int hrb_flow_batch_calculate_optical_flow_async(hrb_flow_batch* b) {
+    HRB_REQUIRE(b, "null handle");
+    return batchCalculate(b, true, "hrb_flow_batch_calculate_optical_flow_async");
 }
 
 uint64_t hrb_kernel_launch_count(void) { return g_launchCount.load(std::memory_order_relaxed); }

@@ -132,6 +132,25 @@ __host__ __device__ inline PassRange passRange(const SearchArgs& a, int step) {
     return step == 1 ? PassRange{0, a.lw, a.rowBegin, a.rowEnd} : PassRange{a.rowBegin, a.rowEnd, 0, a.lw};
 }
 
+// The arguments of one generic pass over the members of a flow batch (hrb_flow_batch): member k's are the ones its lone
+// pass would get.  Passed by value in kernel parameter space (__grid_constant__), so a pass needs no device table that
+// could be overwritten while an earlier batch is still in flight.
+struct SearchBatch {
+    SearchArgs m[HRB_FLOW_BATCH_MAX];
+};
+static_assert(sizeof(SearchBatch) <= 32764, "a full flow batch must fit the kernel parameter space of sm_100a (CUDA 12.1 and later)");
+
+// The flow blur of one member of a flow batch: the final level arrays, the blurred flow and its peak
+struct BlurMember {
+    const int16_t* lvlX;
+    const int16_t* lvlY;
+    int16_t* out;
+    uint32_t* flowMax;
+};
+struct BlurBatch {
+    BlurMember m[HRB_FLOW_BATCH_MAX];
+};
+
 // The search representation of one input slot: 8-bit planes in both orientations, one allocation.
 struct SearchPlanes {
     uint8_t* base = nullptr;   // the allocation
@@ -268,6 +287,9 @@ int launchCopyFrame(hrb_ofc* h, int slot);
 int launchWarpFrames(hrb_ofc* h, int n, const float* t, uint8_t* const* out, int mode);
 // kernels_search.cu
 int launchSearchPass(hrb_ofc* h, const SearchArgs& a, int R, int step);
+// One pass of the n members of a flow batch, on h[0]->stream: a generic pass is one launch over all of them, a tile or
+// small-window pass one launch per member.
+int launchSearchBatch(hrb_ofc* const* h, const SearchBatch& b, int n, int R, int step);
 // The tile and small-window kernels exist for radii 5..16.  Each family is compiled as kSearchParts objects of four
 // consecutive radii (-DHRB_SEARCH_PART, Makefile), so that they build in parallel; radius R lives in part searchPart(R).
 constexpr int kSearchParts = 3;
@@ -279,6 +301,8 @@ template <int PART> int launchTilePart(hrb_ofc* h, const SearchArgs& a, const Se
 template <int PART> int launchCandPart(hrb_ofc* h, const SearchArgs& a, const SearchPlan& p, int R, int step);
 void freeTmaCache(hrb_ofc* h);  // tensor maps of the handle's search planes (kernels_search_slide.cu)
 int launchBlurFlow(hrb_ofc* h, const int16_t* lvlX, const int16_t* lvlY, int nWx, int wsLog2, int16_t* out, uint32_t* flowMax);
+// the blur of the n members of a flow batch in one launch on h[0]->stream (zeroes each member's flowMax first)
+int launchBlurFlowBatch(hrb_ofc* const* h, const BlurBatch& b, int n, int nWx, int wsLog2);
 int launchExpandOffsets(hrb_ofc* h, const int16_t* lvlX, int nWxX, int wsLog2X, const int16_t* lvlY, int nWxY, int wsLog2Y,
                         int16_t* out);
 int microbenchSad(int device, double* gigaAbsdiffPerSec);

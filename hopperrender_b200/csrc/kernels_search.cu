@@ -22,7 +22,12 @@ namespace {
 // flow pixels in (u, v) coordinates (see View); a warp owns 4 consecutive v, a lane one u.  R is compile-time
 // so the candidate displacements fold into the address arithmetic.
 // ------------------------------------------------------------------------------------------------
-template <int R, int STEP, bool WIDE> __global__ void __launch_bounds__(256) sadPassKernel(const SearchArgs a) {
+// The arguments of the pass a CTA computes: a lone pass's, or those of member blockIdx.z of a flow batch (hrb_flow_batch)
+__device__ __forceinline__ const SearchArgs& passArgs(const SearchArgs& a) { return a; }
+__device__ __forceinline__ const SearchArgs& passArgs(const SearchBatch& b) { return b.m[blockIdx.z]; }
+
+template <int R, int STEP, bool WIDE, class P> __global__ void __launch_bounds__(256) sadPassKernel(const __grid_constant__ P p) {
+    const SearchArgs a = passArgs(p);  // a copy: the lone instances compile exactly as when a was the parameter itself
     __shared__ uint32_t s_sums[16][16];  // [window inside the tile][layer]
     const View<STEP> vw(a);
     const int lane = threadIdx.x, warp = threadIdx.y;
@@ -184,14 +189,35 @@ template <int R> int launchGeneric(hrb_ofc* h, const SearchArgs& a, int step) {
     const bool wide = grid.x * grid.y <= 2u * (unsigned)h->smCount;
     if (step == 0) {
         if (wide)
-            sadPassKernel<R, 0, true><<<grid, block, 0, h->stream>>>(a);
+            sadPassKernel<R, 0, true, SearchArgs><<<grid, block, 0, h->stream>>>(a);
         else
-            sadPassKernel<R, 0, false><<<grid, block, 0, h->stream>>>(a);
+            sadPassKernel<R, 0, false, SearchArgs><<<grid, block, 0, h->stream>>>(a);
     } else {
         if (wide)
-            sadPassKernel<R, 1, true><<<grid, block, 0, h->stream>>>(a);
+            sadPassKernel<R, 1, true, SearchArgs><<<grid, block, 0, h->stream>>>(a);
         else
-            sadPassKernel<R, 1, false><<<grid, block, 0, h->stream>>>(a);
+            sadPassKernel<R, 1, false, SearchArgs><<<grid, block, 0, h->stream>>>(a);
+    }
+    HRB_LAUNCH_CHECK();
+    return HRB_OK;
+}
+
+// one generic pass over the members of a flow batch: one launch, grid z = member
+template <int R> int launchGenericBatch(cudaStream_t st, int smCount, const SearchBatch& b, int n, int step) {
+    const dim3 block(32, 8, 1);
+    const PassRange r = passRange(b.m[0], step);
+    const dim3 grid((r.lu - r.u0 + TILE - 1) / TILE, (r.lv - r.v0 + TILE - 1) / TILE, (unsigned)n);
+    const bool wide = grid.x * grid.y * grid.z <= 2u * (unsigned)smCount;
+    if (step == 0) {
+        if (wide)
+            sadPassKernel<R, 0, true, SearchBatch><<<grid, block, 0, st>>>(b);
+        else
+            sadPassKernel<R, 0, false, SearchBatch><<<grid, block, 0, st>>>(b);
+    } else {
+        if (wide)
+            sadPassKernel<R, 1, true, SearchBatch><<<grid, block, 0, st>>>(b);
+        else
+            sadPassKernel<R, 1, false, SearchBatch><<<grid, block, 0, st>>>(b);
     }
     HRB_LAUNCH_CHECK();
     return HRB_OK;
@@ -210,11 +236,11 @@ __device__ __forceinline__ int mirrorBlur(int pos, int dim) {  // blurFlowKernel
 constexpr int BT = 32;          // outputs per tile edge
 constexpr int BIN = BT + 7;     // input rows / columns a tile needs
 
-__global__ void __launch_bounds__(256) blurFlowKernel(const int16_t* __restrict__ lvlX, const int16_t* __restrict__ lvlY, int nWx, int wsLog2,
-                                                     int16_t* __restrict__ out, int lw, int lh, uint32_t* __restrict__ flowMax) {
+// axis 0 blurs lvl into the X plane of out, axis 1 into the Y plane
+__device__ __forceinline__ void blurFlow(const int16_t* __restrict__ lvl, int axis, int nWx, int wsLog2, int16_t* __restrict__ out, int lw, int lh,
+                                         uint32_t* __restrict__ flowMax) {
     __shared__ int16_t s_in[BIN][BIN + 1];
     __shared__ int s_h[BIN][BT];
-    const int16_t* __restrict__ lvl = blockIdx.z == 0 ? lvlX : lvlY;
     const int X0 = blockIdx.x * BT, Y0 = blockIdx.y * BT;
     const int tid = threadIdx.y * 32 + threadIdx.x;
     for (int i = tid; i < BIN * BIN; i += 256) {
@@ -244,12 +270,24 @@ __global__ void __launch_bounds__(256) blurFlowKernel(const int16_t* __restrict_
 #pragma unroll
             for (int k = 0; k < 8; ++k) s += s_h[ly + k][threadIdx.x];
             const int v = s / 64;
-            out[(size_t)blockIdx.z * lw * lh + (size_t)y * lw + x] = (int16_t)v;
+            out[(size_t)axis * lw * lh + (size_t)y * lw + x] = (int16_t)v;
             peak = max(peak, abs(v));
         }
     }
     peak = __reduce_max_sync(0xffffffffu, peak);
     if (threadIdx.x == 0 && (uint32_t)peak > *reinterpret_cast<volatile uint32_t*>(flowMax)) atomicMax(flowMax, (uint32_t)peak);
+}
+
+__global__ void __launch_bounds__(256) blurFlowKernel(const int16_t* __restrict__ lvlX, const int16_t* __restrict__ lvlY, int nWx, int wsLog2,
+                                                     int16_t* __restrict__ out, int lw, int lh, uint32_t* __restrict__ flowMax) {
+    blurFlow(blockIdx.z == 0 ? lvlX : lvlY, blockIdx.z, nWx, wsLog2, out, lw, lh, flowMax);
+}
+
+// over the members of a flow batch: blockIdx.z = 2 * member + axis
+__global__ void __launch_bounds__(256) blurFlowBatchKernel(const __grid_constant__ BlurBatch b, int nWx, int wsLog2, int lw, int lh) {
+    const BlurMember& m = b.m[blockIdx.z >> 1];
+    const int axis = blockIdx.z & 1;
+    blurFlow(axis ? m.lvlY : m.lvlX, axis, nWx, wsLog2, m.out, lw, lh, m.flowMax);
 }
 
 // Fast path for the usual case — last pass at 2x2 windows, even flow dimensions.  The field is constant on aligned 2x2
@@ -262,11 +300,10 @@ constexpr int BC_W = 32, BC_H = 16;  // cells per tile -> 64 x 32 outputs
 __device__ __forceinline__ int mirrorCell(int c, int n) { return c < 0 ? -c - 1 : (c >= n ? 2 * n - c - 1 : c); }
 __device__ __forceinline__ int div64(int s) { return (s + ((s >> 31) & 63)) >> 6; }  // C division: truncates toward zero
 
-__global__ void __launch_bounds__(256) blurFlowCellKernel(const int16_t* __restrict__ lvlX, const int16_t* __restrict__ lvlY, int nCx, int nCy,
-                                                         int16_t* __restrict__ out, int lw, int lh, uint32_t* __restrict__ flowMax) {
+__device__ __forceinline__ void blurFlowCell(const int16_t* __restrict__ lvl, int axis, int nCx, int nCy, int16_t* __restrict__ out, int lw, int lh,
+                                             uint32_t* __restrict__ flowMax) {
     __shared__ int16_t s_in[BC_H + 4][BC_W + 4 + 2];
     __shared__ int s_he[BC_H + 4][BC_W], s_ho[BC_H + 4][BC_W];
-    const int16_t* __restrict__ lvl = blockIdx.z == 0 ? lvlX : lvlY;
     const int C0 = blockIdx.x * BC_W, R0 = blockIdx.y * BC_H;
     const int tid = threadIdx.y * 32 + threadIdx.x;
     for (int i = tid; i < (BC_H + 4) * (BC_W + 4); i += 256) {
@@ -286,7 +323,7 @@ __global__ void __launch_bounds__(256) blurFlowCellKernel(const int16_t* __restr
     int peak = 0;  // largest |flow| this thread wrote: bounds every displacement warpFrames can apply
     const int cx = C0 + threadIdx.x;
     if (cx < nCx) {
-        int16_t* __restrict__ o = out + (size_t)blockIdx.z * lw * lh;
+        int16_t* __restrict__ o = out + (size_t)axis * lw * lh;
 #pragma unroll
         for (int j = 0; j < 2; ++j) {
             const int r = threadIdx.y * 2 + j;
@@ -305,6 +342,17 @@ __global__ void __launch_bounds__(256) blurFlowCellKernel(const int16_t* __restr
     }
     peak = __reduce_max_sync(0xffffffffu, peak);
     if (threadIdx.x == 0 && (uint32_t)peak > *reinterpret_cast<volatile uint32_t*>(flowMax)) atomicMax(flowMax, (uint32_t)peak);
+}
+
+__global__ void __launch_bounds__(256) blurFlowCellKernel(const int16_t* __restrict__ lvlX, const int16_t* __restrict__ lvlY, int nCx, int nCy,
+                                                         int16_t* __restrict__ out, int lw, int lh, uint32_t* __restrict__ flowMax) {
+    blurFlowCell(blockIdx.z == 0 ? lvlX : lvlY, blockIdx.z, nCx, nCy, out, lw, lh, flowMax);
+}
+
+__global__ void __launch_bounds__(256) blurFlowCellBatchKernel(const __grid_constant__ BlurBatch b, int nCx, int nCy, int lw, int lh) {
+    const BlurMember& m = b.m[blockIdx.z >> 1];
+    const int axis = blockIdx.z & 1;
+    blurFlowCell(axis ? m.lvlY : m.lvlX, axis, nCx, nCy, m.out, lw, lh, m.flowMax);
 }
 
 // per-pixel offsetArray [2][lh][lw] from window-level arrays (test taps only)
@@ -350,12 +398,15 @@ SearchPlan planSearchPass(int variant, const SearchArgs& a, int R, int step) {
     return p;
 }
 
-int launchSearchPass(hrb_ofc* h, const SearchArgs& a, int R, int step) {
+static int checkRadius(int R) {
     if (R < 2 || R > 16) {
         setLastError("[hopperrender_b200] search radius %d outside 2..16", R);
         return HRB_ERR_INVALID_ARG;
     }
-    const SearchPlan p = planSearchPass(h->searchVariant, a, R, step);
+    return HRB_OK;
+}
+
+static int launchPlannedPass(hrb_ofc* h, const SearchArgs& a, const SearchPlan& p, int R, int step) {
     profBegin(h, CLS_SEARCH);
     int rc;
     if (p.kernel == SearchPlan::Tile)
@@ -367,6 +418,27 @@ int launchSearchPass(hrb_ofc* h, const SearchArgs& a, int R, int step) {
     else
         rc = withConstant<2, 16>("generic kernel, search radius", R, [&](auto r) { return launchGeneric<decltype(r)::value>(h, a, step); });
     profEnd(h, CLS_SEARCH, rc == HRB_OK ? 1 : 0);
+    return rc;
+}
+
+int launchSearchPass(hrb_ofc* h, const SearchArgs& a, int R, int step) {
+    const int rc = checkRadius(R);
+    if (rc) return rc;
+    return launchPlannedPass(h, a, planSearchPass(h->searchVariant, a, R, step), R, step);
+}
+
+int launchSearchBatch(hrb_ofc* const* h, const SearchBatch& b, int n, int R, int step) {
+    int rc = checkRadius(R);
+    if (rc) return rc;
+    // the plan depends only on the variant, the geometry, R and the step, on which the members agree
+    const SearchPlan p = planSearchPass(h[0]->searchVariant, b.m[0], R, step);
+    if (p.kernel != SearchPlan::Generic) {
+        for (int k = 0; k < n && !rc; ++k) rc = launchPlannedPass(h[k], b.m[k], p, R, step);
+        return rc;
+    }
+    rc = withConstant<2, 16>("generic kernel, search radius", R,
+                             [&](auto r) { return launchGenericBatch<decltype(r)::value>(h[0]->stream, h[0]->smCount, b, n, step); });
+    for (int k = 0; k < n && !rc; ++k) profEnd(h[k], CLS_SEARCH, 1);  // each member's pass ran in one launch
     return rc;
 }
 
@@ -383,6 +455,23 @@ int launchBlurFlow(hrb_ofc* h, const int16_t* lvlX, const int16_t* lvlY, int nWx
         blurFlowKernel<<<grid, block, 0, h->stream>>>(lvlX, lvlY, nWx, wsLog2, out, h->flowWidth, h->flowHeight, flowMax);
     HRB_LAUNCH_CHECK();
     profEnd(h, CLS_BLUR, 1);
+    return HRB_OK;
+}
+
+int launchBlurFlowBatch(hrb_ofc* const* h, const BlurBatch& b, int n, int nWx, int wsLog2) {
+    const dim3 block(32, 8, 1);
+    const hrb_ofc* h0 = h[0];
+    const int lw = h0->flowWidth, lh = h0->flowHeight;
+    for (int k = 0; k < n; ++k) HRB_CUDA(cudaMemsetAsync(b.m[k].flowMax, 0, sizeof(uint32_t), h0->stream));
+    if (wsLog2 == 1 && !(lw & 1) && !(lh & 1) && lw >= 8 && lh >= 8 && nWx == lw / 2 && h0->searchVariant != 1) {
+        const dim3 cgrid((lw / 2 + BC_W - 1) / BC_W, (lh / 2 + BC_H - 1) / BC_H, 2 * n);
+        blurFlowCellBatchKernel<<<cgrid, block, 0, h0->stream>>>(b, lw / 2, lh / 2, lw, lh);
+    } else {
+        const dim3 grid((lw + BT - 1) / BT, (lh + BT - 1) / BT, 2 * n);
+        blurFlowBatchKernel<<<grid, block, 0, h0->stream>>>(b, nWx, wsLog2, lw, lh);
+    }
+    HRB_LAUNCH_CHECK();
+    for (int k = 0; k < n; ++k) profEnd(h[k], CLS_BLUR, 1);
     return HRB_OK;
 }
 

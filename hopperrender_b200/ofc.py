@@ -412,6 +412,45 @@ class SplitSearch:
             pass
 
 
+class FlowBatch:
+    """The flows of many same-size streams, searched together on one GPU (hrb_flow_batch_*): every generic-kernel pass of
+    the ladder, and the blur, is one launch over all calculators.  Afterwards each calculator is in exactly the state its
+    own calculateOpticalFlow(Async) would have left it in.  The calculators must agree on frame size, res_scalar, search
+    radius, search variant and device; each must already hold its own two source frames.  The batch owns no frame or
+    flow memory: close it before its calculators."""
+
+    def __init__(self, calcs):
+        self._lib = L.load()
+        self._calcs = list(calcs)  # keeps the handles alive as long as the batch
+        self._b = C.c_void_p()
+        arr = (C.c_void_p * max(len(self._calcs), 1))(*[c._h.value for c in self._calcs])
+        self._check(self._lib.hrb_flow_batch_create(C.byref(self._b), arr, len(self._calcs)))
+
+    def _check(self, rc):
+        if rc != L.HRB_OK:
+            raise RuntimeError(f"hrb error {rc}: {L.last_error()}")
+
+    def calculateOpticalFlow(self):
+        self._check(self._lib.hrb_flow_batch_calculate_optical_flow(self._b))
+
+    def calculateOpticalFlowAsync(self):
+        self._check(self._lib.hrb_flow_batch_calculate_optical_flow_async(self._b))
+
+    def __len__(self):
+        return len(self._calcs)
+
+    def close(self):
+        if getattr(self, "_b", None) is not None and self._b.value:
+            self._lib.hrb_flow_batch_destroy(self._b)
+            self._b = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def kernel_launch_count():
     return int(L.load().hrb_kernel_launch_count())
 

@@ -224,6 +224,41 @@ HRB_API int hrb_split_calculate_optical_flow(hrb_split* s);
  * (cudaMemcpyAsync when two shards share a device); plain launches, no CUDA graph. */
 HRB_API int hrb_split_calculate_optical_flow_async(hrb_split* s);
 
+/* ---- flow batch: the flows of many same-size streams in one ladder --------------------------------------------- */
+/* A group of n independent handles ("members", one per stream) on one device whose flows are searched together: each
+ * pass of the search ladder that runs the generic kernel (every pass of a reduced-resolution flow) is ONE launch over all
+ * members, and so is the blur, so n short chains of small launches become one chain of launches n times larger.  Passes
+ * that run the tile or small-window kernel (full-resolution flows) run one launch per member, back to back.  Each member
+ * searches its own frames into its own flow: afterwards EVERY member is in exactly the state its own
+ * calculate_optical_flow(_async) would have left it in, bit for bit (offset array, both blurred flows after the swap,
+ * flow peaks, raw frame delta, total_frame_delta with its own SDR / HDR divisor, flow record and calc-time statistics,
+ * taps when its tap mode is on).
+ *
+ * The members must agree on frame width and height, res_scalar, search radius, search variant and device (checked at
+ * create and at every calculate: HRB_ERR_INVALID_ARG naming the field; callers whose streams differ in radius form one
+ * batch per radius).  They may differ in is_hdr, strides, delta / neighbour scalars, levels, max_calc_res (with equal
+ * res_scalar) and frame history.  n must be 1..HRB_FLOW_BATCH_MAX with distinct, non-null handles
+ * (HRB_ERR_INVALID_ARG).  Profile and debug timeline must be off on every member (HRB_ERR_STATE otherwise).
+ *
+ * The batch owns no frame or flow memory: a member remains a normal handle, and the batch must be destroyed before its
+ * members.  It owns one stream (at the priority of the flow streams) on which the ladder runs; plain launches, no CUDA
+ * graph. */
+typedef struct hrb_flow_batch hrb_flow_batch;
+#define HRB_FLOW_BATCH_MAX 64
+/* members[k] is member k; the members' streams must be usable from this thread */
+HRB_API int hrb_flow_batch_create(hrb_flow_batch** out, hrb_ofc* const* members, int n);
+/* waits for the batch's stream, then frees it */
+HRB_API void hrb_flow_batch_destroy(hrb_flow_batch* b);
+/* calculate_optical_flow on every member at once: blocks until every flow is complete, and leaves each member in the
+ * state its own calculate_optical_flow would (flow record, statistics, buffer swap). */
+HRB_API int hrb_flow_batch_calculate_optical_flow(hrb_flow_batch* b);
+/* calculate_optical_flow_async on every member at once.  The batch's stream waits for each member's compute stream (the
+ * ingest of its newest frame, the last readers of the flow buffer it overwrites).  A member with flow overlap on (and
+ * tap mode off) is joined the way its own asynchronous calculate joins it: warp_frames issued afterwards reads the
+ * previous flow, and the next calculate, join_flow or the third update_frame is ordered behind the batch.  Every other
+ * member's compute stream waits for the batch at once. */
+HRB_API int hrb_flow_batch_calculate_optical_flow_async(hrb_flow_batch* b);
+
 /* ---- test taps --------------------------------------------------------------------------------- */
 /* With tap mode on, calculate_optical_flow also records, per (iteration, step) pass: the window sums,
  * the winning layer per window and the offset field after the update.  Off by default (costs memory). */
