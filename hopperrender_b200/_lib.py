@@ -41,6 +41,10 @@ class hrb_ofc_profile(C.Structure):
                 ("n_warp", C.c_uint64), ("n_copy", C.c_uint64)]
 
 
+class hrb_frame_planes(C.Structure):
+    _fields_ = [("y", C.c_void_p), ("y_pitch_bytes", C.c_size_t), ("uv", C.c_void_p), ("uv_pitch_bytes", C.c_size_t)]
+
+
 class hrb_side_data(C.Structure):
     _fields_ = [("guid", C.c_uint8 * 16), ("data", C.c_void_p), ("bytes", C.c_size_t)]
 
@@ -70,6 +74,9 @@ PROTOTYPES = {
     "hrb_ofc_calculate_optical_flow_async": (C.c_int, [_P]),
     "hrb_ofc_synchronize": (C.c_int, [_P]),
     "hrb_ofc_stream": (C.c_int, [_P, C.POINTER(_P)]),
+    "hrb_ofc_update_frame_planes": (C.c_int, [_P, C.POINTER(hrb_frame_planes)]),
+    "hrb_ofc_warp_frames_to": (C.c_int, [_P, C.c_int, C.POINTER(C.c_float), C.c_int, C.POINTER(hrb_frame_planes)]),
+    "hrb_ofc_copy_frame_to": (C.c_int, [_P, C.POINTER(hrb_frame_planes)]),
     "hrb_host_register": (C.c_int, [_P, C.c_size_t]),
     "hrb_host_unregister": (C.c_int, [_P]),
     "hrb_host_alloc": (C.c_int, [C.POINTER(_P), C.c_size_t]),

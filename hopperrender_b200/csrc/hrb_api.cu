@@ -5,7 +5,10 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <mutex>
 #include <new>
+
+#include <cuda.h>
 
 #include "hrb_internal.cuh"
 
@@ -557,7 +560,8 @@ static int enqueueFlow(const Shards& s) {
     return HRB_OK;
 }
 
-static int finishUpdate(hrb_ofc* h) {
+// src: the caller's planes the ingest reads and copies into the new slot; null after an upload into slot [3]
+static int finishUpdate(hrb_ofc* h, const hrb_frame_planes* src) {
     // the new frame sits in slot [3]; rotate [0] <- [1] <- [2] <- [3], the old [0] becomes the next upload target
     // (same result as the reference's write-into-[0]-then-rotate, opticalFlowCalcSDR.cpp:20-26)
     auto rot = [](auto** v) {
@@ -582,7 +586,7 @@ static int finishUpdate(hrb_ofc* h) {
     // enqueued; the third update after it writes one of them and is ordered behind it.  The first two do not touch
     // them, so in the usual update / calculate alternation the ingest of frame N+1 runs beside the search of frame N.
     if (h->flowJoinPending && ++h->updatesSinceFlow >= 3) HRB_CUDA(cudaStreamWaitEvent(h->stream, h->flowJoinEvent, 0));
-    return launchPackFrame(h, 2);
+    return launchPackFrame(h, 2, src);
 }
 
 // `onStream`: the stream the frame copy will be enqueued on; the flow timer starts there (m_ofcStartedEvent is the
@@ -608,7 +612,7 @@ static int uploadFrame(hrb_ofc* h, const uint8_t* input_planes, bool wait) {
     HRB_CUDA(cudaMemcpyAsync(h->inputFrameArray[3], input_planes, h->inFrameBytes, cudaMemcpyHostToDevice, h->upStream));
     HRB_CUDA(cudaEventRecord(h->uploadDoneEvent, h->upStream));
     HRB_CUDA(cudaStreamWaitEvent(h->stream, h->uploadDoneEvent, 0));
-    rc = finishUpdate(h);
+    rc = finishUpdate(h, nullptr);
     if (rc) return rc;
     if (wait) HRB_CUDA(cudaEventSynchronize(h->uploadDoneEvent));  // the caller's buffer is free again; everything else continues asynchronously
     return HRB_OK;
@@ -644,6 +648,124 @@ static int beginOutput(hrb_ofc* h) {
     h->warpStartedValid = true;
     h->outView = h->outCur;
     return HRB_OK;
+}
+
+// Ring slot `slot` as two planes: luma rows, then the chroma rows (both pitches output_stride)
+static hrb_frame_planes ringPlanes(hrb_ofc* h, int slot) {
+    const size_t pitch = (size_t)h->outputStride * h->bpp;
+    uint8_t* base = h->outputRing[slot];
+    return hrb_frame_planes{base, pitch, base + (size_t)h->frameHeight * pitch, pitch};
+}
+
+// ---- checks of caller planes (hrb_frame_planes) ----
+typedef CUresult (*MemGetAddressRangeFn)(CUdeviceptr*, size_t*, CUdeviceptr);
+
+static MemGetAddressRangeFn memGetAddressRange() {
+    static std::once_flag once;
+    static MemGetAddressRangeFn fn = nullptr;
+    std::call_once(once, [] {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuMemGetAddressRange", &p, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+            fn = (MemGetAddressRangeFn)p;
+        cudaGetLastError();
+    });
+    return fn;
+}
+
+// The bytes [lo, hi) one plane of a frame covers
+struct PlaneSpan {
+    uintptr_t lo, hi;
+};
+
+// Checks one plane of `rows` rows (see include/hrb.h, "device frame planes"); the caller has made h's device current.
+// `fn` and `what` name the plane in the message.
+static int checkPlane(hrb_ofc* h, const void* ptr, size_t pitch, int rows, const char* fn, const char* what, PlaneSpan* span) {
+    auto fail = [&](const char* rule) {
+        setLastError("[hopperrender_b200] %s: %s plane %s", fn, what, rule);
+        return HRB_ERR_INVALID_ARG;
+    };
+    if (!ptr) return fail("is null");
+    const size_t bpp = (size_t)h->bpp, rowBytes = (size_t)h->frameWidth * bpp;
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, ptr) != cudaSuccess) {
+        cudaGetLastError();
+        return fail("is not device memory (cudaPointerGetAttributes failed)");
+    }
+    if (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged) return fail("is host memory: it must be device or managed memory of the handle's device");
+    if (attr.device != h->device) return fail("is memory of another device than the handle's");
+    if (pitch < rowBytes) return fail("pitch is below frame_width * bytes per sample");
+    if ((reinterpret_cast<uintptr_t>(ptr) % bpp) != 0 || (pitch % bpp) != 0) return fail("pointer and pitch must be multiples of the sample size");
+    const size_t extent = (size_t)(rows - 1) * pitch + rowBytes;
+    if (extent / bpp >= ((size_t)1 << 31)) return fail("extent exceeds 2^31 samples");
+    const MemGetAddressRangeFn range = memGetAddressRange();
+    if (!range) {
+        setLastError("[hopperrender_b200] %s: cuMemGetAddressRange is not available from the driver", fn);
+        return HRB_ERR_CUDA;
+    }
+    CUdeviceptr base = 0;
+    size_t size = 0;
+    if (range(&base, &size, (CUdeviceptr)reinterpret_cast<uintptr_t>(ptr)) != CUDA_SUCCESS) return fail("lies in no allocation (cuMemGetAddressRange failed)");
+    const uintptr_t lo = reinterpret_cast<uintptr_t>(ptr);
+    if (lo + extent > (uintptr_t)base + size) return fail("extent, (rows - 1) * pitch + frame_width * bytes per sample, runs past the end of its allocation");
+    *span = PlaneSpan{lo, lo + extent};
+    return HRB_OK;
+}
+
+// Checks the n frames f[0..n-1] (a source: n = 1, isDst false): each plane, every plane disjoint from every other, and
+// one pair of pitches for all.
+static int checkFrames(hrb_ofc* h, const hrb_frame_planes* f, int n, bool isDst, const char* fn) {
+    HRB_CUDA(cudaSetDevice(h->device));
+    PlaneSpan spans[2 * HRB_WARP_BATCH_MAX];
+    for (int i = 0; i < n; ++i) {
+        char what[2][32];
+        snprintf(what[0], sizeof what[0], n > 1 ? "dst[%d].y" : (isDst ? "dst.y" : "src.y"), i);
+        snprintf(what[1], sizeof what[1], n > 1 ? "dst[%d].uv" : (isDst ? "dst.uv" : "src.uv"), i);
+        int rc = checkPlane(h, f[i].y, f[i].y_pitch_bytes, h->frameHeight, fn, what[0], &spans[2 * i]);
+        if (!rc) rc = checkPlane(h, f[i].uv, f[i].uv_pitch_bytes, h->frameHeight / 2, fn, what[1], &spans[2 * i + 1]);
+        if (rc) return rc;
+        if (f[i].y_pitch_bytes != f[0].y_pitch_bytes || f[i].uv_pitch_bytes != f[0].uv_pitch_bytes) {
+            setLastError("[hopperrender_b200] %s: the destinations of one call must share one (y_pitch_bytes, uv_pitch_bytes); dst[%d] differs from dst[0]", fn, i);
+            return HRB_ERR_INVALID_ARG;
+        }
+    }
+    for (int a = 0; a < 2 * n; ++a)
+        for (int b = a + 1; b < 2 * n; ++b) {
+            if (spans[a].lo < spans[b].hi && spans[b].lo < spans[a].hi) {
+                if (a / 2 == b / 2)
+                    setLastError("[hopperrender_b200] %s: the Y and UV planes of frame %d overlap", fn, a / 2);
+                else
+                    setLastError("[hopperrender_b200] %s: the destinations dst[%d] and dst[%d] overlap", fn, a / 2, b / 2);
+                return HRB_ERR_INVALID_ARG;
+            }
+        }
+    return HRB_OK;
+}
+
+// warp_frames_batch's checks of the blend scalars and the mode
+static int checkWarpArgs(int n, const float* blending_scalars, int frame_output_mode, const char* fn) {
+    if (n < 1 || n > HRB_WARP_BATCH_MAX) {
+        setLastError("[hopperrender_b200] %s: batch size outside 1..HRB_WARP_BATCH_MAX", fn);
+        return HRB_ERR_INVALID_ARG;
+    }
+    for (int i = 0; i < n; ++i)
+        if (blending_scalars[i] > 1.0f) {  // opticalFlowCalcSDR.cpp:143-146
+            setLastError("[HopperRender] Error in function warpFrames: Blending scalar is greater than 1.0");
+            return HRB_ERR_BLEND_RANGE;
+        }
+    if (frame_output_mode < 0 || frame_output_mode > 6) {
+        setLastError("[hopperrender_b200] %s: frame_output_mode outside 0..6", fn);
+        return HRB_ERR_INVALID_ARG;
+    }
+    return HRB_OK;
+}
+
+static int updateFramePlanes(hrb_ofc* h, const hrb_frame_planes& src, const char* fn) {
+    int rc = checkFrames(h, &src, 1, false, fn);
+    if (rc) return rc;
+    rc = beginUpdate(h, h->stream);
+    if (rc) return rc;
+    return finishUpdate(h, &src);
 }
 
 }  // namespace hrb
@@ -944,10 +1066,14 @@ int hrb_ofc_wait_upload(hrb_ofc* h) {
 
 int hrb_ofc_update_frame_device(hrb_ofc* h, const void* device_planes) {
     HRB_REQUIRE(h && device_planes, "null argument");
-    int rc = beginUpdate(h, h->stream);
-    if (rc) return rc;
-    HRB_CUDA(cudaMemcpyAsync(h->inputFrameArray[3], device_planes, h->inFrameBytes, cudaMemcpyDeviceToDevice, h->stream));
-    return finishUpdate(h);
+    const size_t pitch = (size_t)h->inputStride * h->bpp;
+    uint8_t* base = static_cast<uint8_t*>(const_cast<void*>(device_planes));
+    return updateFramePlanes(h, hrb_frame_planes{base, pitch, base + (size_t)h->frameHeight * pitch, pitch}, __func__);
+}
+
+int hrb_ofc_update_frame_planes(hrb_ofc* h, const hrb_frame_planes* src) {
+    HRB_REQUIRE(h && src, "null argument");
+    return updateFramePlanes(h, *src, __func__);
 }
 
 // Orders the compute stream behind the last flow calculation that was enqueued on the flow stream.
@@ -1021,7 +1147,7 @@ int hrb_ofc_warp_frames(hrb_ofc* h, float blending_scalar, int frame_output_mode
     HRB_REQUIRE(frame_output_mode >= 0 && frame_output_mode <= 6, "frame_output_mode outside 0..6");
     int rc = beginOutput(h);
     if (rc) return rc;
-    uint8_t* out = h->outputRing[h->outCur];
+    const hrb_frame_planes out = ringPlanes(h, h->outCur);
     rc = launchWarpFrames(h, 1, &blending_scalar, &out, frame_output_mode);
     if (rc) return rc;
     HRB_CUDA(cudaEventRecord(h->outReady[h->outCur], h->stream));
@@ -1030,20 +1156,15 @@ int hrb_ofc_warp_frames(hrb_ofc* h, float blending_scalar, int frame_output_mode
 
 int hrb_ofc_warp_frames_batch(hrb_ofc* h, int n, const float* blending_scalars, int frame_output_mode) {
     HRB_REQUIRE(h && blending_scalars, "null argument");
-    HRB_REQUIRE(n >= 1 && n <= HRB_WARP_BATCH_MAX, "batch size outside 1..HRB_WARP_BATCH_MAX");
-    for (int i = 0; i < n; ++i)
-        if (blending_scalars[i] > 1.0f) {  // opticalFlowCalcSDR.cpp:143-146
-            setLastError("[HopperRender] Error in function warpFrames: Blending scalar is greater than 1.0");
-            return HRB_ERR_BLEND_RANGE;
-        }
-    HRB_REQUIRE(frame_output_mode >= 0 && frame_output_mode <= 6, "frame_output_mode outside 0..6");
-    int rc = beginOutput(h);  // waits for the download of the first slot, starts the warp timer
+    int rc = checkWarpArgs(n, blending_scalars, frame_output_mode, __func__);
     if (rc) return rc;
-    uint8_t* outs[HRB_WARP_BATCH_MAX];
+    rc = beginOutput(h);  // waits for the download of the first slot, starts the warp timer
+    if (rc) return rc;
+    hrb_frame_planes outs[HRB_WARP_BATCH_MAX];
     for (int i = 0; i < n; ++i) {
         const int slot = (h->outCur + i) % hrb_ofc::kOutRing;
         if (i) HRB_CUDA(cudaStreamWaitEvent(h->stream, h->outFree[slot], 0));
-        outs[i] = h->outputRing[slot];
+        outs[i] = ringPlanes(h, slot);
     }
     rc = launchWarpFrames(h, n, blending_scalars, outs, frame_output_mode);
     if (rc) return rc;
@@ -1056,10 +1177,28 @@ int hrb_ofc_copy_frame(hrb_ofc* h) {
     const int frameIndex = h->frameCount >= 3 ? 0 : h->frameCount >= 2 ? 1 : 2;  // opticalFlowCalcSDR.cpp:173
     int rc = beginOutput(h);
     if (rc) return rc;
-    rc = launchCopyFrame(h, frameIndex);
+    rc = launchCopyFrame(h, frameIndex, ringPlanes(h, h->outCur));
     if (rc) return rc;
     HRB_CUDA(cudaEventRecord(h->outReady[h->outCur], h->stream));
     return HRB_OK;
+}
+
+// The _to calls write the caller's planes on the compute stream and leave the ring, its cursor, its events and the warp
+// timer (warp_calc_time belongs to the ring's downloads) alone.
+int hrb_ofc_warp_frames_to(hrb_ofc* h, int n, const float* blending_scalars, int frame_output_mode, const hrb_frame_planes* dst) {
+    HRB_REQUIRE(h && blending_scalars && dst, "null argument");
+    int rc = checkWarpArgs(n, blending_scalars, frame_output_mode, __func__);
+    if (!rc) rc = checkFrames(h, dst, n, true, __func__);
+    if (rc) return rc;
+    return launchWarpFrames(h, n, blending_scalars, dst, frame_output_mode);
+}
+
+int hrb_ofc_copy_frame_to(hrb_ofc* h, const hrb_frame_planes* dst) {
+    HRB_REQUIRE(h && dst, "null argument");
+    const int rc = checkFrames(h, dst, 1, true, __func__);
+    if (rc) return rc;
+    const int frameIndex = h->frameCount >= 3 ? 0 : h->frameCount >= 2 ? 1 : 2;  // opticalFlowCalcSDR.cpp:173
+    return launchCopyFrame(h, frameIndex, *dst);
 }
 
 int hrb_ofc_download_frame(hrb_ofc* h, uint8_t* output_planes) {

@@ -282,9 +282,12 @@ struct hrb_ofc {
 namespace hrb {
 
 // kernels_frame.cu
-int launchPackFrame(hrb_ofc* h, int slot);
-int launchCopyFrame(hrb_ofc* h, int slot);
-int launchWarpFrames(hrb_ofc* h, int n, const float* t, uint8_t* const* out, int mode);
+// Ingest into input slot `slot`: src null packs the slot itself (filled by an upload); otherwise the pack reads the planes
+// of src and also writes their samples into the slot.
+int launchPackFrame(hrb_ofc* h, int slot, const hrb_frame_planes* src);
+// copyFrame / warpFrames into destination planes: a ring slot or a caller's surface (the warp's dst[i] share dst[0]'s pitches)
+int launchCopyFrame(hrb_ofc* h, int slot, const hrb_frame_planes& dst);
+int launchWarpFrames(hrb_ofc* h, int n, const float* t, const hrb_frame_planes* dst, int mode);
 // kernels_search.cu
 int launchSearchPass(hrb_ofc* h, const SearchArgs& a, int R, int step);
 // One pass of the n members of a flow batch, on h[0]->stream: a generic pass is one launch over all of them, a tile or

@@ -40,6 +40,27 @@ def _nbytes(a):
     return None
 
 
+def frame_planes(y, uv, height, width, hdr):
+    """hrb_frame_planes of a frame held as two CUDA tensors: y of shape (height, width), uv of shape (height / 2, width)
+    (interleaved U, V), uint8 for SDR, int16 or uint16 for HDR, unit inner stride; the row pitch is stride(0) times the
+    element size.  Raises before any device is touched; the library checks the memory itself."""
+    dtypes = ("torch.int16", "torch.uint16") if hdr else ("torch.uint8",)
+    for name, t, rows in (("y", y, height), ("uv", uv, height // 2)):
+        if not all(hasattr(t, a) for a in ("dtype", "is_cuda", "stride", "data_ptr")):
+            raise TypeError(f"plane {name}: a torch tensor is required, got {type(t).__name__}")
+        if tuple(t.shape) != (rows, width):
+            raise ValueError(f"plane {name}: shape {tuple(t.shape)}, ({rows}, {width}) needed")
+        if str(t.dtype) not in dtypes:
+            raise ValueError(f"plane {name}: dtype {t.dtype}, {' or '.join(dtypes)} needed for {'HDR' if hdr else 'SDR'}")
+        if t.stride(1) != 1:
+            raise ValueError(f"plane {name}: inner stride {t.stride(1)}, 1 needed")
+    for name, t in (("y", y), ("uv", uv)):
+        if not t.is_cuda:
+            raise ValueError(f"plane {name}: a CUDA tensor is required, got one on {t.device}")
+    es = 2 if hdr else 1
+    return L.hrb_frame_planes(y.data_ptr(), y.stride(0) * es, uv.data_ptr(), uv.stride(0) * es)
+
+
 class OpticalFlowCalc:
     """Abstract base (HopperRender/opticalFlowCalc.h:24-138).  Instantiate OpticalFlowCalcSDR / HDR."""
 
@@ -128,6 +149,28 @@ class OpticalFlowCalc:
 
     def calculateOpticalFlowAsync(self):
         self._check(self._lib.hrb_ofc_calculate_optical_flow_async(self._h))
+
+    def _planes(self, y, uv):
+        return frame_planes(y, uv, self._geom.frame_height, self._geom.frame_width, self._is_hdr)
+
+    def updateFramePlanes(self, y, uv):
+        """updateFrameDevice from two CUDA tensors, luma (H, W) and interleaved chroma (H/2, W), each with its own row pitch
+        (hrb_ofc_update_frame_planes).  They are read on streamHandle()."""
+        self._check(self._lib.hrb_ofc_update_frame_planes(self._h, C.byref(self._planes(y, uv))))
+
+    def warpFramesTo(self, blendingScalars, frameOutputMode, outs):
+        """warpFramesBatch into caller tensors: output frame i goes to outs[i] = (y, uv) (hrb_ofc_warp_frames_to); the
+        output ring is not touched.  The frames are ready for work ordered behind streamHandle()."""
+        if len(outs) != len(blendingScalars):
+            raise ValueError(f"{len(blendingScalars)} blending scalars but {len(outs)} destinations")
+        dst = (L.hrb_frame_planes * max(len(outs), 1))(*[self._planes(y, uv) for y, uv in outs])
+        arr = (C.c_float * max(len(blendingScalars), 1))(*[float(b) for b in blendingScalars])
+        self._check(self._lib.hrb_ofc_warp_frames_to(self._h, len(outs), arr, int(frameOutputMode), dst))
+
+    def copyFrameTo(self, out):
+        """copyFrame into a caller tensor pair (y, uv) (hrb_ofc_copy_frame_to)."""
+        y, uv = out
+        self._check(self._lib.hrb_ofc_copy_frame_to(self._h, C.byref(self._planes(y, uv))))
 
     def updateFrameAsync(self, pinnedInputPlanes):
         self._check(self._lib.hrb_ofc_update_frame_async(self._h, _ptr(pinnedInputPlanes)))

@@ -137,7 +137,9 @@ HRB_API int hrb_ofc_set_frame_count(hrb_ofc* h, unsigned int n);
 HRB_API int hrb_ofc_reset(hrb_ofc* h); /* == hrb_ofc_set_frame_count(h, 0) */
 
 /* ---- device-resident variants (benchmark / zero-copy callers) ---------------------------------- */
-/* Same as hrb_ofc_update_frame but the source is already in device memory of the handle's GPU. */
+/* Same as hrb_ofc_update_frame but the source is already in device memory of the handle's GPU.  It is
+ * hrb_ofc_update_frame_planes with y = device_planes, uv = device_planes + H * input_stride * bpp and both pitches
+ * input_stride * bpp bytes: the same checks apply and it is read on the compute stream. */
 HRB_API int hrb_ofc_update_frame_device(hrb_ofc* h, const void* device_planes);
 /* Device address of the output frame most recently written by warp_frames / copy_frame (for a batch: its first frame;
  * the frames of a batch sit in consecutive slots of a ring that advances with every download). */
@@ -163,6 +165,44 @@ HRB_API int hrb_host_register(void* ptr, size_t bytes);
 HRB_API int hrb_host_unregister(void* ptr);
 HRB_API int hrb_host_alloc(void** out, size_t bytes);
 HRB_API int hrb_host_free(void* ptr);
+
+/* ---- device frame planes ------------------------------------------------------------------------------------ */
+/* Source and destination frames as two planes in caller-owned memory on the handle's GPU, as hardware and CUDA decoders
+ * and encoders lay them out: the chroma plane is a pointer of its own (or sits at y + pitch * aligned_height), and the
+ * pitches are in BYTES.  bpp = 1 (NV12) or 2 (P010). */
+typedef struct hrb_frame_planes {
+    void*  y;          size_t y_pitch_bytes;   /* frame_height rows of frame_width samples */
+    void*  uv;         size_t uv_pitch_bytes;  /* frame_height/2 rows of frame_width interleaved U,V samples */
+} hrb_frame_planes;
+/* update_frame_device with the source described by two planes: the same input-slot rotation, frame_count, flow timer
+ * start and ordering behind a flow in flight.  The planes are read by one kernel on the compute stream (hrb_ofc_stream),
+ * which also fills the handle's own input slot (the warps read a frame for up to three source frames): the caller may
+ * overwrite or release the planes with work ordered behind that stream. */
+HRB_API int hrb_ofc_update_frame_planes(hrb_ofc* h, const hrb_frame_planes* src);
+/* warp_frames_batch into caller surfaces: output frame i goes to dst[i] (n in 1..HRB_WARP_BATCH_MAX) and is, bit for bit,
+ * the frame warp_frames_batch puts into ring slot i, in every mode.  The output stripe (set_output_stripe) applies: only
+ * its luma rows and their chroma rows are written.  No other byte of a destination is written: not the pitch padding,
+ * not the rows outside the stripe, not the gap between the planes.  Every destination of one call has the same
+ * (y_pitch_bytes, uv_pitch_bytes).  The warp's two-sample stores need every plane base and both pitches to be multiples of
+ * 2 * bpp bytes; otherwise every item takes the general form with scalar stores (same result, slower). */
+HRB_API int hrb_ofc_warp_frames_to(hrb_ofc* h, int n, const float* blending_scalars, int frame_output_mode, const hrb_frame_planes* dst);
+/* copy_frame into a caller surface, with the same stripe and byte rules as warp_frames_to. */
+HRB_API int hrb_ofc_copy_frame_to(hrb_ofc* h, const hrb_frame_planes* dst);
+/* The _to calls do not touch the output ring, its cursor or its events: download_frame and output_device_ptr keep
+ * referring to the last ring frame, and warp_calc_time stays what the ring path's downloads set.  Their results are
+ * visible to work ordered behind hrb_ofc_stream.
+ *
+ * Every plane is checked before anything is enqueued; a failure returns HRB_ERR_INVALID_ARG with a message naming the
+ * plane and the rule:
+ *   - the plane is not null;
+ *   - it is device or managed memory of the handle's device (cudaPointerGetAttributes): host memory, pageable or pinned,
+ *     and memory of another device are refused;
+ *   - its pitch is at least frame_width * bpp, and its pointer and pitch are multiples of bpp;
+ *   - its extent (rows - 1) * pitch + frame_width * bpp lies inside the allocation that holds it (cuMemGetAddressRange),
+ *     and below 2^31 samples;
+ *   - the Y and UV planes of a frame do not overlap, and the destinations of one call are pairwise disjoint.
+ * The blend scalars and the mode are checked as warp_frames_batch checks them (HRB_ERR_BLEND_RANGE for a scalar above 1,
+ * HRB_ERR_INVALID_ARG for a mode outside 0..6). */
 
 /* ---- side data of the source frames ----------------------------------------------------------------------------- */
 /* The filter reads the IMediaSideData blobs of the input sample (HDR10 / HDR10+ / Dolby Vision metadata and RPU, control
