@@ -45,6 +45,20 @@ class hrb_frame_planes(C.Structure):
     _fields_ = [("y", C.c_void_p), ("y_pitch_bytes", C.c_size_t), ("uv", C.c_void_p), ("uv_pitch_bytes", C.c_size_t)]
 
 
+class hrb_delivery_desc(C.Structure):
+    _fields_ = [("source_frame_time", C.c_longlong), ("target_frame_time", C.c_longlong), ("frame_output_mode", C.c_int),
+                ("scene_change_threshold", C.c_int), ("active", C.c_int), ("auto_adjust", C.c_int)]
+
+
+class hrb_delivery_frame(C.Structure):
+    _fields_ = [("source", C.c_uint), ("index", C.c_int), ("blend", C.c_double), ("step", C.c_ulonglong)]
+
+
+class hrb_delivery_outcome(C.Structure):
+    _fields_ = [("warped", C.c_int), ("scene_change", C.c_int), ("delta1", C.c_longlong), ("delta2", C.c_longlong),
+                ("frame_delta", C.c_uint)]
+
+
 class hrb_side_data(C.Structure):
     _fields_ = [("guid", C.c_uint8 * 16), ("data", C.c_void_p), ("bytes", C.c_size_t)]
 
@@ -81,6 +95,14 @@ PROTOTYPES = {
     "hrb_host_unregister": (C.c_int, [_P]),
     "hrb_host_alloc": (C.c_int, [C.POINTER(_P), C.c_size_t]),
     "hrb_host_free": (C.c_int, [_P]),
+    "hrb_delivery_create": (C.c_int, [C.POINTER(_P), _P, C.POINTER(hrb_delivery_desc)]),
+    "hrb_delivery_destroy": (None, [_P]),
+    "hrb_delivery_next_count": (C.c_int, [_P, C.POINTER(C.c_int)]),
+    "hrb_delivery_step": (C.c_int, [_P, C.POINTER(hrb_delivery_frame), C.c_int, C.POINTER(C.c_int)]),
+    "hrb_delivery_step_to": (C.c_int, [_P, C.POINTER(hrb_frame_planes), C.c_int, C.POINTER(hrb_delivery_frame), C.POINTER(C.c_int)]),
+    "hrb_delivery_outcome_of": (C.c_int, [_P, C.c_ulonglong, C.c_int, C.POINTER(hrb_delivery_outcome)]),
+    "hrb_delivery_set": (C.c_int, [_P, C.POINTER(hrb_delivery_desc)]),
+    "hrb_delivery_new_segment": (C.c_int, [_P, C.c_double]),
     "hrb_ofc_set_output_stripe": (C.c_int, [_P, C.c_int, C.c_int]),
     "hrb_split_plan": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_int)]),
     "hrb_split_create": (C.c_int, [C.POINTER(_P), C.POINTER(_P), C.c_int]),
@@ -116,6 +138,7 @@ PROTOTYPES = {
 
 HRB_OK, HRB_ERR_INVALID_ARG, HRB_ERR_CUDA, HRB_ERR_BLEND_RANGE, HRB_ERR_NO_DEVICE, HRB_ERR_STATE = range(6)
 TAP_WINDOW_SUMS, TAP_WINDOW_LAYER, TAP_OFFSETS = 0, 1, 2
+DELIVERY_MAX_FRAMES = 16
 BUF_OFFSET_ARRAY, BUF_FLOW_FOR_WARP, BUF_FLOW_LATEST, BUF_OUTPUT_FRAME, BUF_RAW_FRAME_DELTA, BUF_FLOW_PEAK = range(6)
 
 _lib = None

@@ -5,6 +5,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <deque>
 #include <mutex>
 #include <new>
 
@@ -230,12 +231,26 @@ static int endPass(hrb_ofc* h, const SearchArgs& a, int step, int prevNWx, int p
     return HRB_OK;
 }
 
+// After pass 0 of a handle with a delivery: rawDeltaDev holds the flow's raw frame delta.  Inside a graph capture the record
+// becomes an external event-record node, so that the delivery's decision kernel, on the compute stream, waits for pass 0
+// of the launched graph and not for the whole ladder.
+static int recordPass0(hrb_ofc* h) {
+    cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+    HRB_CUDA(cudaStreamIsCapturing(h->stream, &st));
+    if (st == cudaStreamCaptureStatusActive)
+        HRB_CUDA(cudaEventRecordWithFlags(h->pass0Event, h->stream, cudaEventRecordExternal));
+    else
+        HRB_CUDA(cudaEventRecord(h->pass0Event, h->stream));
+    return HRB_OK;
+}
+
 // One iteration (two passes) of the ladder on one handle; the passes compute the windows of flow rows [rowBegin, rowEnd).
 static int issueIteration(hrb_ofc* h, int R, int ws, int iter, int prevNWx, int prevNWy, int rowBegin, int rowEnd, bool issue) {
     for (int step = 0; step < 2; ++step) {
         SearchArgs a;
         int rc = beginPass(h, R, ws, iter, step, prevNWx, prevNWy, rowBegin, rowEnd, a);
         if (!rc && issue) rc = launchSearchPass(h, a, R, step);
+        if (!rc && issue && a.rawDelta && h->pass0Event) rc = recordPass0(h);
         if (!rc) rc = endPass(h, a, step, prevNWx, prevNWy);
         if (rc) return rc;
     }
@@ -465,10 +480,11 @@ static int launchFlowKernels(hrb_ofc* h, int R, int ws0, int iterations) {
     key.deltaScalar = h->deltaScalar;
     key.neighborBiasScalar = h->neighborBiasScalar;
     key.variant = h->searchVariant;
+    key.pass0 = h->pass0Event;
     hrb_ofc::FlowGraph* hit = nullptr;
     for (auto& g : h->flowGraphs)
         if (g.plane1 == key.plane1 && g.plane2 == key.plane2 && g.blurOut == key.blurOut && g.R == key.R && g.deltaScalar == key.deltaScalar &&
-            g.neighborBiasScalar == key.neighborBiasScalar && g.variant == key.variant)
+            g.neighborBiasScalar == key.neighborBiasScalar && g.variant == key.variant && g.pass0 == key.pass0)
             hit = &g;
     if (!hit) {
         if (h->flowGraphs.size() >= 64) dropFlowGraphs(h);  // 12 radii x 4 slot rotations fit; beyond that parameters keep changing (UI): start over
@@ -716,7 +732,7 @@ static int checkPlane(hrb_ofc* h, const void* ptr, size_t pitch, int rows, const
 // one pair of pitches for all.
 static int checkFrames(hrb_ofc* h, const hrb_frame_planes* f, int n, bool isDst, const char* fn) {
     HRB_CUDA(cudaSetDevice(h->device));
-    PlaneSpan spans[2 * HRB_WARP_BATCH_MAX];
+    PlaneSpan spans[2 * HRB_DELIVERY_MAX_FRAMES];
     for (int i = 0; i < n; ++i) {
         char what[2][32];
         snprintf(what[0], sizeof what[0], n > 1 ? "dst[%d].y" : (isDst ? "dst.y" : "src.y"), i);
@@ -771,6 +787,13 @@ static int updateFramePlanes(hrb_ofc* h, const hrb_frame_planes& src, const char
 }  // namespace hrb
 
 using namespace hrb;
+
+// The calls a delivery takes over (include/hrb.h, "delivery loop") refuse while one is attached.
+static bool delivering(hrb_ofc* h, const char* fn) {
+    if (!h->delivery) return false;
+    setLastError("[hopperrender_b200] %s: the handle has a delivery attached (hrb_delivery_destroy it first)", fn);
+    return true;
+}
 
 #define HRB_REQUIRE(cond, msg)                                       \
     do {                                                             \
@@ -1130,16 +1153,19 @@ static int calculateFlow(const Shards& s, bool async) {
 
 int hrb_ofc_calculate_optical_flow_async(hrb_ofc* h) {
     HRB_REQUIRE(h, "null handle");
+    if (delivering(h, __func__)) return HRB_ERR_STATE;
     return calculateFlow(Shards(h), true);
 }
 
 int hrb_ofc_calculate_optical_flow(hrb_ofc* h) {
     HRB_REQUIRE(h, "null handle");
+    if (delivering(h, __func__)) return HRB_ERR_STATE;
     return calculateFlow(Shards(h), false);
 }
 
 int hrb_ofc_warp_frames(hrb_ofc* h, float blending_scalar, int frame_output_mode) {
     HRB_REQUIRE(h, "null handle");
+    if (delivering(h, __func__)) return HRB_ERR_STATE;
     if (blending_scalar > 1.0f) {  // opticalFlowCalcSDR.cpp:143-146
         setLastError("[HopperRender] Error in function warpFrames: Blending scalar is greater than 1.0");
         return HRB_ERR_BLEND_RANGE;
@@ -1156,6 +1182,7 @@ int hrb_ofc_warp_frames(hrb_ofc* h, float blending_scalar, int frame_output_mode
 
 int hrb_ofc_warp_frames_batch(hrb_ofc* h, int n, const float* blending_scalars, int frame_output_mode) {
     HRB_REQUIRE(h && blending_scalars, "null argument");
+    if (delivering(h, __func__)) return HRB_ERR_STATE;
     int rc = checkWarpArgs(n, blending_scalars, frame_output_mode, __func__);
     if (rc) return rc;
     rc = beginOutput(h);  // waits for the download of the first slot, starts the warp timer
@@ -1174,10 +1201,12 @@ int hrb_ofc_warp_frames_batch(hrb_ofc* h, int n, const float* blending_scalars, 
 
 int hrb_ofc_copy_frame(hrb_ofc* h) {
     HRB_REQUIRE(h, "null handle");
+    if (delivering(h, __func__)) return HRB_ERR_STATE;
     const int frameIndex = h->frameCount >= 3 ? 0 : h->frameCount >= 2 ? 1 : 2;  // opticalFlowCalcSDR.cpp:173
     int rc = beginOutput(h);
     if (rc) return rc;
-    rc = launchCopyFrame(h, frameIndex, ringPlanes(h, h->outCur));
+    const hrb_frame_planes out = ringPlanes(h, h->outCur);
+    rc = launchCopyFrame(h, frameIndex, &out);
     if (rc) return rc;
     HRB_CUDA(cudaEventRecord(h->outReady[h->outCur], h->stream));
     return HRB_OK;
@@ -1187,6 +1216,7 @@ int hrb_ofc_copy_frame(hrb_ofc* h) {
 // timer (warp_calc_time belongs to the ring's downloads) alone.
 int hrb_ofc_warp_frames_to(hrb_ofc* h, int n, const float* blending_scalars, int frame_output_mode, const hrb_frame_planes* dst) {
     HRB_REQUIRE(h && blending_scalars && dst, "null argument");
+    if (delivering(h, __func__)) return HRB_ERR_STATE;
     int rc = checkWarpArgs(n, blending_scalars, frame_output_mode, __func__);
     if (!rc) rc = checkFrames(h, dst, n, true, __func__);
     if (rc) return rc;
@@ -1195,10 +1225,11 @@ int hrb_ofc_warp_frames_to(hrb_ofc* h, int n, const float* blending_scalars, int
 
 int hrb_ofc_copy_frame_to(hrb_ofc* h, const hrb_frame_planes* dst) {
     HRB_REQUIRE(h && dst, "null argument");
+    if (delivering(h, __func__)) return HRB_ERR_STATE;
     const int rc = checkFrames(h, dst, 1, true, __func__);
     if (rc) return rc;
     const int frameIndex = h->frameCount >= 3 ? 0 : h->frameCount >= 2 ? 1 : 2;  // opticalFlowCalcSDR.cpp:173
-    return launchCopyFrame(h, frameIndex, *dst);
+    return launchCopyFrame(h, frameIndex, dst);
 }
 
 int hrb_ofc_download_frame(hrb_ofc* h, uint8_t* output_planes) {
@@ -1641,6 +1672,8 @@ int hrb_split_create(hrb_split** out, hrb_ofc* const* shards, int n) {
         HRB_REQUIRE(shards[k], "null handle");
         for (int j = 0; j < k; ++j) HRB_REQUIRE(shards[j] != shards[k], "a handle appears twice");
     }
+    for (int k = 0; k < n; ++k)
+        if (delivering(shards[k], __func__)) return HRB_ERR_STATE;
     int rc = checkShards(shards, n, "hrb_split_create");
     if (rc) return rc;
     std::vector<int> b((size_t)n + 1);
@@ -1664,6 +1697,7 @@ int hrb_split_create(hrb_split** out, hrb_ofc* const* shards, int n) {
     hrb_split* s = new (std::nothrow) hrb_split();
     HRB_REQUIRE(s, "out of host memory");
     s->shard.assign(shards, shards + n);
+    for (hrb_ofc* h : s->shard) h->groups++;
     s->bounds = b;
     s->done.assign((size_t)n, nullptr);
     for (int k = 0; k < n; ++k) {
@@ -1681,6 +1715,7 @@ int hrb_split_create(hrb_split** out, hrb_ofc* const* shards, int n) {
 
 void hrb_split_destroy(hrb_split* s) {
     if (!s) return;
+    for (hrb_ofc* h : s->shard) h->groups--;
     for (auto e : s->done)
         if (e) cudaEventDestroy(e);
     delete s;
@@ -1744,11 +1779,14 @@ int hrb_flow_batch_create(hrb_flow_batch** out, hrb_ofc* const* members, int n) 
         HRB_REQUIRE(members[k], "null handle");
         for (int j = 0; j < k; ++j) HRB_REQUIRE(members[j] != members[k], "a handle appears twice");
     }
+    for (int k = 0; k < n; ++k)
+        if (delivering(members[k], __func__)) return HRB_ERR_STATE;
     const int rc = checkMembers(members, n, "hrb_flow_batch_create");
     if (rc) return rc;
     hrb_flow_batch* b = new (std::nothrow) hrb_flow_batch();
     HRB_REQUIRE(b, "out of host memory");
     b->member.assign(members, members + n);
+    for (hrb_ofc* h : b->member) h->groups++;
     b->device = members[0]->device;
     int prioLow = 0, prioHigh = 0;
     cudaError_t e = cudaSetDevice(b->device);
@@ -1766,6 +1804,7 @@ int hrb_flow_batch_create(hrb_flow_batch** out, hrb_ofc* const* members, int n) 
 
 void hrb_flow_batch_destroy(hrb_flow_batch* b) {
     if (!b) return;
+    for (hrb_ofc* h : b->member) h->groups--;
     cudaSetDevice(b->device);
     if (b->stream) {
         cudaStreamSynchronize(b->stream);
@@ -1827,6 +1866,352 @@ int hrb_flow_batch_calculate_optical_flow(hrb_flow_batch* b) {
 int hrb_flow_batch_calculate_optical_flow_async(hrb_flow_batch* b) {
     HRB_REQUIRE(b, "null handle");
     return batchCalculate(b, true, "hrb_flow_batch_calculate_optical_flow_async");
+}
+
+// ---- delivery loop ---------------------------------------------------------------------------------
+}  // extern "C"
+
+// DeliverToRenderer's state (CHopperRender, HopperRender.cpp:944-1211) over one handle.  The host keeps everything that
+// needs no delta value: the blending scalar, the interpolation state, and the frame numbers of the delta history with
+// their pruning; the deltas themselves live in a device ring, appended and read by the decision kernel.
+struct hrb_delivery {
+    enum { Deactivated = 0, NotNeeded = 1, Active = 2 };  // ActiveState, HopperRender.h:20-25
+    static constexpr int kRing = 16;  // device delta ring and kept outcomes; the rule reads at most 12 entries
+    hrb_ofc* h = nullptr;
+    hrb_delivery_desc desc{};
+    int state = Deactivated;          // m_iIntActiveState
+    long long playback = 0;           // m_rtCurrPlaybackFrameTime
+    double blend = 0.0;               // m_dBlendingScalar
+    std::deque<long long> history;    // frame numbers of frameDeltaHistory; entry k's delta is ring[(appends - size + k) % 16]
+    unsigned long long appends = 0;   // deltas appended to the ring so far
+    unsigned long long steps = 0;
+    double warpTime = 0.0;            // GPU time of the warps / copy of the newest finished step (auto-tuner)
+    bool timing = false;              // tBegin / tEnd hold a step not yet read
+    uint32_t* ringDev = nullptr;
+    uint32_t* gateDev = nullptr;
+    DeliveryRecord* recDev = nullptr;   // [kRing], step s in s % kRing
+    DeliveryRecord* recHost = nullptr;  // pinned copy of recDev
+    cudaEvent_t recEvent[kRing] = {};
+    cudaEvent_t pass0 = nullptr, tBegin = nullptr, tEnd = nullptr;
+};
+
+namespace hrb {
+
+// m_iNumIntFrames, HopperRender.cpp:945
+static int numIntFrames(double blend, long long target, long long playback) {
+    return (int)std::max(std::ceil((1.0 - blend) / ((double)target / (double)playback)), 1.0);
+}
+
+// HopperRender.cpp:1192-1197
+static double advanceBlend(double blend, long long target, long long playback) {
+    blend += (double)target / (double)playback;
+    if (blend >= 1.0) blend -= 1.0;
+    return blend;
+}
+
+// The largest step the settings can produce (the blending scalar is >= 0, and the count falls as it grows).
+static int checkCount(int state, long long target, long long playback, const char* fn) {
+    if (state == hrb_delivery::Active && numIntFrames(0.0, target, playback) > HRB_DELIVERY_MAX_FRAMES) {
+        setLastError("[hopperrender_b200] %s: a frame-time ratio of %lld / %lld needs more than %d output frames per source frame", fn, target, playback,
+                     HRB_DELIVERY_MAX_FRAMES);
+        return HRB_ERR_INVALID_ARG;
+    }
+    return HRB_OK;
+}
+
+static int checkDesc(const hrb_delivery_desc* d, const char* fn) {
+    if (d->frame_output_mode < 0 || d->frame_output_mode > 6) {
+        setLastError("[hopperrender_b200] %s: frame_output_mode outside 0..6", fn);
+        return HRB_ERR_INVALID_ARG;
+    }
+    if (d->source_frame_time <= 0 || d->target_frame_time <= 0) {
+        setLastError("[hopperrender_b200] %s: frame times must be positive", fn);
+        return HRB_ERR_INVALID_ARG;
+    }
+    return HRB_OK;
+}
+
+// UpdateInterpolationStatus, HopperRender.cpp:819-831
+static void updateInterpolationStatus(hrb_delivery* d) {
+    if (d->state && d->playback > d->desc.target_frame_time)
+        d->state = hrb_delivery::Active;
+    else if (d->state)
+        d->state = hrb_delivery::NotNeeded;
+    d->history.clear();
+}
+
+static int deliveryCount(const hrb_delivery* d) {
+    return d->state == hrb_delivery::Active ? numIntFrames(d->blend, d->desc.target_frame_time, d->playback) : 1;
+}
+
+// autoAdjustSettings, HopperRender.cpp:1438-1463, on the newest finished flow and the newest finished step's outputs
+static int autoAdjust(hrb_delivery* d) {
+    hrb_ofc* h = d->h;
+    int rc = resolveFinishedFlows(h);
+    if (rc) return rc;
+    if (d->timing) {
+        const cudaError_t q = cudaEventQuery(d->tEnd);
+        if (q == cudaSuccess) {
+            float ms = 0;
+            HRB_CUDA(cudaEventElapsedTime(&ms, d->tBegin, d->tEnd));
+            d->warpTime = (double)ms / 1e3;
+            d->timing = false;
+        } else if (q == cudaErrorNotReady) {
+            cudaGetLastError();  // still running: the previous measurement stands
+        } else {
+            HRB_CUDA(q);
+        }
+    }
+    const double sourceFrameTime = (double)d->playback / 10000000.0;
+    const double currMax = h->ofcCalcTime + d->warpTime;
+    if (currMax * 1.4 > sourceFrameTime) {  // UPPER_PERF_BUFFER, config.h:14
+        if (h->searchRadius > 5) h->searchRadius--;
+    } else if (currMax * 1.6 < sourceFrameTime) {  // LOWER_PERF_BUFFER, config.h:15
+        if (h->searchRadius < 16) h->searchRadius++;
+    }
+    return HRB_OK;
+}
+
+// One DeliverToRenderer call: into ring slots outCur .. outCur+n-1 (dst null) or into dst[0..n-1].
+static int deliveryStep(hrb_delivery* d, const hrb_frame_planes* dst, int capacity, hrb_delivery_frame* frames, int* nOut, const char* fn) {
+    hrb_ofc* h = d->h;
+    const int n = deliveryCount(d);
+    if (capacity < n) {
+        setLastError("[hopperrender_b200] %s: the step produces %d frames, capacity is %d", fn, n, capacity);
+        return HRB_ERR_INVALID_ARG;
+    }
+    const bool active = d->state == hrb_delivery::Active;
+    double blends[HRB_DELIVERY_MAX_FRAMES];
+    float ts[HRB_DELIVERY_MAX_FRAMES];
+    for (int i = 0; i < n; ++i) {
+        blends[i] = i == 0 ? d->blend : active ? advanceBlend(blends[i - 1], d->desc.target_frame_time, d->playback) : d->blend;
+        ts[i] = (float)blends[i];
+        if (ts[i] > 1.0f) {  // opticalFlowCalcSDR.cpp:143-146
+            setLastError("[HopperRender] Error in function warpFrames: Blending scalar is greater than 1.0");
+            return HRB_ERR_BLEND_RANGE;
+        }
+    }
+    if (dst) {
+        const int rc = checkFrames(h, dst, n, true, fn);
+        if (rc) return rc;
+    }
+    HRB_CUDA(cudaSetDevice(h->device));
+    if (d->desc.auto_adjust) {
+        const int rc = autoAdjust(d);
+        if (rc) return rc;
+    }
+    const unsigned fc = h->frameCount;
+    const bool flow = active && fc >= 3;
+    if (flow) {
+        const int rc = calculateFlow(Shards(h), true);
+        if (rc) return rc;
+        // The decision reads rawDeltaDev once pass 0 has written it.  The next flow is forked behind the compute stream,
+        // i.e. behind the decision kernel enqueued below, so it cannot overwrite rawDeltaDev before the kernel has read it.
+        HRB_CUDA(cudaStreamWaitEvent(h->stream, d->pass0, 0));
+        d->appends++;
+        // frameDeltaHistory, HopperRender.cpp:959-973: entries older than 3 s of source frames leave
+        const long long framesIn3s = (long long)(3.0 * 10000000.0 / (double)d->desc.source_frame_time);
+        d->history.push_back(fc);
+        while (!d->history.empty() && (long long)fc - d->history.front() > framesIn3s) d->history.pop_front();
+    }
+    const unsigned long long step = d->steps;
+    const int rec = (int)(step % hrb_delivery::kRing);
+    DeliveryDecision dd;
+    dd.rawDelta = h->rawDeltaDev;
+    dd.divisor = (unsigned)(h->flowHeight * h->flowWidth * (h->hdr ? 6 : 10));
+    dd.ring = d->ringDev;
+    dd.append = flow ? 1 : 0;
+    dd.slot = (int)((d->appends + hrb_delivery::kRing - 1) % hrb_delivery::kRing);
+    dd.n = (int)d->history.size();
+    dd.count = dd.n >= 3 ? std::min(dd.n - 2, 10) : 0;
+    dd.threshold = d->desc.scene_change_threshold;
+    dd.copy = flow ? 0 : 1;
+    dd.gate = d->gateDev;
+    dd.out = d->recDev + rec;
+    int rc = launchDeliveryDecision(h, dd);
+    if (rc) return rc;
+    HRB_CUDA(cudaMemcpyAsync(d->recHost + rec, d->recDev + rec, sizeof(DeliveryRecord), cudaMemcpyDeviceToHost, h->stream));
+    HRB_CUDA(cudaEventRecord(d->recEvent[rec], h->stream));
+
+    // the outputs: warps under "no scene change" and copies under "scene change", or copies the host already knows of
+    hrb_frame_planes outs[HRB_DELIVERY_MAX_FRAMES];
+    if (!dst) {
+        rc = beginOutput(h);  // waits for the download of the first slot, starts the warp timer
+        if (rc) return rc;
+        for (int i = 0; i < n; ++i) {
+            const int slot = (h->outCur + i) % hrb_ofc::kOutRing;
+            if (i) HRB_CUDA(cudaStreamWaitEvent(h->stream, h->outFree[slot], 0));
+            outs[i] = ringPlanes(h, slot);
+        }
+        dst = outs;
+    }
+    HRB_CUDA(cudaEventRecord(d->tBegin, h->stream));
+    const int copyIndex = fc >= 3 ? 0 : fc >= 2 ? 1 : 2;  // opticalFlowCalcSDR.cpp:173
+    if (flow) {
+        for (int i0 = 0; i0 < n && !rc; i0 += HRB_WARP_BATCH_MAX)
+            rc = launchWarpFrames(h, std::min(n - i0, HRB_WARP_BATCH_MAX), ts + i0, dst + i0, d->desc.frame_output_mode, d->gateDev, 0);
+        if (!rc) rc = launchCopyFrame(h, copyIndex, dst, n, d->gateDev, 1);
+    } else {
+        rc = launchCopyFrame(h, copyIndex, dst, n);
+    }
+    if (rc) return rc;
+    HRB_CUDA(cudaEventRecord(d->tEnd, h->stream));
+    d->timing = true;
+    if (dst == outs)
+        for (int i = 0; i < n; ++i) HRB_CUDA(cudaEventRecord(h->outReady[(h->outCur + i) % hrb_ofc::kOutRing], h->stream));
+
+    for (int i = 0; i < n; ++i) frames[i] = hrb_delivery_frame{fc, i, blends[i], step};
+    if (active) d->blend = advanceBlend(blends[n - 1], d->desc.target_frame_time, d->playback);
+    d->steps++;
+    *nOut = n;
+    return HRB_OK;
+}
+
+}  // namespace hrb
+
+extern "C" {
+
+void hrb_delivery_destroy(hrb_delivery* d) {
+    if (!d) return;
+    hrb_ofc* h = d->h;
+    if (h) {
+        cudaSetDevice(h->device);
+        cudaStreamSynchronize(h->flowStream);
+        cudaStreamSynchronize(h->stream);
+        // the graphs that record this delivery's pass-0 event go with it
+        for (auto& g : h->flowGraphs)
+            if (g.pass0 == d->pass0 && g.exec) {
+                cudaGraphExecDestroy(g.exec);
+                g.exec = nullptr;
+            }
+        h->flowGraphs.erase(std::remove_if(h->flowGraphs.begin(), h->flowGraphs.end(), [](const hrb_ofc::FlowGraph& g) { return !g.exec; }), h->flowGraphs.end());
+        if (h->delivery == d) {
+            h->delivery = nullptr;
+            h->pass0Event = nullptr;
+        }
+    }
+    cudaFree(d->ringDev);
+    cudaFree(d->gateDev);
+    cudaFree(d->recDev);
+    if (d->recHost) cudaFreeHost(d->recHost);
+    for (auto e : d->recEvent)
+        if (e) cudaEventDestroy(e);
+    if (d->pass0) cudaEventDestroy(d->pass0);
+    if (d->tBegin) cudaEventDestroy(d->tBegin);
+    if (d->tEnd) cudaEventDestroy(d->tEnd);
+    delete d;
+}
+
+int hrb_delivery_create(hrb_delivery** out, hrb_ofc* h, const hrb_delivery_desc* desc) {
+    HRB_REQUIRE(out && desc, "null argument");
+    *out = nullptr;
+    int rc = checkDesc(desc, __func__);
+    if (!rc) rc = checkCount(desc->active ? hrb_delivery::Active : hrb_delivery::Deactivated, desc->target_frame_time, desc->source_frame_time, __func__);
+    if (rc) return rc;
+    HRB_REQUIRE(h, "null handle");
+    if (h->delivery || h->groups) {
+        setLastError("[hopperrender_b200] %s: the handle already has a delivery, or belongs to a split group or a flow batch", __func__);
+        return HRB_ERR_STATE;
+    }
+    HRB_CUDA(cudaSetDevice(h->device));
+    hrb_delivery* d = new (std::nothrow) hrb_delivery();
+    HRB_REQUIRE(d, "out of host memory");
+    d->desc = *desc;
+    d->state = desc->active ? hrb_delivery::Active : hrb_delivery::Deactivated;  // as the filter starts: no status update yet
+    d->playback = desc->source_frame_time;
+    cudaError_t e = cudaMalloc(&d->ringDev, hrb_delivery::kRing * sizeof(uint32_t));
+    if (e == cudaSuccess) e = cudaMemsetAsync(d->ringDev, 0, hrb_delivery::kRing * sizeof(uint32_t), h->stream);
+    if (e == cudaSuccess) e = cudaMalloc(&d->gateDev, sizeof(uint32_t));
+    if (e == cudaSuccess) e = cudaMalloc(&d->recDev, hrb_delivery::kRing * sizeof(DeliveryRecord));
+    if (e == cudaSuccess) e = cudaMallocHost(&d->recHost, hrb_delivery::kRing * sizeof(DeliveryRecord));
+    for (auto& ev : d->recEvent)
+        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&d->pass0, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventCreate(&d->tBegin);
+    if (e == cudaSuccess) e = cudaEventCreate(&d->tEnd);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    if (e != cudaSuccess) {
+        setLastError("[hopperrender_b200] CUDA error %d (%s) in hrb_delivery_create", (int)e, cudaGetErrorString(e));
+        hrb_delivery_destroy(d);
+        return HRB_ERR_CUDA;
+    }
+    d->h = h;
+    h->delivery = d;
+    h->pass0Event = d->pass0;
+    *out = d;
+    return HRB_OK;
+}
+
+int hrb_delivery_next_count(hrb_delivery* d, int* n) {
+    HRB_REQUIRE(d && n, "null argument");
+    *n = deliveryCount(d);
+    return HRB_OK;
+}
+
+int hrb_delivery_step(hrb_delivery* d, hrb_delivery_frame* frames, int capacity, int* n) {
+    HRB_REQUIRE(d && frames && n, "null argument");
+    return deliveryStep(d, nullptr, capacity, frames, n, __func__);
+}
+
+int hrb_delivery_step_to(hrb_delivery* d, const hrb_frame_planes* dst, int capacity, hrb_delivery_frame* frames, int* n) {
+    HRB_REQUIRE(d && dst && frames && n, "null argument");
+    return deliveryStep(d, dst, capacity, frames, n, __func__);
+}
+
+int hrb_delivery_outcome_of(hrb_delivery* d, unsigned long long step, int wait, hrb_delivery_outcome* out) {
+    HRB_REQUIRE(d && out, "null argument");
+    HRB_REQUIRE(step < d->steps && step + hrb_delivery::kRing >= d->steps, "step not among the last 16 steps");
+    HRB_CUDA(cudaSetDevice(d->h->device));
+    const int rec = (int)(step % hrb_delivery::kRing);
+    if (wait) {
+        HRB_CUDA(cudaEventSynchronize(d->recEvent[rec]));
+    } else {
+        const cudaError_t q = cudaEventQuery(d->recEvent[rec]);
+        if (q == cudaErrorNotReady) {
+            cudaGetLastError();
+            setLastError("[hopperrender_b200] %s: the decision of step %llu is still in flight", __func__, step);
+            return HRB_ERR_STATE;
+        }
+        HRB_CUDA(q);
+    }
+    const DeliveryRecord& r = d->recHost[rec];
+    out->warped = r.warped;
+    out->scene_change = r.sceneChange;
+    out->delta1 = r.d1;
+    out->delta2 = r.d2;
+    out->frame_delta = r.frameDelta;
+    return HRB_OK;
+}
+
+int hrb_delivery_set(hrb_delivery* d, const hrb_delivery_desc* desc) {
+    HRB_REQUIRE(d && desc, "null argument");
+    int rc = checkDesc(desc, __func__);
+    if (rc) return rc;
+    HRB_REQUIRE(desc->source_frame_time == d->desc.source_frame_time, "source_frame_time differs from the delivery's (a new source rate is a new delivery)");
+    // UpdateUserSettings, HopperRender.cpp:1355-1390, then UpdateInterpolationStatus
+    const int state = !desc->active ? (int)hrb_delivery::Deactivated : d->state ? d->state : (int)hrb_delivery::Active;
+    const int after = state && d->playback > desc->target_frame_time ? (int)hrb_delivery::Active : state ? (int)hrb_delivery::NotNeeded : state;
+    rc = checkCount(after, desc->target_frame_time, d->playback, __func__);
+    if (rc) return rc;
+    d->desc = *desc;
+    d->state = state;
+    updateInterpolationStatus(d);
+    return HRB_OK;
+}
+
+int hrb_delivery_new_segment(hrb_delivery* d, double rate) {
+    HRB_REQUIRE(d, "null argument");
+    HRB_REQUIRE(rate > 0.0 && std::isfinite(rate), "rate must be a positive number");
+    // NewSegment, HopperRender.cpp:834-844
+    const long long playback = (long long)((double)d->desc.source_frame_time * (1.0 / rate));
+    HRB_REQUIRE(playback > 0, "rate too high for the source frame time");
+    const int after = d->state && playback > d->desc.target_frame_time ? (int)hrb_delivery::Active : d->state ? (int)hrb_delivery::NotNeeded : d->state;
+    const int rc = checkCount(after, d->desc.target_frame_time, playback, __func__);
+    if (rc) return rc;
+    d->playback = playback;
+    updateInterpolationStatus(d);
+    d->h->frameCount = 0;
+    return HRB_OK;
 }
 
 uint64_t hrb_kernel_launch_count(void) { return g_launchCount.load(std::memory_order_relaxed); }

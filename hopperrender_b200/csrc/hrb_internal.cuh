@@ -262,6 +262,7 @@ struct hrb_ofc {
         const void* plane2;
         const void* blurOut;
         int R, deltaScalar, neighborBiasScalar, variant;
+        cudaEvent_t pass0;  // pass0Event the graph records (an external event node), or null
         cudaGraphExec_t exec;
         unsigned launches;
     };
@@ -277,6 +278,11 @@ struct hrb_ofc {
     std::vector<SideBlob> sideData;        // IMediaSideData blobs of the newest source frame (opaque, host memory)
     unsigned long long* dbgDev = nullptr;  // per-CTA timelines of the search passes (debug aid, off by default)
     size_t dbgStride = 0;                  // words per pass
+    // delivery loop (hrb_delivery): the attached delivery, and the event a flow records right after its pass 0, when
+    // rawDeltaDev holds the flow's raw frame delta (null without a delivery)
+    hrb_delivery* delivery = nullptr;
+    cudaEvent_t pass0Event = nullptr;
+    int groups = 0;  // split groups and flow batches the handle belongs to
 };
 
 namespace hrb {
@@ -285,9 +291,32 @@ namespace hrb {
 // Ingest into input slot `slot`: src null packs the slot itself (filled by an upload); otherwise the pack reads the planes
 // of src and also writes their samples into the slot.
 int launchPackFrame(hrb_ofc* h, int slot, const hrb_frame_planes* src);
-// copyFrame / warpFrames into destination planes: a ring slot or a caller's surface (the warp's dst[i] share dst[0]'s pitches)
-int launchCopyFrame(hrb_ofc* h, int slot, const hrb_frame_planes& dst);
-int launchWarpFrames(hrb_ofc* h, int n, const float* t, const hrb_frame_planes* dst, int mode);
+// copyFrame / warpFrames into destination planes: ring slots or a caller's surfaces (dst[i] share dst[0]'s pitches).
+// gate: null, or a device word; then every CTA returns at once unless *gate == gateWhen (the delivery loop's decision).
+// The copy writes the same frame into each of its n destinations (n <= kCopyDstMax).
+constexpr int kCopyDstMax = 16;
+int launchCopyFrame(hrb_ofc* h, int slot, const hrb_frame_planes* dst, int n = 1, const uint32_t* gate = nullptr, uint32_t gateWhen = 0);
+int launchWarpFrames(hrb_ofc* h, int n, const float* t, const hrb_frame_planes* dst, int mode, const uint32_t* gate = nullptr, uint32_t gateWhen = 0);
+// kernels_delivery.cu: the delivery loop's scene-change decision (see hrb_api.cu, hrb_delivery)
+struct DeliveryRecord {  // mirrors hrb_delivery_outcome
+    int warped, sceneChange;
+    long long d1, d2;
+    unsigned frameDelta;
+};
+struct DeliveryDecision {
+    const uint32_t* rawDelta;  // the flow's raw frame delta (valid when append)
+    unsigned divisor;          // lh * lw * (hdr ? 6 : 10)
+    uint32_t* ring;            // [16] frame deltas: history entry k sits at ring[(seq of k) % 16]
+    int append;                // the step computed a flow: ring[slot] = rawDelta / divisor
+    int slot;                  // ring index of the newest history entry (nxt)
+    int n;                     // history entries after the append
+    int count;                 // min(n - 2, 10): the entries averaged
+    long long threshold;
+    int copy;                  // the host knows the outputs are copies (inactive, frame_count < 3)
+    uint32_t* gate;            // receives sceneChange (read by the gated warps and copy)
+    DeliveryRecord* out;
+};
+int launchDeliveryDecision(hrb_ofc* h, const DeliveryDecision& d);
 // kernels_search.cu
 int launchSearchPass(hrb_ofc* h, const SearchArgs& a, int R, int step);
 // One pass of the n members of a flow batch, on h[0]->stream: a generic pass is one launch over all of them, a tile or

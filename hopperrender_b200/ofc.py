@@ -494,6 +494,107 @@ class FlowBatch:
             pass
 
 
+class Delivery:
+    """The filter's delivery loop (DeliverToRenderer, HopperRender.cpp:944-1211) over one calculator (hrb_delivery_*):
+    output count, auto-tuner, flow, frame-delta history, scene-change rule and blending scalar, with the scene-change
+    decision taken on the GPU.  While it is open, calculateOpticalFlow(Async), warpFrames* and copyFrame* on the
+    calculator raise; ingest and downloads stay available.  Close it before the calculator.
+
+    deliver() has the signature and the info dicts of hopperrender_b200.replay.DeliveryLoop.deliver; deliver_to() writes
+    into caller tensors and leaves the decision in flight (outcome() fetches it)."""
+
+    def __init__(self, calc, source_frame_time=417083, target_frame_time=69444, frame_output=2, scene_change_threshold=200,
+                 active=True, auto_adjust=True):
+        self._lib = L.load()
+        self.calc = calc  # keeps the handle alive as long as the delivery
+        self._d = C.c_void_p()
+        self._desc = L.hrb_delivery_desc(int(source_frame_time), int(target_frame_time), int(frame_output), int(scene_change_threshold),
+                                         1 if active else 0, 1 if auto_adjust else 0)
+        self._check(self._lib.hrb_delivery_create(C.byref(self._d), calc._h, C.byref(self._desc)))
+        self._frames = (L.hrb_delivery_frame * L.DELIVERY_MAX_FRAMES)()
+
+    def _check(self, rc):
+        if rc != L.HRB_OK:
+            raise RuntimeError(f"hrb error {rc}: {L.last_error()}")
+
+    def next_count(self):
+        n = C.c_int()
+        self._check(self._lib.hrb_delivery_next_count(self._d, C.byref(n)))
+        return n.value
+
+    def _infos(self, n):
+        return [{"source": f.source, "index": f.index, "blend": f.blend, "step": f.step} for f in self._frames[:n]]
+
+    def step(self):
+        """One step into the output ring: fetch its frames with len(result) downloads."""
+        n = C.c_int()
+        self._check(self._lib.hrb_delivery_step(self._d, self._frames, L.DELIVERY_MAX_FRAMES, C.byref(n)))
+        return self._infos(n.value)
+
+    def outcome(self, step, wait=True):
+        """{warped, scene_change, delta1, delta2, frame_delta} of a step; None while in flight when wait is False."""
+        o = L.hrb_delivery_outcome()
+        rc = self._lib.hrb_delivery_outcome_of(self._d, int(step), 1 if wait else 0, C.byref(o))
+        if rc == L.HRB_ERR_STATE and not wait:
+            return None
+        self._check(rc)
+        return {"warped": bool(o.warped), "scene_change": bool(o.scene_change), "delta1": o.delta1, "delta2": o.delta2,
+                "frame_delta": o.frame_delta}
+
+    def deliver(self, in_buffer, out_buffer, sink=None, side_data=None):
+        """updateFrame, one step into the ring, one downloadFrame per output frame; sink(out_buffer, info) as in
+        replay.DeliveryLoop.deliver.  Returns the number of frames delivered."""
+        c = self.calc
+        c.updateFrame(in_buffer)
+        frames = self.step()
+        radius = c.m_opticalFlowSearchRadius
+        for info in frames:
+            c.downloadFrame(out_buffer)
+            o = self.outcome(info["step"])
+            info.update(warped=o["warped"], scene_change=o["scene_change"], radius=radius, side_data=side_data, outcome=o)
+            if sink is not None:
+                sink(out_buffer, info)
+        return len(frames)
+
+    def deliver_to(self, y, uv, outs):
+        """updateFramePlanes(y, uv), then one step into outs[i] = (y, uv) tensors (at least next_count() of them).  The
+        frames are ready for work ordered behind calc.streamHandle(); returns their infos (outcome(info["step"]) gives
+        the decision)."""
+        c = self.calc
+        c.updateFramePlanes(y, uv)
+        dst = (L.hrb_frame_planes * max(len(outs), 1))(*[c._planes(a, b) for a, b in outs])
+        n = C.c_int()
+        self._check(self._lib.hrb_delivery_step_to(self._d, dst, len(outs), self._frames, C.byref(n)))
+        return self._infos(n.value)
+
+    def set_settings(self, frame_output=None, scene_change_threshold=None, active=None, auto_adjust=None, target_frame_time=None):
+        """UpdateUserSettings (HopperRender.cpp:1355-1390) for the delivery's own settings; clears the delta history."""
+        d = L.hrb_delivery_desc.from_buffer_copy(self._desc)
+        for k, v in (("frame_output_mode", frame_output), ("scene_change_threshold", scene_change_threshold), ("target_frame_time", target_frame_time)):
+            if v is not None:
+                setattr(d, k, int(v))
+        for k, v in (("active", active), ("auto_adjust", auto_adjust)):
+            if v is not None:
+                setattr(d, k, 1 if v else 0)
+        self._check(self._lib.hrb_delivery_set(self._d, C.byref(d)))
+        self._desc = d
+
+    def new_segment(self, rate=1.0):
+        """NewSegment (HopperRender.cpp:834-844): seek or playback-speed change."""
+        self._check(self._lib.hrb_delivery_new_segment(self._d, float(rate)))
+
+    def close(self):
+        if getattr(self, "_d", None) is not None and self._d.value:
+            self._lib.hrb_delivery_destroy(self._d)
+            self._d = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def kernel_launch_count():
     return int(L.load().hrb_kernel_launch_count())
 

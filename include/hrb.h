@@ -204,6 +204,82 @@ HRB_API int hrb_ofc_copy_frame_to(hrb_ofc* h, const hrb_frame_planes* dst);
  * The blend scalars and the mode are checked as warp_frames_batch checks them (HRB_ERR_BLEND_RANGE for a scalar above 1,
  * HRB_ERR_INVALID_ARG for a mode outside 0..6). */
 
+/* ---- delivery loop ------------------------------------------------------------------------------------------------ */
+/* The filter's DeliverToRenderer (HopperRender.cpp:944-1211) on top of one handle: for every source frame it decides how
+ * many output frames to produce, advances the blending scalar, runs the search-radius auto-tuner and applies the
+ * scene-change rule that chooses warp_frames or copy_frame.  The scene-change decision is taken by a kernel on the GPU,
+ * so a step never waits for a flow calculation: the warps of a step keep running beside the search of its flow.
+ *
+ * One step is one DeliverToRenderer call, in its order:
+ *   1. the output count n (m_iNumIntFrames, :945): ceil((1 - blend) / (target / playback)) when interpolation is active,
+ *      otherwise 1;
+ *   2. the auto-tuner (:951, :1438-1463) when auto_adjust is on;
+ *   3. calculate_optical_flow_async when active and frame_count >= 3, and the frame-delta history (:959-973);
+ *   4. the warp-or-copy choice for all n output frames (:1126-1183);
+ *   5. the blend-scalar advance (:1192-1197).
+ * The caller does the ingest (update_frame, _async, _device or _planes) of a source frame before the step that delivers
+ * it.  hrb_delivery_step writes the n frames into the output ring: fetch them with n download_frame(_async) calls, in
+ * order.  hrb_delivery_step_to writes output frame i into dst[i]: the frames are ready for work ordered behind
+ * hrb_ofc_stream.  Steps of more than HRB_WARP_BATCH_MAX frames run as two warp batches under the same decision.  A step
+ * of more than HRB_DELIVERY_MAX_FRAMES frames (the output ring's size) cannot be delivered: create, set and new_segment
+ * refuse settings whose target / playback ratio needs one, with HRB_ERR_INVALID_ARG.
+ *
+ * Exclusive use: while a delivery is attached to a handle, calculate_optical_flow(_async), warp_frames(_batch, _to) and
+ * copy_frame(_to) on that handle return HRB_ERR_STATE (the delta history would no longer describe the flows).  Ingest,
+ * downloads, get_state / peek_state and set_params stay allowed.  A handle has at most one delivery, and the delivery is
+ * destroyed before its handle.  A handle in a split group or a flow batch cannot have a delivery, and a handle with a
+ * delivery cannot join either (HRB_ERR_STATE).
+ *
+ * Outcomes: the decision of step s (warped, scene change, the rule's two deltas d1 and d2, the frame delta the step
+ * appended) is copied to host memory behind the step's kernels.  hrb_delivery_outcome_of(s, wait = 0) returns
+ * HRB_ERR_STATE while it is still in flight; wait = 1 blocks until it has landed.  The last HRB_DELIVERY_MAX_FRAMES steps
+ * are kept (older ones: HRB_ERR_INVALID_ARG).
+ *
+ * Auto-tuner inputs: the newest FINISHED flow calculation's time (what peek_state reports) plus the GPU time of the
+ * warps / copy of the newest step whose outputs have finished, measured by events around them.  The filter reads the
+ * flow it has just computed and the time until its downloads ended; neither is available without waiting. */
+#define HRB_DELIVERY_MAX_FRAMES 16
+typedef struct hrb_delivery hrb_delivery;
+typedef struct hrb_delivery_desc {
+    long long source_frame_time;   /* 100-ns units, rtSourceFrameTime (417083 = 23.976 fps); > 0 */
+    long long target_frame_time;   /* 100-ns units, rtTargetFrameTime (69444 = 144 fps); > 0 */
+    int frame_output_mode;         /* 0..6 (HRB_MODE_*) */
+    int scene_change_threshold;    /* m_iSceneChangeThreshold; HopperRender's default is 200 */
+    int active;                    /* interpolation switched on (m_iIntActiveState != Deactivated) */
+    int auto_adjust;               /* run the search-radius auto-tuner (autoAdjustSettings, HopperRender.cpp:1438-1463) */
+} hrb_delivery_desc;
+/* One output frame of a step: known when the step returns. */
+typedef struct hrb_delivery_frame {
+    unsigned int source;           /* frame_count of the source frame it belongs to */
+    int index;                     /* 0 .. n-1 inside the step */
+    double blend;                  /* m_dBlendingScalar the frame is warped at */
+    unsigned long long step;       /* the step's number (0 for the first step of a delivery) */
+} hrb_delivery_frame;
+/* The decision of one step, taken on the GPU. */
+typedef struct hrb_delivery_outcome {
+    int warped;                    /* 1: the step's frames were warped; 0: copied (copy_frame) */
+    int scene_change;              /* sceneChangeDetected of HopperRender.cpp:1126-1176 */
+    long long delta1, delta2;      /* cur - average and cur - nxt of the rule (0 with fewer than 3 history entries) */
+    unsigned int frame_delta;      /* total_frame_delta of the flow the step computed (0: the step computed no flow) */
+} hrb_delivery_outcome;
+/* The descriptor is checked before the handle: HRB_ERR_INVALID_ARG for a null out / descriptor, a mode outside 0..6, a
+ * non-positive frame time, a ratio needing more than HRB_DELIVERY_MAX_FRAMES outputs per step, or a null handle. */
+HRB_API int hrb_delivery_create(hrb_delivery** out, hrb_ofc* h, const hrb_delivery_desc* desc);
+HRB_API void hrb_delivery_destroy(hrb_delivery* d);
+/* the number of output frames the next step will produce */
+HRB_API int hrb_delivery_next_count(hrb_delivery* d, int* n);
+/* One step into the output ring; frames[0..n-1] describe the n frames (capacity >= n, else HRB_ERR_INVALID_ARG). */
+HRB_API int hrb_delivery_step(hrb_delivery* d, hrb_delivery_frame* frames, int capacity, int* n);
+/* One step into dst[0..n-1] (capacity >= n; the planes are checked as warp_frames_to checks them). */
+HRB_API int hrb_delivery_step_to(hrb_delivery* d, const hrb_frame_planes* dst, int capacity, hrb_delivery_frame* frames, int* n);
+HRB_API int hrb_delivery_outcome_of(hrb_delivery* d, unsigned long long step, int wait, hrb_delivery_outcome* out);
+/* UpdateUserSettings (HopperRender.cpp:1355-1390): mode, threshold, activation, auto-tuner and target frame time; clears
+ * the delta history.  source_frame_time must be the one the delivery was created with.  The calculator's scalars and
+ * levels are set with hrb_ofc_set_params. */
+HRB_API int hrb_delivery_set(hrb_delivery* d, const hrb_delivery_desc* desc);
+/* NewSegment (HopperRender.cpp:834-844): playback frame time = source frame time / rate, history cleared, frame_count 0 */
+HRB_API int hrb_delivery_new_segment(hrb_delivery* d, double rate);
+
 /* ---- side data of the source frames ----------------------------------------------------------------------------- */
 /* The filter reads the IMediaSideData blobs of the input sample (HDR10 / HDR10+ / Dolby Vision metadata and RPU, control
  * flags, content light level, EIA-608 captions, 3D offset: HopperRender.cpp:875-900) and sets them on EVERY output sample it
