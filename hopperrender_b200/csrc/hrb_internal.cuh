@@ -271,6 +271,11 @@ struct hrb_ofc {
     std::vector<hrb::PassTapDev> taps;
     hrb::Profile prof;
     hrb::TmaCache* tmaCache = nullptr;  // TMA descriptors of the search planes, encoded on first use
+    struct TileResidency {
+        const void* kernel;
+        int nwv, ctasPerSm;
+    };
+    std::vector<TileResidency> tileResidency;  // CTAs per SM the runtime places, per tile kernel instance and height
     struct SideBlob {
         uint8_t guid[16];
         std::vector<uint8_t> bytes;

@@ -674,8 +674,9 @@ __global__ void __maxnreg__(128)
         } else {
             // add the CTA's sums to the window's scratch; the LAST CTA to arrive (ticket) finds them complete, finalizes the
             // window and leaves scratch and ticket zeroed for the next pass — no finalize kernel, no memset between passes.
-            // A sharded pass (split search) has windows of at most 128 rows here, and every CTA covering an owned window
-            // lies inside the stripe (tiles are 128 rows, stripes start at multiples of 128): the count is unchanged.
+            // A tile lies inside one window (chooseWarps), so the window's CTAs are its tiles.  A sharded pass (split
+            // search) has windows of at most 128 rows here, hence 128-row tiles, and every CTA covering an owned window
+            // lies inside the stripe (stripes start at multiples of 128): the count is unchanged.
             const int wu = U0 >> wsLog2, wv = V0 >> wsLog2;
             const int wx = View<STEP>::wx(wu, wv), wy = View<STEP>::wy(wu, wv);
             const size_t widx = (size_t)(wy * a.nWx + wx);
@@ -805,30 +806,57 @@ template <int WSC> int tileSmem(const TileParams& tp) {
     return tp.lumaBytes + tp.chromaBytes + nWin * 4 + ((nWin + 15) & ~15) + 128;  // boxes, window displacements, window states, alignment slack
 }
 
+// CTAs of sadTileKernel<R, STEP, WSC> with nwv warps the runtime places on one SM, asked once per handle.  The kernel's
+// dynamic shared-memory limit is raised first (the runtime counts 0 CTAs for a kernel not allowed that much), and the
+// carve-out is set to the maximum, so that the driver does not pick a smaller one that drops a CTA.
+template <int R, int STEP, int WSC> int residentTiles(hrb_ofc* h, int nwv, int smem, int& perSm) {
+    const void* fn = reinterpret_cast<const void*>(sadTileKernel<R, STEP, WSC>);
+    for (const auto& e : h->tileResidency)
+        if (e.kernel == fn && e.nwv == nwv) {
+            perSm = e.ctasPerSm;
+            return HRB_OK;
+        }
+    const int rc = allowDynamicSmem<sadTileKernel<R, STEP, WSC>>(h->device, smem);
+    if (rc) return rc;
+    HRB_CUDA(cudaFuncSetAttribute(sadTileKernel<R, STEP, WSC>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    HRB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, sadTileKernel<R, STEP, WSC>, 32 * nwv, smem));
+    h->tileResidency.push_back({fn, nwv, perSm});
+    return HRB_OK;
+}
+
 // Warps per CTA (tile rows / 32): the choice that needs the fewest rounds of resident CTAs, then the smallest halo share.
-template <int R, int WSC> int chooseWarps(const hrb_ofc* h, int lu, int lv) {
-    if (WSC >= 128) return 4;
-    int best = 4;
+// Classes 64 and 128 count rounds from the CTAs per SM the runtime places.  A tile of class 128 lies inside one window
+// (32 * nwv divides ws: the window's CTAs are counted by its arrival ticket), and a tile of class 64 holds whole window
+// rows, at most 8 windows (s_red).  Classes 16 and 32 keep the fixed residency estimate their shapes were tuned with.
+template <int R, int STEP, int WSC> int chooseWarps(hrb_ofc* h, int lu, int lv, int ws, int& nwvOut) {
+    nwvOut = 4;
     double bestCost = 1e30;
-    for (int nwv = 2; nwv <= 6; ++nwv) {
-        if (WSC == 64 && (nwv & 1)) continue;  // the tile holds whole window rows
-        if (WSC == 64 && nwv > 4) continue;    // s_red holds 8 windows
+    for (int nwv = 2; nwv <= 8; ++nwv) {
+        if (WSC >= 128 ? (nwv != 4 && nwv != 8) || ws % (32 * nwv) : WSC == 64 ? (nwv & 1) != 0 : nwv > 6) continue;
         const TileParams tp = tileParams<R, WSC>(nwv);
-        if (tp.boxHC > 256) continue;
+        if (tp.boxHC > 256) continue;  // the chroma box is one TMA box
         const int smem = tileSmem<WSC>(tp);
-        const int perSm = min(min((233472) / (smem + 1040), 3), 2048 / (32 * nwv));  // __launch_bounds__(192, 3)
+        int perSm = min(min((233472) / (smem + 1040), 3), 2048 / (32 * nwv));
+        if (WSC >= 64) {
+            const int rc = residentTiles<R, STEP, WSC>(h, nwv, smem, perSm);
+            if (rc) return rc;
+        }
         if (perSm < 1) continue;
         const long tiles = (long)((lu + 127) / 128) * ((lv + 32 * nwv - 1) / (32 * nwv));
         const long slots = (long)h->smCount * perSm;
         const long rounds = (tiles + slots - 1) / slots;
-        // a round costs the tile's rows plus the candidate span; few resident warps hide latency badly
-        const double cost = (double)rounds * (32 * nwv + CandSpan<R>::SPAN) * (1.0 + 2.0 / (perSm * nwv));
+        // a round costs the tile's rows plus the candidate span; few resident warps hide latency badly.  Class 128 counts
+        // the tiles of the busiest SM instead of rounds: its grids are one round at either height, and the rows that SM
+        // stages (the span once per tile) are what a taller tile saves
+        const long perBusiest = WSC >= 128 ? (tiles + h->smCount - 1) / h->smCount : rounds;
+        const long resident = WSC >= 128 ? min((long)perSm, perBusiest) : perSm;
+        const double cost = (double)perBusiest * (32 * nwv + CandSpan<R>::SPAN) * (1.0 + 2.0 / (resident * nwv));
         if (cost < bestCost) {
             bestCost = cost;
-            best = nwv;
+            nwvOut = nwv;
         }
     }
-    return best;
+    return HRB_OK;
 }
 
 template <int R, int STEP, int WSC> int launchTile(hrb_ofc* h, const SearchArgs& a, const SearchPlan& p) {
@@ -838,11 +866,14 @@ template <int R, int STEP, int WSC> int launchTile(hrb_ofc* h, const SearchArgs&
     const int dimU = STEP == 1 ? a.W : a.H, dimV = STEP == 1 ? a.H : a.W;
     const uint8_t* c1 = STEP == 1 ? a.c1 : a.cT1;
     const int pitch = STEP == 1 ? a.pitch : a.pitchT;
-    TileParams tp = tileParams<R, WSC>(chooseWarps<R, WSC>(h, lu, lv));
+    int nwv;
+    int rc = chooseWarps<R, STEP, WSC>(h, lu, lv, a.ws, nwv);
+    if (rc) return rc;
+    TileParams tp = tileParams<R, WSC>(nwv);
     tp.useTma = p.useTma;
     tp.forceSlow = p.forceSlow;
     const int smem = tileSmem<WSC>(tp);
-    const int rc = allowDynamicSmem<sadTileKernel<R, STEP, WSC>>(h->device, smem);
+    rc = allowDynamicSmem<sadTileKernel<R, STEP, WSC>>(h->device, smem);
     if (rc) return rc;
     const CUtensorMap* mC = tp.useTma ? tensorMapFor(h, c1, dimU, dimV / 2, pitch, C::BW, tp.boxHC) : nullptr;
     CUtensorMap dummy;
